@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle/_ref)
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/*.npy
 
 Workload (config.workload): BASELINE.json configs[1] — 1-D BQ, 64 observations, expected_Z_var over
 a 10^6-point grid (SURVEY.md §8(d) generator).  A *step* is one pass of the hot path over the
@@ -420,6 +421,14 @@ def cfg_c5_problems(world, rank, dev, rounds=20):
     return out
 
 
+def dump_outputs(path, arrays):
+    """Writes `arrays` as <path>/<name>.npy (float64).  The inputs are seeded, so two builds run with the same arguments can
+    be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_cuda(args):
     import torch
     import torch.distributed as dist
@@ -579,6 +588,12 @@ def run_cuda(args):
     barrier()
     launches = batch.launch_count - launches0
     ms_per_step = max_over_ranks(float(np.sum(step_ms)), dev, world) / args.steps
+    if args.dump_outputs and rank == 0:
+        # what the last timed step handed its caller (rank 0's shard, 16 MB, and the global pair), before the sustained loop
+        # reuses the buffers
+        last_esm, last_ev = (sets[(args.steps - 1) % NSETS][1:] if sets is not None else (esm[0], evv))
+        dump_outputs(args.dump_outputs, {"esm": last_esm.cpu().numpy(), "expected_Z_var": last_ev.cpu().numpy(),
+                                         "argmin": np.array(result, dtype=np.float64)})
     value = na_total / (ms_per_step * 1e-3)
     clocks = sampler.stop() if sampler else None
 
@@ -733,7 +748,12 @@ def main():
     ap.add_argument("--no-sustained", action="store_true", help="skip the >= 2 s sustained loop")
     ap.add_argument("--cpu-points", type=int, default=40000,
                     help="points per host core of the cpu_baseline sample (default: ~10 s of CPU work per core)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (esm and expected variance of every point "
+                         "of rank 0's grid, the (min, index) pair) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_cuda(args)

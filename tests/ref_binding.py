@@ -2,9 +2,9 @@
 a ctypes stub over the C-ABI of include/bq_b200.h and the three scoring loops of the reference's ``BQ`` class
 (bayesian_quadrature/bq.py:399-402, :420-422, :442-444) replaced by ONE library call each.
 
-``patch_reference(BQ)`` applies it to the reference's own class (oracle/_ref, test infrastructure) so that
-tests/test_gpu_reference_binding.py can run the reference's scoring tests through libbq_b200.so.  Nothing of
-bayesian_quadrature_b200's Python layer is used here: this file talks to the shared library only."""
+``patch_reference(BQ)`` applies it to a class with the reference ``BQ`` object's attributes (the reference's own class, or
+the state holder of tests/test_gpu_reference_binding.py, which runs the reference's scoring tests through libbq_b200.so).
+Nothing of bayesian_quadrature_b200's Python layer is used here: this file talks to the shared library only."""
 import ctypes
 import logging
 import os
