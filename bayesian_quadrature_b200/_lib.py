@@ -44,7 +44,10 @@ SYMBOLS = {
     "bqb_batch_info": (ctypes.c_int, [_vp, _dp, _dp, _dp, _ip, _dp]),
     "bqb_score_device": (ctypes.c_int, [_vp, _vp, _ll, ctypes.c_int, _vp, _vp, _vp, _ll, _vp, _vp]),
     "bqb_score_device_range": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, _ll, ctypes.c_int, _vp, _vp, _vp, _ll, _vp, _vp]),
+    "bqb_score_device_grouped": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, _ll, ctypes.c_int, ctypes.c_int, _vp, _vp, _vp, _ll,
+                                                _vp, _vp]),
     "bqb_sum_neg_accum_device": (ctypes.c_int, [_vp, _vp, _ll, ctypes.c_int, _ll, _vp, _vp]),
+    "bqb_sum_neg_accum_groups_device": (ctypes.c_int, [_vp, _vp, _ll, ctypes.c_int, ctypes.c_int, _ll, _vp, _ll, _vp]),
     "bqb_predict_device": (ctypes.c_int, [_vp, _vp, _ll, ctypes.c_int, _vp, _vp, _ll, _vp]),
     "bqb_predict_host": (ctypes.c_int, [_vp, _dp, _ll, ctypes.c_int, _dp, _dp]),
     "bqb_expected_var_host": (ctypes.c_int, [_vp, ctypes.c_int, _dp, ctypes.c_int, _dp, _ip]),
@@ -332,6 +335,28 @@ class Batch(object):
         _check(load().bqb_score_device_range(self._h, int(inst0), int(n_inst), _ptr(x_a), stride, na, _ptr(esm), _ptr(em),
                                              _ptr(status), out_stride, _ptr(flags), _vp(stream) if stream else None),
                "bqb_score_device_range")
+
+    def score_device_grouped(self, inst0, n_inst, x_a, xa_group, esm, em=None, status=None, flags=None, stream=None):
+        """score_device_range where instance inst0 + i reads row i // xa_group of x_a [n_inst / xa_group, na] (or the shared
+        [na]); inst0 must be a multiple of xa_group."""
+        if x_a.dim() == 1:
+            stride, na = 0, x_a.shape[0]
+        else:
+            stride, na = x_a.stride(0), x_a.shape[1]
+            if xa_group >= 1 and x_a.shape[0] < -(-int(n_inst) // int(xa_group)):
+                raise ValueError("x_a has %d rows; %d instances in groups of %d read %d" % (
+                    x_a.shape[0], n_inst, xa_group, -(-int(n_inst) // int(xa_group))))
+        out_stride = esm.stride(0) if esm.dim() == 2 else esm.shape[0]
+        _check(load().bqb_score_device_grouped(self._h, int(inst0), int(n_inst), _ptr(x_a), stride, int(xa_group), na, _ptr(esm),
+                                               _ptr(em), _ptr(status), out_stride, _ptr(flags), _vp(stream) if stream else None),
+               "bqb_score_device_grouped")
+
+    def sum_neg_accum_groups_device(self, esm, n_groups, group_size, acc, stream=None):
+        """acc[g] += sum over rows g*group_size ... (g+1)*group_size - 1 of -esm, in row order, for g < n_groups."""
+        acc_stride = acc.stride(0) if acc.dim() == 2 else acc.shape[0]
+        _check(load().bqb_sum_neg_accum_groups_device(self._h, _ptr(esm), esm.stride(0), int(n_groups), int(group_size), esm.shape[1],
+                                                      _ptr(acc), acc_stride, _vp(stream) if stream else None),
+               "bqb_sum_neg_accum_groups_device")
 
     def sum_neg_accum_device(self, esm, n_rows, acc, stream=None):
         """acc[p] += sum over the first n_rows rows of -esm[:, p], in row order (running form of mean_neg_device)."""

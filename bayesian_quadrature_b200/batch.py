@@ -2,7 +2,7 @@
 a batch of problems doing rounds of expected-variance active sampling, problems sharded across
 GPUs with no collective; SURVEY.md §8(e), §8(f).2).
 
-Per problem the semantics are those of the reference's ``BQ`` object under fixed hyper-parameters:
+Per problem the semantics are those of the reference's ``BQ`` object under the batch's hyper-parameters:
 ``init`` draws and filters candidates (bq.py:967-991), a round scores a query grid with
 ``expected_squared_mean`` (bq.py:379-402), picks the first minimiser of ``-esm`` (bq.py:660-663,
 deterministic mode), and ``add_observation`` merges or appends the new point and re-initialises
@@ -10,12 +10,26 @@ deterministic mode), and ``add_observation`` merges or appends the new point and
 problem has its own ``RandomState(seed + p)`` candidate stream (the reference uses one global
 RNG), and device arrays are padded to the batch's largest ``ns`` / ``nc``.
 
+``choose_next(x_a, n=...)`` marginalises over hyper-parameter samples like the reference's ``BQ.choose_next``
+(bq.py:659-681): ``sample_hypers`` slice-samples every problem's chain with one batched log-density evaluation per
+step (``log_lh``), and ``marginal_loss`` scores the P x S (problem, sample) instances in chunks of whole problems.  Chain p
+draws from its own counter-based stream keyed by the pair (seed, p) (the reference's single global libc ``rand`` stream
+cannot be split per problem; SURVEY appendix A.4 documents the same choice for the candidate streams).
+
 All per-problem bookkeeping is numpy-vectorised over the batch; scoring, the per-problem argmin
 and the model setup run on the device through the C-ABI.
 """
+import logging
+import time
+
 import numpy as np
 
 from . import _lib
+from . import util
+from .bq import _SETUP_ERRORS
+
+logger = logging.getLogger("bayesian_quadrature")
+_NAMES = ("h", "w", "s")                     # GaussianKernel parameters, then the noise: columns of one GP's (h, w, s)
 
 
 def filter_candidates_batch(x_c, x_s, ns, thresh):
@@ -100,6 +114,9 @@ class BatchBQ(object):
         if self.batch is not None:
             self.batch.close()
             self.batch = None
+        for b in getattr(self, "_sample_batches", {}).values():
+            b.close()
+        self._sample_batches = {}
 
     # ---------------------------------------------------------------- bq.py:132-171 / :967-991 per problem
     def _check_info(self, info):
@@ -182,11 +199,200 @@ class BatchBQ(object):
     def Z_var(self):
         return self.info["Z_var"]
 
+    # ---------------------------------------------------------------- hyper-parameter samples (bq.py:533-598)
+    def _hyp_rows(self, hypers_tl, hypers_l, params):
+        """[..., 6] hyper-parameter rows (h, w, s of gp_log_l, then of gp_l): the batch's own with the named entries
+        replaced by hypers_tl / hypers_l [P, ..., len(params)]."""
+        hypers_tl, hypers_l = np.asarray(hypers_tl, dtype=np.float64), np.asarray(hypers_l, dtype=np.float64)
+        k = len(params)
+        if hypers_tl.shape != hypers_l.shape or hypers_tl.shape[0] != self.P or hypers_tl.shape[-1] != k:
+            raise ValueError("hypers_tl and hypers_l must be [P, ..., %d] arrays of the same shape" % k)
+        mid = hypers_tl.shape[1:-1]
+        hyp = np.array(np.broadcast_to(self.hyp.reshape((self.P,) + (1,) * len(mid) + (6,)), (self.P,) + mid + (6,)))
+        for j, name in enumerate(params):
+            if name not in _NAMES:
+                raise ValueError("unknown hyper-parameter %r (BatchBQ has %s)" % (name, ", ".join(_NAMES)))
+            c = _NAMES.index(name)
+            hyp[..., c], hyp[..., 3 + c] = hypers_tl[..., j], hypers_l[..., j]
+        return hyp
+
+    @staticmethod
+    def _valid_hyp(hyp):
+        """The values GP.set_param accepts: finite, h and w positive, s non-negative."""
+        return (np.isfinite(hyp).all(axis=-1) & (hyp[..., [0, 1, 3, 4]] > 0).all(axis=-1)
+                & (hyp[..., [2, 5]] >= 0).all(axis=-1))
+
+    def log_lh(self, hypers_tl, hypers_l, params):
+        """Joint log marginal likelihood ``gp_log_l.log_lh + gp_l.log_lh`` of every problem under its own proposal
+        hypers_tl[p] / hypers_l[p] ([P, len(params)]): entry p is what the reference's ``_make_llh_params(params)``
+        (bq.py:533-552) returns for problem p -- l_c recomputed from the candidates, -inf for an invalid value, a Gram
+        matrix that is not positive definite or the "GP mean is too large" guard (bq.py:942-947); a log likelihood that
+        does not come out finite (a numerically singular Gram matrix) is -inf too, so that no chain of sample_hypers can
+        settle on it.
+
+        One setup of all P problems on the batch itself; the batch's own hyper-parameters are set up again afterwards
+        (the setup is deterministic, so the scoring model, Z_mean and Z_var are exactly what they were)."""
+        hyp = self._hyp_rows(hypers_tl, hypers_l, params)
+        ok = self._valid_hyp(hyp)
+        hyp[~ok] = self.hyp[~ok]                          # rows the device must not see; their result is -inf
+        try:
+            self.batch.set_hypers(hyp)
+            info = self.batch.setup_device(check_max=True)
+        finally:
+            self.batch.set_hypers(self.hyp)
+            self._check_info(self.batch.setup_device())
+        return np.where(ok & (info["status"] == _lib.SETUP_OK) & np.isfinite(info["log_lh"]), info["log_lh"], -np.inf)
+
+    def sample_hypers(self, params, n, nburn=10, seed=0, first_problem=0, max_steps=None, stats=None):
+        """Slice-sample the named hyper-parameters of both GPs of every problem (``BQ.sample_hypers``, bq.py:565-598):
+        one chain per problem, started at the batch's hyper-parameters with window 2 * len(params), n samples after
+        nburn.  Each sampler step is ONE ``log_lh`` evaluation of all problems.  Chain p draws from the counter stream
+        keyed by the pair (seed, first_problem + p) (``util.stream_keys``, ``util.slice_sample_batch``), so its samples do
+        not depend on the other problems of the batch; ``first_problem`` is the index of the batch's first problem in the
+        caller's numbering (a shard or a sub-batch then draws the streams the whole batch would).  ``max_steps`` /
+        ``stats``: see ``util.slice_sample_batch``.  Returns (hypers_tl, hypers_l), each [P, n, len(params)].  A problem
+        whose start has zero probability raises RuntimeError (the reference would search for better starting parameters
+        instead)."""
+        k = len(params)
+        cols = [_NAMES.index(p) if p in _NAMES else -1 for p in params]
+        if min(cols + [0]) < 0:
+            raise ValueError("unknown hyper-parameter in %s (BatchBQ has %s)" % (params, ", ".join(_NAMES)))
+        x0 = np.concatenate([self.hyp[:, cols], self.hyp[:, [3 + c for c in cols]]], axis=1)
+        f = lambda X: self.log_lh(X[:, :k], X[:, k:], params)
+        keys = util.stream_keys(seed, int(first_problem) + np.arange(self.P))
+        try:
+            s = util.slice_sample_batch(f, x0, n, 2 * k, keys, nburn=nburn, max_steps=max_steps, stats=stats)
+        except RuntimeError as e:
+            if getattr(e, "chain", None) is None:
+                raise
+            raise RuntimeError("problem %d: zero probability at the starting hyper-parameters" % e.chain) from e
+        return s[:, :, :k], s[:, :, k:]
+
+    #: device memory of the model blocks of one marginal_loss chunk (whole problems x samples)
+    MODEL_CHUNK_BYTES = 4 << 30
+    #: the [problems x samples, na] score buffer of one scoring launch (64 MB stays L2-resident on a B200, as BQ.LOSS_CHUNK_BYTES)
+    LOSS_CHUNK_BYTES = 64 << 20
+
+    def _sample_batch(self, n_inst):
+        """A device batch of n_inst (problem, sample) instances of the current capacity class, kept between calls."""
+        cache = self.__dict__.setdefault("_sample_batches", {})
+        for key in [k for k in cache if k[1] != self._cap_class]:
+            cache.pop(key).close()
+        key = (n_inst, self._cap_class)
+        if key not in cache:                              # (at most two sizes: full chunks and the last one)
+            cache[key] = _lib.Batch(n_inst, self._cap_class, device=self.device)
+        return cache[key]
+
+    def _chunks(self, S, na):
+        """(problems per setup chunk, problems per scoring launch) under MODEL_CHUNK_BYTES / LOSS_CHUNK_BYTES."""
+        model_bytes = 8 * _lib.load().bqb_model_doubles(self.batch._h)
+        per_score = max(1, min(self.P, self.LOSS_CHUNK_BYTES // max(8 * S * max(na, 1), 1)))
+        per_setup = max(1, min(self.P, self.MODEL_CHUNK_BYTES // (S * model_bytes)))
+        if per_setup >= per_score:
+            per_setup -= per_setup % per_score               # whole scoring launches per setup chunk
+        return per_setup, min(per_score, per_setup)
+
+    def _query(self, x_a):
+        import torch
+        dev = torch.device("cuda", self.device)
+        if isinstance(x_a, torch.Tensor):
+            return None, x_a.to(dev, torch.float64).contiguous()
+        x_a = np.ascontiguousarray(x_a, dtype=np.float64)
+        return x_a, torch.from_numpy(x_a).to(dev)
+
+    def marginal_loss(self, x_a, hypers_tl, hypers_l, params, timings=None):
+        """Marginal loss of choose_next for every problem: the mean over its S samples (hypers_tl / hypers_l
+        [P, S, len(params)]) of ``-expected_squared_mean(x_a)`` (bq.py:640-663), as a [P, na] CUDA tensor; row p is
+        ``BQ(problem p).marginal_loss(x_a, hypers_tl[p], hypers_l[p], params)``.  Each sample is set up with the semantics
+        of ``_set_gp_log_l_params`` / ``_set_gp_l_params`` (bq.py:933-965: l_c recomputed, "GP mean is too large" guard).
+        ``x_a`` is a shared grid [na] or per-problem grids [P, na] (numpy or a float64 CUDA tensor).
+
+        The P x S instances are set up in chunks of whole problems (MODEL_CHUNK_BYTES of model blocks) and scored in
+        launches of whole problems (LOSS_CHUNK_BYTES of scores): the S samples of a problem read its grid row
+        (``score_device_grouped``) and a segmented reduction adds their -esm in sample order, the additions of
+        ``values[0].mean(axis=0)``.
+        ``timings``, when a dict, receives the seconds spent in the three phases ("setup", "score", "reduce"; CUDA events
+        around each launch, which then synchronise after every scoring launch -- for measurements only)."""
+        import torch
+        hyp = self._hyp_rows(hypers_tl, hypers_l, params)
+        if hyp.ndim != 3:
+            raise ValueError("hypers_tl and hypers_l must be [P, S, %d]" % len(params))
+        S = hyp.shape[1]
+        if S < 1:
+            raise ValueError("at least one hyper-parameter sample per problem")
+        _, x_d = self._query(x_a)
+        if x_d.dim() not in (1, 2) or (x_d.dim() == 2 and x_d.shape[0] != self.P):
+            raise ValueError("x_a must be [na] or [P, na]")
+        na = x_d.shape[-1]
+        self.sync_host()
+        ok = self._valid_hyp(hyp)
+        if not ok.all():
+            p, i = np.argwhere(~ok)[0]
+            raise ValueError("invalid hyper-parameters %s in sample %d of problem %d" % (hyp[p, i], i, p))
+        stride = min(self.cap, self._cap_class)
+        per_setup, per_score = self._chunks(S, na)
+        dev = x_d.device
+        loss = torch.zeros(self.P, na, dtype=torch.float64, device=dev)
+        if na == 0:
+            return loss
+        esm = torch.empty(per_score * S, na, dtype=torch.float64, device=dev)
+        flags = torch.zeros(per_score * S, dtype=torch.int32, device=dev)
+        bad_esm = torch.zeros(self.P, dtype=torch.bool, device=dev)
+        bad_xa = torch.zeros(self.P, dtype=torch.bool, device=dev)
+        for p0 in range(0, self.P, per_setup):
+            cp = min(per_setup, self.P - p0)
+            rep = lambda a: np.repeat(a[p0:p0 + cp], S, axis=0)
+            batch = self._sample_batch(cp * S)
+            t0 = time.perf_counter()
+            info = batch.setup(rep(self.ns), rep(self.nc), rep(self.x_s[:, :stride]), rep(self.l_s[:, :stride]), rep(self.x_c),
+                               hyp[p0:p0 + cp].reshape(cp * S, 6), rep(self.prior), check_max=True)
+            bad = np.nonzero(info["status"])[0]
+            if bad.size:
+                p, i = divmod(int(bad[0]), S)
+                logger.error("error with parameters %s", hyp[p0 + p, i])
+                exc, msg = _SETUP_ERRORS.get(int(info["status"][bad[0]]), (RuntimeError, "device setup failed"))
+                raise exc("%s (problem %d, sample %d)" % (msg, p0 + p, i))
+            if timings is not None:
+                timings["setup"] = timings.get("setup", 0.0) + time.perf_counter() - t0     # setup synchronises
+            for q0 in range(0, cp, per_score):
+                cq = min(per_score, cp - q0)
+                rows = x_d if x_d.dim() == 1 else x_d[p0 + q0:p0 + q0 + cq]
+                ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)] if timings is not None else None
+                if ev:
+                    ev[0].record()
+                batch.score_device_grouped(q0 * S, cq * S, rows, S, esm, None, None, flags)
+                if ev:
+                    ev[1].record()
+                batch.sum_neg_accum_groups_device(esm, cq, S, loss[p0 + q0:p0 + q0 + cq])
+                if ev:
+                    ev[2].record()
+                    ev[2].synchronize()
+                    timings["score"] = timings.get("score", 0.0) + ev[0].elapsed_time(ev[1]) / 1e3
+                    timings["reduce"] = timings.get("reduce", 0.0) + ev[1].elapsed_time(ev[2]) / 1e3
+                fl = flags[:cq * S].view(cq, S)
+                bad_esm[p0 + q0:p0 + q0 + cq] |= ((fl & (_lib.ST_ESM_BAD | _lib.ST_EM_BAD)) != 0).any(dim=1)
+                bad_xa[p0 + q0:p0 + q0 + cq] |= ((fl & _lib.ST_XA_BAD) != 0).any(dim=1)
+        loss /= S                                         # bq.py:662
+        if bool(bad_xa.any().item()):
+            raise ValueError("invalid value in x_a of problem %d" % int(torch.nonzero(bad_xa)[0, 0].item()))
+        if bool(bad_esm.any().item()):
+            raise RuntimeError("invalid expected squared mean under a sampled hyper-parameter set of problem %d"
+                               % int(torch.nonzero(bad_esm)[0, 0].item()))
+        return loss
+
     # ---------------------------------------------------------------- one active-sampling round
-    def choose_next(self, x_a, on_device=False):
+    def choose_next(self, x_a, on_device=False, n=None, params=None, hypers=None, seed=None, max_steps=None):
         """Deterministic choose_next of every problem over a shared grid ``x_a`` [na] or per-problem grids
         [P, na]: index and location of the first maximiser of expected_squared_mean.  ``x_a`` may be a float64
-        CUDA tensor (it is then not uploaded again); with ``on_device=True`` the result is a pair of CUDA tensors."""
+        CUDA tensor (it is then not uploaded again); with ``on_device=True`` the result is a pair of CUDA tensors.
+
+        With ``n`` (and ``params``), the loss is marginalised over hyper-parameter samples like the reference's
+        ``BQ.choose_next(x_a, n, params)`` (bq.py:659-681): ``sample_hypers(params, n, nburn=1, seed, max_steps)`` draws
+        them, or ``hypers=(hypers_tl, hypers_l)`` ([P, S, len(params)]) gives them; the choice is the first minimiser of
+        each problem's ``marginal_loss``.  Without ``seed``, the r-th sampling round of this batch uses the seed
+        ``util.stream_keys(batch seed, r)``: every round draws fresh streams, as the reference's global stream advances."""
+        if n is not None or hypers is not None:
+            return self._choose_marginal(x_a, on_device, n, params, hypers, seed, max_steps)
         import torch
         dev = torch.device("cuda", self.device)
         if isinstance(x_a, torch.Tensor):
@@ -212,6 +418,30 @@ class BatchBQ(object):
             x_next = x_d[self._idxs] if x_d.dim() == 1 else x_d.gather(1, self._idxs[:, None])[:, 0]
             return self._idxs, x_next
         idx = self._idxs.cpu().numpy()
+        if x_a is None:
+            x_a = x_d.cpu().numpy()
+        x_next = x_a[idx] if x_a.ndim == 1 else x_a[np.arange(self.P), idx]
+        return idx, x_next
+
+    def _choose_marginal(self, x_a, on_device, n, params, hypers, seed, max_steps):
+        import torch
+        if params is None:
+            raise ValueError("params names the sampled hyper-parameters")
+        if hypers is None:
+            if seed is None:
+                r = self.__dict__.get("_sample_rounds", 0)
+                self._sample_rounds = r + 1
+                seed = int(util.stream_keys(self.seed, r))
+            hypers = self.sample_hypers(params, n, nburn=1, seed=seed, max_steps=max_steps)
+        x_a, x_d = self._query(x_a)
+        loss = self.marginal_loss(x_d, hypers[0], hypers[1], params)
+        mins = torch.empty(self.P, dtype=torch.float64, device=x_d.device)
+        idxs = torch.empty(self.P, dtype=torch.int64, device=x_d.device)
+        self.batch.argmin_rows_device(loss, mins, idxs)
+        if on_device:
+            x_next = x_d[idxs] if x_d.dim() == 1 else x_d.gather(1, idxs[:, None])[:, 0]
+            return idxs, x_next
+        idx = idxs.cpu().numpy()
         if x_a is None:
             x_a = x_d.cpu().numpy()
         x_next = x_a[idx] if x_a.ndim == 1 else x_a[np.arange(self.P), idx]

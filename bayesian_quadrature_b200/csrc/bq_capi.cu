@@ -23,6 +23,8 @@ cudaError_t launch_argmin_partials(double *bv, long long *bi, int nblocks, long 
 cudaError_t launch_mean_neg(const double *esm, long long stride, int n_inst, long long na, double *loss, cudaStream_t s);
 cudaError_t launch_pack_info(const double *models, long long model_stride, int off_lc, int n_inst, double *out, cudaStream_t s);
 cudaError_t launch_sum_neg_accum(const double *esm, long long stride, int n_rows, long long na, double *acc, cudaStream_t s);
+cudaError_t launch_sum_neg_groups(const double *esm, long long stride, int n_groups, int group_size, long long na, double *acc,
+                                  long long acc_stride, cudaStream_t s);
 cudaError_t launch_expected_var(const double *esm, long long na, double msm, double *out, cudaStream_t s);
 cudaError_t launch_argmin(const double *v, long long n, double *scratch_val, long long *scratch_idx, int sm_count,
                           cudaStream_t s);
@@ -477,7 +479,7 @@ static int check_ready(bqb_batch *b, const char *who) {
 
 static int score_device_impl(bqb_batch *b, const double *d_x_a, long long xa_stride, int na, double *d_esm, double *d_em,
                              int *d_status, long long out_stride, int *d_flags, const int *d_perm, void *stream, int first = 0,
-                             int count = -1);
+                             int count = -1, int xa_group = 1);
 
 int bqb_score_device(bqb_batch *b, const double *d_x_a, long long xa_stride, int na, double *d_esm, double *d_em,
                      int *d_status, long long out_stride, int *d_flags, void *stream) {
@@ -488,6 +490,14 @@ int bqb_score_device_range(bqb_batch *b, int inst0, int n_inst, const double *d_
                            double *d_em, int *d_status, long long out_stride, int *d_flags, void *stream) {
     if (!b || inst0 < 0 || n_inst < 1 || inst0 + n_inst > b->n_inst) return fail(BQB_EINVAL, "bqb_score_device_range: bad instance range");
     return score_device_impl(b, d_x_a, xa_stride, na, d_esm, d_em, d_status, out_stride, d_flags, nullptr, stream, inst0, n_inst);
+}
+
+int bqb_score_device_grouped(bqb_batch *b, int inst0, int n_inst, const double *d_x_a, long long xa_stride, int xa_group, int na,
+                             double *d_esm, double *d_em, int *d_status, long long out_stride, int *d_flags, void *stream) {
+    if (!b || inst0 < 0 || n_inst < 1 || inst0 + n_inst > b->n_inst) return fail(BQB_EINVAL, "bqb_score_device_grouped: bad instance range");
+    if (xa_group < 1 || inst0 % xa_group) return fail(BQB_EINVAL, "bqb_score_device_grouped: inst0 must be a multiple of xa_group >= 1");
+    return score_device_impl(b, d_x_a, xa_stride, na, d_esm, d_em, d_status, out_stride, d_flags, nullptr, stream, inst0, n_inst,
+                             xa_group);
 }
 
 // A query vector "looks sorted" if ~2000 evenly spaced samples are ascending at stride 1 and at the sampling stride.
@@ -536,7 +546,8 @@ static bool want_presort(const bqb_batch *b, const double *x, int n) {
 // Instances [first, first + count) (count < 0: all).  The per-instance rows of x_a / esm / em / status / flags are relative
 // to `first` (row 0 belongs to instance `first`), so a caller can walk a large batch through one chunk-sized buffer.
 static int score_device_impl(bqb_batch *b, const double *d_x_a, long long xa_stride, int na, double *d_esm, double *d_em,
-                             int *d_status, long long out_stride, int *d_flags, const int *d_perm, void *stream, int first, int count) {
+                             int *d_status, long long out_stride, int *d_flags, const int *d_perm, void *stream, int first, int count,
+                             int xa_group) {
     int rc = check_ready(b, "bqb_score_device");
     if (rc) return rc;
     if (!d_x_a || !d_esm || na < 0 || out_stride < na) return fail(BQB_EINVAL, "bqb_score_device: bad arguments");
@@ -545,7 +556,8 @@ static int score_device_impl(bqb_batch *b, const double *d_x_a, long long xa_str
     CU(cudaSetDevice(b->device));
     ScoreArgs a;
     a.cut_arg = b->cut_arg; a.work = b->d_work_ctr; a.nb_max = b->nb_max; a.nrow_max = b->nrow_max;
-    a.models = b->d_models; a.lay = b->lay; a.x_a = d_x_a - (size_t)first * xa_stride; a.xa_stride = xa_stride; a.na = na;
+    a.models = b->d_models; a.lay = b->lay; a.x_a = d_x_a - (size_t)(first / xa_group) * xa_stride; a.xa_stride = xa_stride;
+    a.xa_group = xa_group; a.na = na;
     a.esm = d_esm - (size_t)first * out_stride; a.em = d_em ? d_em - (size_t)first * out_stride : nullptr;
     a.status = d_status ? d_status - (size_t)first * out_stride : nullptr; a.out_stride = out_stride; a.exp_tab = b->d_tab;
     a.flags = d_flags ? d_flags - first : nullptr; a.ndb_max = b->ndb_max; a.perm = d_perm;
@@ -755,6 +767,18 @@ int bqb_sum_neg_accum_device(bqb_batch *b, const double *d_esm, long long stride
     if (na == 0 || n_rows == 0) return 0;
     CU(cudaSetDevice(b->device));
     CU(launch_sum_neg_accum(d_esm, stride, n_rows, na, d_acc, (cudaStream_t)stream));
+    b->launches++;
+    return 0;
+}
+
+int bqb_sum_neg_accum_groups_device(bqb_batch *b, const double *d_esm, long long stride, int n_groups, int group_size, long long na,
+                                    double *d_acc, long long acc_stride, void *stream) {
+    if (!b || na < 0 || n_groups < 0 || group_size < 0) return fail(BQB_EINVAL, "bqb_sum_neg_accum_groups_device: bad arguments");
+    if (na == 0 || n_groups == 0 || group_size == 0) return 0;                  // nothing is read or written
+    if (!d_esm || !d_acc || stride < na || (n_groups > 1 && acc_stride < na))
+        return fail(BQB_EINVAL, "bqb_sum_neg_accum_groups_device: bad arguments");
+    CU(cudaSetDevice(b->device));
+    CU(launch_sum_neg_groups(d_esm, stride, n_groups, group_size, na, d_acc, acc_stride, (cudaStream_t)stream));
     b->launches++;
     return 0;
 }

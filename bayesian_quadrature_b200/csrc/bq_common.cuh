@@ -84,8 +84,9 @@ __host__ __device__ inline Layout make_layout(int nsp_cap) {
 struct ScoreArgs {
     const double *models = nullptr;     // [B][lay.total]
     Layout lay;
-    const double *x_a = nullptr;        // [na] (xa_stride = 0) or [B][xa_stride]
+    const double *x_a = nullptr;        // [na] (xa_stride = 0) or [B / xa_group][xa_stride]
     long long xa_stride = 0;
+    int xa_group = 1;                   // instance inst reads query row inst / xa_group (samples of one problem share a grid)
     int na = 0;
     double *esm = nullptr, *em = nullptr;   // [B][out_stride]; em may be null (esm too when ev is given)
     int *status = nullptr;              // [B][out_stride]; may be null

@@ -26,6 +26,23 @@ __global__ void sum_neg_accum_kernel(const double *__restrict__ esm, long long s
     }
 }
 
+// Segmented form for many problems with S samples each: acc[g][p] += -esm[g*S][p] - esm[g*S+1][p] - ... in row order.  Per group
+// these are the additions of sum_neg_accum_kernel, so one group reproduces it bit for bit and a problem's samples may arrive
+// in chunks.  HBM-bound: every esm element is read once, acc is read and written once per launch.
+__global__ void sum_neg_groups_kernel(const double *__restrict__ esm, long long stride, int n_groups, int group_size, long long na,
+                                      double *__restrict__ acc, long long acc_stride) {
+    for (int g = blockIdx.y; g < n_groups; g += gridDim.y) {
+        const double *e = esm + (size_t)g * group_size * stride;
+        double *a = acc + (size_t)g * acc_stride;
+        for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < na; p += (long long)gridDim.x * blockDim.x) {
+            double s = a[p];
+#pragma unroll 4
+            for (int r = 0; r < group_size; ++r) s += -e[(size_t)r * stride + p];
+            a[p] = s;
+        }
+    }
+}
+
 __global__ void expected_var_kernel(const double *__restrict__ esm, long long na, double msm, double *__restrict__ out) {
     for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < na; p += (long long)gridDim.x * blockDim.x)
         out[p] = msm - esm[p];
@@ -128,6 +145,14 @@ cudaError_t launch_mean_neg(const double *esm, long long stride, int n_inst, lon
 cudaError_t launch_sum_neg_accum(const double *esm, long long stride, int n_rows, long long na, double *acc, cudaStream_t s) {
     const int blocks = (int)((na + 255) / 256 < 2368 ? (na + 255) / 256 : 2368);
     sum_neg_accum_kernel<<<blocks > 0 ? blocks : 1, 256, 0, s>>>(esm, stride, n_rows, na, acc);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_sum_neg_groups(const double *esm, long long stride, int n_groups, int group_size, long long na, double *acc,
+                                  long long acc_stride, cudaStream_t s) {
+    const int bx = (int)((na + 255) / 256 < 2368 ? (na + 255) / 256 : 2368);
+    const int by = n_groups < 65535 ? n_groups : 65535;
+    sum_neg_groups_kernel<<<dim3(bx > 0 ? bx : 1, by > 0 ? by : 1), 256, 0, s>>>(esm, stride, n_groups, group_size, na, acc, acc_stride);
     return cudaGetLastError();
 }
 

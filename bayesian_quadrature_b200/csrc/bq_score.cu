@@ -823,7 +823,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) bq_score_kernel(ScoreArgs a)
     const int tol2_hi = __double2hiint(s_small[H_TOL2MAX]) + 1;
     double *scr = s_scr + warp * SM::scr(nrow_res);        // rows: 0 qs, 1 qt, 2 tm, 3 isclose, 4.. dense rows, then x_a
 
-    const double *xa = a.x_a + (size_t)inst * a.xa_stride;
+    const double *xa = a.x_a + (size_t)(inst / a.xa_group) * a.xa_stride;
     double *o_esm = a.esm ? a.esm + (size_t)inst * a.out_stride : nullptr;   // optional when the fused epilogue writes ev
     double *o_em = a.em ? a.em + (size_t)inst * a.out_stride : nullptr;
     int *o_st = a.status ? a.status + (size_t)inst * a.out_stride : nullptr;

@@ -56,7 +56,7 @@ __global__ void __launch_bounds__(GEN_THREADS * GEN_WARPS) bq_score_generic_kern
     const double Zm = M[H_ZM];
     const double *xs = M + lay.off_xs, *tol = M + lay.off_tol, *atl = M + lay.off_atl, *xc = M + lay.off_xc;
     const double *Fl = M + lay.off_af_l_tri, *Fd = M + lay.off_af_l_dense, *Ft = M + lay.off_af_tl_tri;
-    const double *xa = a.x_a + (size_t)inst * a.xa_stride;
+    const double *xa = a.x_a + (size_t)(inst / a.xa_group) * a.xa_stride;
     double *o_esm = a.esm ? a.esm + (size_t)inst * a.out_stride : nullptr;
     double *o_em = a.em ? a.em + (size_t)inst * a.out_stride : nullptr;
     int *o_st = a.status ? a.status + (size_t)inst * a.out_stride : nullptr;

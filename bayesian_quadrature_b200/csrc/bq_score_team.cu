@@ -204,7 +204,7 @@ __global__ void __launch_bounds__(TEAMS *TW * 32, 1) bq_score_team_kernel(ScoreA
     const int tol2_hi = __double2hiint(s_small[H_TOL2MAX]) + 1;
     unsigned long long n_dmma = 0;
 
-    const double *xa = a.x_a + (size_t)inst * a.xa_stride;
+    const double *xa = a.x_a + (size_t)(inst / a.xa_group) * a.xa_stride;
     double *o_esm = a.esm ? a.esm + (size_t)inst * a.out_stride : nullptr;
     double *o_em = a.em ? a.em + (size_t)inst * a.out_stride : nullptr;
     int *o_st = a.status ? a.status + (size_t)inst * a.out_stride : nullptr;

@@ -98,6 +98,150 @@ def slice_sample(logpdf, niter, w, xval, nburn=1, freq=1):
     return samples[nburn:][::freq]
 
 
+def _splitmix64(z):
+    with np.errstate(over="ignore"):                     # arithmetic modulo 2^64 is the hash
+        z = z + np.uint64(0x9E3779B97F4A7C15)
+        z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+        z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+        return z ^ (z >> np.uint64(31))
+
+
+def counter_uniform(keys, counters):
+    """Uniform doubles in [0, 1), one per (stream key, draw counter) pair (integer arrays of one shape): a splitmix64
+    hash of the key, mixed with the counter and hashed again, keeps its top 53 bits.  A stream is a pure function of its
+    key, so that many chains can draw from their own streams in any interleaving."""
+    z = _splitmix64(_splitmix64(_u64(keys)) ^ _u64(counters))
+    return (z >> np.uint64(11)).astype(DTYPE) * (1.0 / 9007199254740992.0)
+
+
+def _u64(v):
+    """Integers as uint64 words (negative values wrap modulo 2^64)."""
+    v = np.asarray(v)
+    return v.astype(np.uint64) if v.dtype.kind == "u" else v.astype(np.int64).astype(np.uint64)
+
+
+def stream_keys(seed, problems):
+    """Stream keys of problems ``problems`` under ``seed``: seed and problem index are hashed as separate words
+    (splitmix64(splitmix64(seed) ^ p)), so that no (seed, p) pair shares the stream of another."""
+    return _splitmix64(_splitmix64(_u64(np.full(np.shape(problems), seed))) ^ _u64(problems))
+
+
+_START, _NEW, _LEFT, _RIGHT, _SHRINK, _DONE = range(6)
+
+
+def slice_sample_batch(logpdf, x0, n, w, keys, nburn=1, max_steps=None, stats=None):
+    """``slice_sample`` for many independent chains advanced in lock-step: chain p starts at x0[p] and returns
+    ``samples[nburn:]`` of nburn + n iterations, i.e. an array [P, n, d].
+
+    ``logpdf(X)`` takes the [P, d] points of all chains and returns their [P] log densities; it is called once per step,
+    where every unfinished chain has exactly one point to evaluate (finished chains pass their last sample).  Per chain the
+    algorithm is that of ``slice_sample``: a random unit direction, stepping-out of at most 101 steps per side, shrinkage,
+    and a retry of the iteration when the window collapses below 1e-9.  The density of the current point is the one
+    computed when it was accepted (``slice_sample`` evaluates it again, to the same value).  The slice height is
+    drawn as ``height + log(u)``: ``slice_sample``'s ``log(u * exp(height))`` is infinite, and the chain stuck, once a
+    joint log likelihood exceeds 709.
+
+    Chain p draws from the counter stream ``counter_uniform(keys[p], 0, 1, 2, ...)``: per iteration one draw for the slice
+    height, d for the direction (each minus 0.5, then normalised), one per shrinkage proposal.  Its samples therefore depend
+    only on its key, its start and its own densities.  (``slice_sample`` shares the global libc and numpy streams instead.)
+    A start of density -inf raises RuntimeError naming the chain.
+
+    The chains advance in lock-step, so the slowest one sets the number of steps.  ``max_steps`` (default: no limit)
+    caps the ``logpdf`` calls of this run: a chain that has not finished by then stays at its last accepted point for
+    the samples it still owes (a shorter chain, not a different algorithm).  ``stats``, when a dict, receives "steps" (the
+    ``logpdf`` calls made) and "unfinished" (the indices of the chains the cap stopped)."""
+    x0 = np.array(x0, dtype=DTYPE, ndmin=2)
+    P, d = x0.shape
+    keys = _u64(keys).reshape(P)
+    if max_steps is not None and max_steps < 1:
+        raise ValueError("max_steps must be at least 1")
+    n_calls = 0
+    niter = nburn + int(n)
+    samples = np.empty((P, niter, d))
+    samples[:, 0] = x0
+    rows = np.arange(P)
+    it = np.zeros(P, dtype=np.int64)                     # index of the current point in samples
+    ctr = np.zeros(P, dtype=np.uint64)
+    phase = np.full(P, _START if niter > 1 else _DONE)
+    height, logy, left, right, loc = (np.zeros(P) for _ in range(5))
+    direction = np.zeros((P, d))
+    steps = np.zeros(P, dtype=np.int64)
+
+    def draw(sel, k):
+        c = ctr[sel][:, None] + np.arange(k, dtype=np.uint64)[None, :]
+        ctr[sel] += np.uint64(k)
+        return counter_uniform(np.broadcast_to(keys[sel][:, None], c.shape), c)
+
+    def begin(sel):                                      # a new iteration from the current point
+        u = draw(sel, 1)[:, 0]
+        with np.errstate(divide="ignore"):
+            logy[sel] = height[sel] + np.log(u)           # log(u * exp(height)) without the overflow of exp above 709
+        dv = draw(sel, d) - 0.5
+        nrm = dv[:, 0] * dv[:, 0]
+        for c in range(1, d):
+            nrm += dv[:, c] * dv[:, c]
+        direction[sel] = dv / np.sqrt(nrm)[:, None]
+        left[sel], right[sel], steps[sel] = -w, w, 0
+        phase[sel] = _LEFT
+
+    while True:
+        if (phase == _NEW).any():
+            begin(phase == _NEW)
+        collapsed = (phase == _SHRINK) & ((right - left) < 1e-9)
+        if collapsed.any():
+            begin(collapsed)
+        shrink = phase == _SHRINK
+        if shrink.any():
+            loc[shrink] = draw(shrink, 1)[:, 0] * (right[shrink] - left[shrink]) + left[shrink]
+        if (phase == _DONE).all():
+            break
+        if max_steps is not None and n_calls >= max_steps:
+            for p in np.nonzero(phase != _DONE)[0]:
+                samples[p, it[p] + 1:] = samples[p, it[p]]
+            break
+        cur = samples[rows, it]
+        off = np.select([phase == _LEFT, phase == _RIGHT, phase == _SHRINK], [left, right, loc], 0.0)
+        move = (phase == _LEFT) | (phase == _RIGHT) | (phase == _SHRINK)
+        pts = np.where(move[:, None], cur + off[:, None] * direction, cur)
+        f = np.asarray(logpdf(pts), dtype=DTYPE).reshape(P)
+        n_calls += 1
+        ph = phase.copy()
+
+        sel = ph == _START
+        if sel.any():
+            bad = sel & (f == -np.inf)
+            if bad.any():
+                err = RuntimeError("zero probability encountered at the start of chain %d" % int(np.argmax(bad)))
+                err.chain = int(np.argmax(bad))
+                raise err
+            height[sel] = f[sel]
+            phase[sel] = _NEW
+        for side, sign, nxt in ((_LEFT, -1.0, _RIGHT), (_RIGHT, 1.0, _SHRINK)):
+            sel = ph == side
+            if sel.any():
+                up = sel & (f >= logy)
+                bound = left if side == _LEFT else right
+                bound[up] += sign * w
+                steps[up] += 1
+                out = sel & (~up | (steps > 100))
+                phase[out], steps[out] = nxt, 0
+        sel = ph == _SHRINK
+        if sel.any():
+            acc = sel & (f > logy)
+            it[acc] += 1
+            samples[rows[acc], it[acc]] = pts[acc]
+            height[acc] = f[acc]
+            phase[acc] = np.where(it[acc] == niter - 1, _DONE, _NEW)
+            rej = sel & ~acc
+            neg = rej & (loc < 0)
+            left[neg] = loc[neg]
+            pos = rej & ~(loc < 0)
+            right[pos] = loc[pos]
+    if stats is not None:
+        stats["steps"], stats["unfinished"] = n_calls, np.nonzero(phase != _DONE)[0]
+    return samples[:, nburn:]
+
+
 def find_good_parameters(logpdf, x0, method, ntry=10):
     """Maximise `logpdf` with scipy (util.py:151-169): up to `ntry` restarts, returns None when no
     restart reaches a log-density above MIN."""

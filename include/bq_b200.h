@@ -156,6 +156,13 @@ int bqb_score_host(bqb_batch *b, const double *x_a, long long xa_stride, int na,
 int bqb_score_device_range(bqb_batch *b, int inst0, int n_inst, const double *d_x_a, long long xa_stride, int na, double *d_esm,
                            double *d_em, int *d_status, long long out_stride, int *d_flags, void *stream);
 
+/* bqb_score_device_range where xa_group consecutive instances share one query row: instance i reads row
+ * (i - inst0) / xa_group of x_a (when xa_stride != 0).  The S hyper-parameter samples of a problem (bq.py:640-652) are scored
+ * against that problem's grid without replicating it S times.  inst0 must be a multiple of xa_group (BQB_EINVAL otherwise),
+ * so that a chunk starts on a problem boundary; esm / em / status / d_flags keep one row per instance.  Never sorts x_a. */
+int bqb_score_device_grouped(bqb_batch *b, int inst0, int n_inst, const double *d_x_a, long long xa_stride, int xa_group, int na,
+                             double *d_esm, double *d_em, int *d_status, long long out_stride, int *d_flags, void *stream);
+
 /* Batched prediction at na points for every instance (SURVEY.md §8(f).4): l_mean = gp_l.mean(x), the mean of the final
  * approximation (BQ.l_mean, bq.py:177-200), and v_log_l = diag gp_log_l.cov(x), from which BQ.l_var (bq.py:202-231) is
  * max(v_log_l * l_mean^2, 0).  Same layout conventions as bqb_score_*; requires s_l = 0 (the scoring factors are those
@@ -184,6 +191,13 @@ int bqb_mean_neg_device(bqb_batch *b, const double *d_esm, long long stride, lon
  * the partial sum a rank contributes when the samples are sharded across GPUs (all-reduce, then divide). */
 int bqb_sum_neg_accum_device(bqb_batch *b, const double *d_esm, long long stride, int n_rows, long long na, double *d_acc,
                              void *stream);
+
+/* Segmented bqb_sum_neg_accum_device over n_groups groups of group_size consecutive rows of esm:
+ * d_acc[g][p] += -esm[g*group_size][p] - esm[g*group_size+1][p] - ... in row order (row g of d_acc at g * acc_stride).  Each
+ * group performs the additions of bqb_sum_neg_accum_device, so that dividing by the number of samples gives every problem's
+ * values[0].mean(axis=0) of bq.py:640-663 when the rows of a group are its hyper-parameter samples.  DEVICE pointers. */
+int bqb_sum_neg_accum_groups_device(bqb_batch *b, const double *d_esm, long long stride, int n_groups, int group_size, long long na,
+                                    double *d_acc, long long acc_stride, void *stream);
 
 /* Deterministic minimum of a DEVICE vector and the FIRST index attaining it (np.min / np.argmin of
  * bq.py:663).  Results are written to HOST scalars; synchronises `stream`. */
