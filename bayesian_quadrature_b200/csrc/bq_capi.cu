@@ -14,9 +14,9 @@
 #include "bq_common.cuh"
 
 namespace bqb {
-void launch_setup(const SetupArgs &a, int n_inst, cudaStream_t stream);
 cudaError_t launch_setup2(const SetupArgs &a, int n_inst, cudaStream_t stream);
 int setup2_two_cta_limit(int nc_max);
+size_t setup2_scratch_stride(int cap);
 cudaError_t launch_score(const ScoreArgs &a, int n_inst, int sm_count, cudaStream_t stream, int *grid_x = nullptr);
 cudaError_t launch_score_generic(const ScoreArgs &a, int n_inst, cudaStream_t stream, int *grid_x);
 cudaError_t launch_argmin_partials(double *bv, long long *bi, int nblocks, long long offset, double *pair, cudaStream_t s);
@@ -52,7 +52,7 @@ struct bqb_batch {
     int device, n_inst, ns_cap, sm_count;
     Layout lay;
     double *d_models = nullptr, *d_tab = nullptr, *d_work = nullptr;
-    int work_inst = 0, n_cap = 0;
+    int work_inst = 0;
     size_t work_stride = 0;
     // staged inputs: x_s / l_s rows have the device stride ns_cap, so that observations can be appended in place
     int *d_ns = nullptr, *d_nc = nullptr;
@@ -66,7 +66,7 @@ struct bqb_batch {
     int kind = 0, n_xo = 0;
     long long xo_stride = 0;
     bool generic = false;
-    bool big_class = false;            // capacity 512: no tensor-core scoring kernels, no first-generation setup kernel
+    bool big_class = false;            // capacity 512: no tensor-core scoring kernels
     double *d_period = nullptr, *d_xo = nullptr, *d_pxo = nullptr, *d_wp = nullptr, *d_gz = nullptr;
     int *d_inst_list = nullptr;        // setup launch groups (instances ordered by size class)
     // scoring: relevance cut-off (bq_score.cu, CUT_ARG; +inf = dense) and the optional executed-work counter
@@ -141,19 +141,17 @@ int bqb_batch_create(bqb_batch **out, int device, int n_inst, int ns_max) {
     for (int j = 0; j < 2048; ++j) tab[j] = (double)exp2l((long double)j / 2048);
     for (int j = 0; j < 512; ++j) tab[2048 + j] = (double)exp2l((long double)j / 512);
     CU(cudaMemcpy(b->d_tab, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice));
-    // leading dimension of the setup scratch matrices: sized for the capacity CLASS, because bqb_batch_stage and
-    // bqb_batch_add_observations let ns grow up to bqb_batch_capacity(), not just up to ns_max
-    b->n_cap = cap + NC_MAX;
-    b->work_stride = 4 * (size_t)b->n_cap * b->n_cap + 32 * (size_t)b->n_cap;
     b->work_inst = n_inst < 2048 ? n_inst : 2048;
     if (cap > 256) {
-        // 257 .. 512 observations: second-generation setup kernel with its packed triangle in this scratch, generic scoring
+        // 257 .. 512 observations: generic scoring
         b->big_class = true;
         b->generic = true;
-        b->work_stride = ((size_t)b->n_cap * (b->n_cap + 1) / 2 + 64) & ~(size_t)1;
         if (b->work_inst > 256) b->work_inst = 256;
     }
-    CU(cudaMalloc(&b->d_work, sizeof(double) * b->work_stride * b->work_inst));
+    // setup scratch sized for the capacity CLASS, because bqb_batch_stage and bqb_batch_add_observations let ns grow up
+    // to bqb_batch_capacity(), not just up to ns_max
+    b->work_stride = setup2_scratch_stride(cap);
+    if (b->work_stride) CU(cudaMalloc(&b->d_work, sizeof(double) * b->work_stride * b->work_inst));
     CU(cudaMalloc(&b->d_ns, sizeof(int) * n_inst));
     CU(cudaMalloc(&b->d_nc, sizeof(int) * n_inst));
     CU(cudaMalloc(&b->d_xs, sizeof(double) * (size_t)n_inst * cap));
@@ -195,8 +193,8 @@ static int run_setup(bqb_batch *b, int check_max, cudaStream_t s) {
     SetupArgs a;
     a.ns = b->d_ns; a.nc = b->d_nc; a.x_s = b->d_xs; a.l_s = b->d_ls; a.x_c = b->d_xc; a.hyp = b->d_hyp; a.prior = b->d_prior;
     a.in_stride = b->ns_cap; a.check_max = check_max; a.models = b->d_models; a.lay = b->lay;
-    a.work = b->d_work; a.work_stride = b->work_stride; a.n_cap = b->n_cap;
-    // counts on the host before the launch (they size the second-generation kernel's shared memory); the device-side
+    a.work = b->d_work; a.work_stride = b->work_stride;
+    // counts on the host before the launch (they size the setup kernel's shared memory); the device-side
     // round kernels (add_observations, draw_candidates) change them without the host seeing it
     if (!b->counts_fresh) {
         CU(cudaMemcpyAsync(b->h_ns.data(), b->d_ns, sizeof(int) * B, cudaMemcpyDeviceToHost, s));
@@ -204,7 +202,6 @@ static int run_setup(bqb_batch *b, int check_max, cudaStream_t s) {
         CU(cudaStreamSynchronize(s));
         b->counts_fresh = true;
     }
-    static const bool v1 = getenv("BQB_SETUP_V1") && atoi(getenv("BQB_SETUP_V1"));
     int n_max = 8, nc_max = 1;
     for (int i = 0; i < B; ++i) {
         const int ns_i = b->h_ns[i], nc_i = b->h_nc[i];
@@ -215,15 +212,13 @@ static int run_setup(bqb_batch *b, int check_max, cudaStream_t s) {
     a.n_max = n_max; a.nc_max = nc_max;
     a.kind = b->kind; a.period = b->d_period; a.xo = b->d_xo; a.pxo = b->d_pxo; a.n_xo = b->n_xo; a.xo_stride = b->xo_stride;
     a.wp = b->d_wp; a.gz = b->d_gz;
-    if (v1 && (b->kind || b->n_xo || b->big_class))
-        return fail(BQB_EUNSUPPORTED, "BQB_SETUP_V1: the first-generation setup kernel has no periodic kernel / trapezoid mode and ends at 256 observations");
     a.inst_list = nullptr;
-    // Launch groups: the second-generation kernel runs two CTAs per SM while two instances fit its shared memory, sized for the
+    // Launch groups: the setup kernel runs two CTAs per SM while two instances fit its shared memory, sized for the
     // LARGEST instance of a launch.  When a few large instances (many surviving candidates) would push a big batch into the
     // one-CTA variant, they get a launch of their own (C5: the last rounds, profiles/c5_rounds_r02.txt).
     std::vector<int> order;
     int n_small_grp = B;
-    if (!v1 && B > 4 * b->sm_count) {
+    if (B > 4 * b->sm_count) {
         const int lim = setup2_two_cta_limit(nc_max);
         if (lim > 0 && n_max > lim) {
             std::vector<int> big;
@@ -254,8 +249,7 @@ static int run_setup(bqb_batch *b, int check_max, cudaStream_t s) {
         for (int i0 = g0; i0 < g1; i0 += b->work_inst) {
             const int cnt = (g1 - i0 < b->work_inst) ? g1 - i0 : b->work_inst;
             a.inst0 = i0;
-            if (v1) { launch_setup(a, cnt, s); CU(cudaGetLastError()); }
-            else CU(launch_setup2(a, cnt, s));
+            CU(launch_setup2(a, cnt, s));
             b->launches++;
         }
     }

@@ -115,7 +115,7 @@ struct ScoreArgs {
     long long xo_stride = 0;
 };
 
-// Arguments of one setup launch (bq_setup.cu, bq_setup2.cu); shared with the C-ABI layer (bq_capi.cu)
+// Arguments of one setup launch (bq_setup2.cu); shared with the C-ABI layer (bq_capi.cu)
 struct SetupArgs {
     // inputs, one row per instance
     const int *ns, *nc;
@@ -128,10 +128,9 @@ struct SetupArgs {
     // outputs
     double *models;            // [B][lay.total]
     Layout lay;
-    // scratch, per instance: 4 matrices of n_cap^2 + 32 vectors of n_cap
+    // scratch, per instance: the packed triangle of instances too large for shared memory (setup2_scratch_stride)
     double *work;
     size_t work_stride;
-    int n_cap;
     int inst0;                 // first instance of this chunk
     const int *inst_list;      // bq_setup2.cu: when set, CTA b works on instance inst_list[inst0 + b] (launch groups by size)
     int n_max, nc_max;         // bq_setup2.cu: largest ns + nc / nc over the instances of the launch (size the shared memory)

@@ -1307,8 +1307,7 @@ BQB_LAUNCH_REL_DECL(128) {
 }
 #elif BQB_SCORE_CLASS == 160
 BQB_LAUNCH_REL_DECL(160) {      // resident only up to ns = 128 here (the scratch of 16 warps), streamed above
-    static const bool force_stream = getenv("BQB_FORCE_STREAM") && atoi(getenv("BQB_FORCE_STREAM"));      // tuning aid
-    if (!force_stream && smem_need<40, 1, 16, false, 512>(a, 0) <= SMEM_LIMIT)
+    if (smem_need<40, 1, 16, false, 512>(a, 0) <= SMEM_LIMIT)
         return launch_cfg<40, 1, 16, 1, false, 512, false, true, 24>(with_env(a), n_inst, sm_count, stream, grid_x);
     if (smem_need<40, 1, 16, true, 2048>(a, 2 * 40) <= SMEM_LIMIT)
         return launch_cfg<40, 1, 16, 1, true, 2048, false, true, 24>(with_env(a), n_inst, sm_count, stream, grid_x);
@@ -1328,21 +1327,11 @@ BQB_LAUNCH_DECL(16) { return launch_cfg<4, 2, 8, 2, false, 2048, false, false>(a
 #elif BQB_SCORE_CLASS == 64
 // (rolled pairs, free-running warps and 4 x 4-warp CTAs were all slower with band skipping: 0.31 / 0.37 / 0.34 / 0.47 ms vs 0.28)
 // (the band-relative loops <16, NT=1, 16 warps, BK=16> measured 0.364 ms against 0.286: at ns = 64 the band is most of the tile)
-cudaError_t launch_score_team_64(const ScoreArgs &a, int n_inst, int sm_count, cudaStream_t stream, int *grid_x);
 // Round-2 experiments on this class (profiles/score64_experiments_r02.md; 10^6 points, ns = 64, ms): this kernel 0.285; free
 // running (ALIGN = 0) 0.335; barrier groups of 4 / 2 warps (ALIGN = 4 / 2) 0.284 / 0.293; rolled row-block loop 0.333; NT = 1
 // with three CTAs per SM 0.43-0.57; 512-entry table 0.288; one CTA per SM 0.422 (=> T = 0.149 + 2.18 / warps: latency bound);
-// the team kernel of bq_score_team.cu (cross-kernel tile shared by four warps through shared memory, 20-32 warps per SM)
-// 0.298-0.333.  BQB_TEAM=1 selects the team kernel (kept as a cross-check of this one in the tests).
-BQB_LAUNCH_DECL(64) {
-    const char *env = getenv("BQB_TEAM");                  // read per launch (tests switch it between calls)
-    const int use_team = env ? atoi(env) : 0;
-    if (use_team) {
-        const cudaError_t e = launch_score_team_64(a, n_inst, sm_count, stream, grid_x);
-        if (e != cudaErrorInvalidConfiguration) return e;
-    }
-    return launch_cfg<16, 2, 8, 2, false, 2048, 1, false>(a, n_inst, sm_count, stream, grid_x);
-}
+// a team kernel (cross-kernel tile shared by four warps through shared memory, 20-32 warps per SM) 0.298-0.333.
+BQB_LAUNCH_DECL(64) { return launch_cfg<16, 2, 8, 2, false, 2048, 1, false>(a, n_inst, sm_count, stream, grid_x); }
 #elif BQB_SCORE_CLASS == 128
 BQB_LAUNCH_REL_DECL(128);
 BQB_LAUNCH_DECL(128) {
@@ -1357,12 +1346,11 @@ BQB_LAUNCH_DECL(128) {
 #elif BQB_SCORE_CLASS == 160
 BQB_LAUNCH_REL_DECL(160);
 BQB_LAUNCH_DECL(160) {       // absolute tile: resident while the instances' operands fit (ns <= 136 ... 144 depending on the candidates), then streamed
-    static const bool force_stream = getenv("BQB_FORCE_STREAM") && atoi(getenv("BQB_FORCE_STREAM"));      // tuning aid
     if (rel_variant() == 1) {
         const cudaError_t e = launch_score_rel_160(a, n_inst, sm_count, stream, grid_x);
         if (e != cudaErrorInvalidConfiguration) return e;
     }
-    if (!force_stream && smem_need<40, 2, 8, false, 512>(a, 0) <= SMEM_LIMIT)
+    if (smem_need<40, 2, 8, false, 512>(a, 0) <= SMEM_LIMIT)
         return launch_cfg<40, 2, 8, 1, false, 512, false, true>(a, n_inst, sm_count, stream, grid_x);
     return launch_cfg<40, 2, 8, 1, true, 2048, false, true>(a, n_inst, sm_count, stream, grid_x);
 }

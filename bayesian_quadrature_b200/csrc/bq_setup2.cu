@@ -1,14 +1,14 @@
-// Setup kernel, second generation: one CTA per model instance with the working matrix RESIDENT IN SHARED MEMORY as a
-// packed lower triangle (row i starts at i (i + 1) / 2).
+// Setup kernel: one CTA per model instance (one BQ problem under one hyper-parameter set) with the working matrix
+// RESIDENT IN SHARED MEMORY as a packed lower triangle (row i starts at i (i + 1) / 2).
 //
-// Same results contract as bq_setup.cu (which stays selectable, BQB_SETUP_V1=1, and is what the cross-check test
-// compares against): it replaces, once per instance, what the reference does per query point through the `gp`
-// package and linalg_c (Gram build bq.py:465, dpotrf linalg_c.pyx:86, gp.mean / cov bq.py:493-496), computes
-// Z_mean (bq_c.pyx:157-213), Z_var (bq_c.pyx:264-355 with gauss_c.pyx:416-531 / :235-339 fused) and log_lh
-// (bq.py:546), and emits the operands of the scoring kernel in DMMA fragment order.
+// It replaces, once per instance instead of once per query point, what the reference does through the `gp` package
+// and linalg_c (Gram build bq.py:465, dpotrf linalg_c.pyx:86, gp.mean / cov bq.py:493-496), computes Z_mean
+// (bq_c.pyx:157-213), Z_var (bq_c.pyx:264-355 with gauss_c.pyx:416-531 / :235-339 fused) and log_lh (bq.py:546),
+// and emits the operands of the scoring kernel in DMMA fragment order.
 //
-// What changed against the first generation (profiles/ncu_setup_r01: FP64 pipe 10 % busy, 57 % of the stall samples on
-// CTA barriers behind one-warp / one-thread phases, 440 MB of global scratch thrashing the L2 at C5 scale):
+// Why it is built this way (an earlier kernel with dense matrices in global scratch, profiles/ncu_setup_r01: FP64 pipe
+// 10 % busy, 57 % of the stall samples on CTA barriers behind one-warp / one-thread phases, 440 MB of global scratch
+// thrashing the L2 at C5 scale):
 //   * ONE packed triangle serves K_tl -> L_tl -> L_tl^-1 (in place), then K_l -> L -> [L_ss^-1; C L_cc] (in place),
 //     then (s_l != 0 only) K_l + s_l^2 I.  n (n + 1) / 2 doubles: 92 KB at n = 152.  Two CTAs of 256 threads per SM
 //     while two instances fit (n <= 155 with ten candidates; decided by the occupancy query at launch) and the launch
@@ -27,7 +27,6 @@
 //     Z_var multiply by reciprocals instead of dividing; L_tl^-1 is read back from its fragment-ordered copy in the
 //     model block for beta' K_tl^-1 beta.
 #include <cstdio>
-#include <cstdlib>
 
 #include "bq_common.cuh"
 
@@ -488,7 +487,10 @@ __global__ void __launch_bounds__(NT, 512 / NT) bq_setup2_kernel(SetupArgs a) {
     __syncthreads();
     if (s_fail) { if (tid == 0) M[H_STATUS] = s_fail; return; }
 
-    // ---- P0b: observations in ascending order of x (stable rank sort); see bq_setup.cu
+    // ---- P0b: observations in ascending order of x (stable rank sort).  Every result of this kernel and of the scoring
+    // kernel is invariant under a permutation of the observations (up to rounding), and with sorted observations the
+    // k-steps that matter for a query point are few and contiguous (band skipping, bq_score.cu) whatever order the
+    // caller -- or add_observation, which appends -- left them in.  Already sorted input is left exactly as it is.
     for (int i = tid; i < ns; i += NT) {
         const double xi = tmp[i];
         int rank = 0;
@@ -949,6 +951,9 @@ static cudaError_t launch_one(const SetupArgs &a, int n_inst, size_t bytes, cuda
     return a.kind ? launch_kind<TSMEM, NT, 1>(a, n_inst, bytes, stream) : launch_kind<TSMEM, NT, 0>(a, n_inst, bytes, stream);
 }
 
+// opt-in maximum of dynamic shared memory per CTA minus the kernel's static shared memory
+constexpr size_t S2_CTA_SMEM_MAX = 227 * 1024 - 256;
+
 // Largest instance order n for which two 256-thread CTAs of the setup kernel fit one SM (0: none), given the launch's nc_max.
 int setup2_two_cta_limit(int nc_max) {
     static int cache[NC_MAX + 2];
@@ -960,7 +965,7 @@ int setup2_two_cta_limit(int nc_max) {
         const int mid = (lo + hi + 1) / 2;
         const size_t bytes = sizeof(double) * (size_t)s2_carve(mid, nc_max, true).total;
         int per_sm = 0;
-        bool ok = bytes <= 227 * 1024 - 256 &&
+        bool ok = bytes <= S2_CTA_SMEM_MAX &&
                   cudaFuncSetAttribute(bq_setup2_kernel<true, 256, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) == cudaSuccess &&
                   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bq_setup2_kernel<true, 256, 0>, 256, bytes) == cudaSuccess && per_sm >= 2;
         if (ok) lo = mid; else hi = mid - 1;
@@ -970,12 +975,19 @@ int setup2_two_cta_limit(int nc_max) {
     return cache[nc_max] = lo;
 }
 
+// Global scratch (doubles per instance, SetupArgs::work_stride) that launch_setup2 can need for instances of capacity
+// class cap: 0 when the largest instance (cap observations, NC_MAX candidates) keeps its triangle in shared memory, else
+// the stride of a packed triangle of that order.
+size_t setup2_scratch_stride(int cap) {
+    const int n = cap + NC_MAX;
+    if (sizeof(double) * (size_t)s2_carve(n, NC_MAX, true).total <= S2_CTA_SMEM_MAX) return 0;
+    return ((size_t)n * (n + 1) / 2 + 64) & ~(size_t)1;
+}
+
 // a.n_max / a.nc_max must be >= ns + nc / nc of every instance of the launch (instances above report SETUP_BAD_INPUT)
 cudaError_t launch_setup2(const SetupArgs &a, int n_inst, cudaStream_t stream) {
-    const size_t cta_max = 227 * 1024 - 256;                 // opt-in maximum minus the kernel's static shared memory
     const size_t bytes_sm = sizeof(double) * (size_t)s2_carve(a.n_max, a.nc_max, true).total;
-    static const int force_nt = getenv("BQB_SETUP_NT") ? atoi(getenv("BQB_SETUP_NT")) : 0;
-    if (bytes_sm <= cta_max) {
+    if (bytes_sm <= S2_CTA_SMEM_MAX) {
         // two CTAs of 256 threads per SM when two instances fit (their serial phases overlap), else one of 512
         int per_sm = 0;
         cudaError_t e = cudaFuncSetAttribute(bq_setup2_kernel<true, 256, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes_sm);
@@ -985,7 +997,7 @@ cudaError_t launch_setup2(const SetupArgs &a, int n_inst, cudaStream_t stream) {
         int dev = 0, sms = 148;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if ((per_sm >= 2 && n_inst > sms && force_nt != 512) || force_nt == 256) return launch_one<true, 256>(a, n_inst, bytes_sm, stream);
+        if (per_sm >= 2 && n_inst > sms) return launch_one<true, 256>(a, n_inst, bytes_sm, stream);
         return launch_one<true, 512>(a, n_inst, bytes_sm, stream);
     }
     const size_t bytes = sizeof(double) * (size_t)s2_carve(a.n_max, a.nc_max, false).total;

@@ -574,12 +574,10 @@ def test_conditioning_sweep_against_truth(lib, tag):
 
 
 @pytest.mark.parametrize("ns,nc", [(64, 4), (40, 2), (17, 0), (64, 6)])
-def test_team_kernel_of_the_64_class_agrees(lib, oracle, ns, nc, monkeypatch):
-    """The 64-observation class has a second scoring kernel (bq_score_team.cu, BQB_TEAM=1: four warps share one cross-kernel
-    tile through shared memory, contiguous k-step bands at exact granularity).  Same sums in a different order: scores agree
-    with the default kernel to ~1e-12 and with the oracle to the parity tolerance, statuses exactly -- grid, scattered
-    points, shortcut / jitter-pattern / invalid points, dense cut-off, fused expected-variance epilogue and prediction mode."""
-    import torch
+def test_64_class_kernel_vs_oracle(lib, oracle, ns, nc):
+    """The scoring kernel of the 64-observation class against the oracle, with the relevance cut-off and dense: a grid,
+    scattered points, shortcut / near-shortcut points, points on and near the candidates (jitter patterns) and invalid
+    points."""
     from bayesian_quadrature_b200 import synthetic
     rs = np.random.RandomState(ns)
     x_s, l_s = synthetic.observations(ns)
@@ -595,43 +593,13 @@ def test_team_kernel_of_the_64_class_agrees(lib, oracle, ns, nc, monkeypatch):
     for cut in (72.0, float("inf")):
         b.set_cutoff(cut)
         for name, x_a in (("grid", grid), ("points", pts)):
-            monkeypatch.setenv("BQB_TEAM", "0")
-            e0, m0, s0 = b.score_host(x_a)
-            ev0, f0 = b.expected_var_host(x_a)
-            p0 = b.predict_host(x_a[np.isfinite(x_a)])
-            monkeypatch.setenv("BQB_TEAM", "1")
-            e1, m1, s1 = b.score_host(x_a)
-            ev1, f1 = b.expected_var_host(x_a)
-            p1 = b.predict_host(x_a[np.isfinite(x_a)])
             tag = "%s ns=%d nc=%d cut=%g" % (name, ns, nc, cut)
-            assert (s0 == s1).all() and f0 == f1, tag
+            esm, em, st = b.score_host(x_a)
+            o_esm, o_em, o_st = m.esm_and_em(x_a)
+            assert ((st[0] & 3) == (o_st & 3)).all(), tag
             ok = np.isfinite(x_a)
-            # points ON a candidate have a Schur pivot of 1e-4 of the diagonal (the jitter): rounding differences of the two
-            # summation orders are amplified 1e4-fold there
-            rt = 1e-11 if name == "grid" else 1e-9
-            assert_close(e1[0][ok], e0[0][ok], "esm " + tag, rtol=rt, atol=1e-300)
-            assert_close(m1[0][ok], m0[0][ok], "em " + tag, rtol=rt, atol=1e-300)
-            # ev = Zm^2 + Zv - esm cancels near the data: judged on the scale of its terms, point by point (the two
-            # kernels' esm may differ by rt * |esm|, and so may ev)
-            fin = ok & np.isfinite(e0[0]) & np.isfinite(ev0)
-            assert (np.isfinite(ev0) == np.isfinite(ev1)).all(), tag
-            bound = rt * np.abs(e0[0][fin]) + 1e-11 * info["Z_mean"][0] ** 2
-            assert (np.abs(ev1[fin] - ev0[fin]) <= bound).all(), ("ev " + tag, float(np.max(np.abs(ev1[fin] - ev0[fin]) / bound)))
-            assert_close(p1[0][0], p0[0][0], "l_mean " + tag, rtol=1e-11, atol=1e-11 * np.abs(p0[0][0]).max())    # k . alpha cancels in the far field
-            assert_close(p1[1][0], p0[1][0], "v_log_l " + tag, rtol=1e-9, atol=1e-12)
-            if cut == 72.0:
-                o_esm, o_em, o_st = m.esm_and_em(x_a)
-                assert ((s1[0] & 3) == (o_st & 3)).all()
-                assert_close(e1[0][ok], o_esm[ok], "esm vs oracle " + tag)
-    # device entry point with the fused epilogue: same (min, first index)
-    x_d = torch.from_numpy(grid).cuda()
-    esm = torch.empty_like(x_d); ev = torch.empty_like(x_d); pair = torch.empty(2, dtype=torch.float64, device="cuda")
-    res = []
-    for t in ("0", "1"):
-        monkeypatch.setenv("BQB_TEAM", t)
-        b.choose_step_device(x_d, esm, ev, pair)
-        res.append(pair.cpu().numpy().copy())
-    assert res[0][1] == res[1][1] and abs(res[0][0] - res[1][0]) <= 1e-11 * abs(res[0][0])
+            assert_close(esm[0][ok], o_esm[ok], "esm " + tag)
+            assert_close(em[0][ok], o_em[ok], "em " + tag)
     b.close()
 
 
