@@ -32,6 +32,7 @@ SYMBOLS = {
     "bqb_batch_setup": (ctypes.c_int, [_vp, _ip, _ip, _dp, _dp, ctypes.c_int, _dp, _dp, _dp, ctypes.c_int, _vp]),
     "bqb_batch_stage": (ctypes.c_int, [_vp, _ip, _dp, _dp, ctypes.c_int, _dp, _dp, _vp]),
     "bqb_batch_set_hypers": (ctypes.c_int, [_vp, _dp, _vp]),
+    "bqb_batch_log_lh_grad": (ctypes.c_int, [_vp, _dp, _ip, ctypes.c_int, ctypes.c_int, _dp, _dp, _ip, _vp]),
     "bqb_batch_set_approx": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, _dp, ctypes.c_int, _ll, ctypes.c_int]),
     "bqb_batch_setup_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp]),
     "bqb_batch_seed_candidates": (ctypes.c_int, [_vp, ctypes.POINTER(ctypes.c_uint), _vp]),
@@ -198,6 +199,23 @@ class Batch(object):
         """Replace the hyper-parameters [n_inst, 6] of the staged instances (the next setup_device uses them)."""
         hyp = _d(hyp).reshape(self.n_inst, 6)
         _check(load().bqb_batch_set_hypers(self._h, _pd(hyp), _vp(stream) if stream else None), "bqb_batch_set_hypers")
+
+    def log_lh_grad(self, hyp, inst=None, check_max=True, stream=None):
+        """Joint log marginal likelihood and its gradient for rows of hyper-parameters hyp [n, 6] (h, w, s of gp_log_l,
+        then of gp_l); row r is instance inst[r] (default: instance r).  Evaluated on the staged observations and
+        candidates; the set-up model is left untouched.  Returns (log_lh [n], grad [n, 6], status [n]); a row whose status
+        is not SETUP_OK has log_lh -inf and a NaN gradient."""
+        hyp = _d(hyp).reshape(-1, 6)
+        n = hyp.shape[0]
+        if inst is not None:
+            inst = np.ascontiguousarray(inst, dtype=np.int32).reshape(-1)
+            if inst.shape[0] != n:
+                raise ValueError("inst must have one entry per row of hyp")
+        llh, grad, st = np.empty(n), np.empty((n, 6)), np.empty(n, dtype=np.int32)
+        _check(load().bqb_batch_log_lh_grad(self._h, _pd(hyp), inst.ctypes.data_as(_ip) if inst is not None else None, n,
+                                            int(check_max), _pd(llh), _pd(grad), st.ctypes.data_as(_ip),
+                                            _vp(stream) if stream else None), "bqb_batch_log_lh_grad")
+        return llh, grad, st
 
     def set_approx(self, kernel_kind=0, period=None, xo=None, p_xo=None, force_generic=False):
         """Kernel kind (0 Gaussian, 1 periodic with period [n_inst, 2] = p of gp_log_l / gp_l) and, when ``xo`` / ``p_xo``

@@ -243,6 +243,66 @@ class BatchBQ(object):
             self._check_info(self.batch.setup_device())
         return np.where(ok & (info["status"] == _lib.SETUP_OK) & np.isfinite(info["log_lh"]), info["log_lh"], -np.inf)
 
+    def _log_lh_grad_rows(self, rows, hyp):
+        """(log_lh [r], grad [r, 6]) of the problems ``rows`` under the hyper-parameter rows hyp [r, 6], with the -inf
+        semantics of log_lh (the gradient is NaN there).  Only the valid rows reach the device."""
+        rows = np.asarray(rows, dtype=np.int64)
+        ll, grad = np.full(rows.size, -np.inf), np.full((rows.size, 6), np.nan)
+        ok = self._valid_hyp(hyp)
+        if ok.any():
+            l, g, st = self.batch.log_lh_grad(hyp[ok], inst=rows[ok], check_max=True)
+            good = (st == _lib.SETUP_OK) & np.isfinite(l)
+            idx = np.nonzero(ok)[0][good]
+            ll[idx], grad[idx] = l[good], g[good]
+        return ll, grad
+
+    def log_lh_grad(self, hypers_tl, hypers_l, params):
+        """``log_lh`` with its gradient: the joint log marginal likelihood of every problem under hypers_tl[p] /
+        hypers_l[p] ([P, len(params)]) and its derivatives with respect to those named parameters, from one launch of the
+        gradient kernel (the closed-form derivative of both GPs' log likelihoods, including the dependence of l_c on the
+        parameters of gp_log_l).  Returns (log_lh [P], grad_tl [P, k], grad_l [P, k]).  log_lh is -inf where ``log_lh``
+        gives -inf, and the gradient is NaN there.  The batch's model is not touched."""
+        hyp = self._hyp_rows(hypers_tl, hypers_l, params)
+        if hyp.ndim != 2:
+            raise ValueError("hypers_tl and hypers_l must be [P, %d]" % len(params))
+        ll, g = self._log_lh_grad_rows(np.arange(self.P), hyp)
+        cols = [_NAMES.index(p) for p in params]
+        return ll, g[:, cols], g[:, [3 + c for c in cols]]
+
+    def fit_hypers(self, params, maxiter=200):
+        """Maximise every problem's joint log marginal likelihood over the named parameters of both GPs
+        (``BQ.fit_hypers``, bq.py:554-562), starting from the batch's hyper-parameters.  The optimiser is
+        ``util.lbfgs_batch`` in the logarithms of the parameters, with the gradient from ``log_lh_grad``; each of its
+        steps evaluates only the problems that are still running.  The fitted values are written into ``self.hyp`` and
+        the model is set up again under them; the candidates stay as they are (the reference's fit only recomputes l_c).
+
+        A problem whose start has zero probability raises RuntimeError naming it, before anything changes.  Fitting "s"
+        needs s > 0 at the start for both GPs of every problem (ValueError otherwise).  Returns a dict: log_lh [P] at the
+        fitted point, converged [P], iterations [P] and evaluations (problem evaluations in total)."""
+        cols = [_NAMES.index(p) if p in _NAMES else -1 for p in params]
+        if not params or min(cols) < 0:
+            raise ValueError("unknown hyper-parameter in %s (BatchBQ has %s)" % (params, ", ".join(_NAMES)))
+        cols6 = cols + [3 + c for c in cols]
+        if not (self.hyp[:, cols6] > 0).all():
+            raise ValueError("fitting %s needs positive starting values (it works with their logarithms)" % list(params))
+
+        def fg(X, rows):
+            hyp = self.hyp[rows].copy()
+            hyp[:, cols6] = np.exp(X)
+            ll, g = self._log_lh_grad_rows(rows, hyp)
+            return ll, g[:, cols6] * hyp[:, cols6]           # d ll / d log(theta)
+        try:
+            res = util.lbfgs_batch(fg, np.log(self.hyp[:, cols6]), maxiter=maxiter)
+        except RuntimeError as e:
+            if getattr(e, "row", None) is None:
+                raise
+            raise RuntimeError("problem %d: zero probability at the starting hyper-parameters" % e.row) from e
+        self.hyp[:, cols6] = np.exp(res["x"])
+        self.batch.set_hypers(self.hyp)
+        self._check_info(self.batch.setup_device())
+        return {"log_lh": res["f"], "converged": res["converged"], "iterations": res["iterations"],
+                "evaluations": res["evaluations"]}
+
     def sample_hypers(self, params, n, nburn=10, seed=0, first_problem=0, max_steps=None, stats=None):
         """Slice-sample the named hyper-parameters of both GPs of every problem (``BQ.sample_hypers``, bq.py:565-598):
         one chain per problem, started at the batch's hyper-parameters with window 2 * len(params), n samples after

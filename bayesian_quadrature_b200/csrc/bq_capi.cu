@@ -15,6 +15,7 @@
 
 namespace bqb {
 cudaError_t launch_setup2(const SetupArgs &a, int n_inst, cudaStream_t stream);
+cudaError_t launch_llgrad(LLGradArgs a, int n_rows, int work_inst, cudaStream_t stream, int *launches);
 int setup2_two_cta_limit(int nc_max);
 size_t setup2_scratch_stride(int cap);
 cudaError_t launch_score(const ScoreArgs &a, int n_inst, int sm_count, cudaStream_t stream, int *grid_x = nullptr);
@@ -69,6 +70,10 @@ struct bqb_batch {
     bool big_class = false;            // capacity 512: no tensor-core scoring kernels
     double *d_period = nullptr, *d_xo = nullptr, *d_pxo = nullptr, *d_wp = nullptr, *d_gz = nullptr;
     int *d_inst_list = nullptr;        // setup launch groups (instances ordered by size class)
+    // bqb_batch_log_lh_grad: hyper-parameter rows, instance list and output rows (grown on demand)
+    double *d_llg_hyp = nullptr, *d_llg_out = nullptr;
+    int *d_llg_inst = nullptr;
+    size_t cap_llg = 0;
     // scoring: relevance cut-off (bq_score.cu, CUT_ARG; +inf = dense) and the optional executed-work counter
     double cut_arg = 72.0;
     unsigned long long *d_work_ctr = nullptr;
@@ -177,7 +182,7 @@ void bqb_batch_destroy(bqb_batch *b) {
     cudaSetDevice(b->device);
     void *ptrs[] = {b->d_models, b->d_tab, b->d_work, b->d_ns, b->d_nc, b->d_xs, b->d_ls, b->d_xc, b->d_hyp, b->d_prior,
                     b->d_xa, b->d_esm, b->d_em, b->d_st, b->d_red_val, b->d_red_idx, b->d_flags, b->d_mt, b->d_mti, b->d_overflow, b->d_work_ctr, b->d_xsorted, b->d_perm, b->d_iota, b->d_sort_tmp,
-                    b->d_period, b->d_xo, b->d_pxo, b->d_wp, b->d_gz, b->d_inst_list};
+                    b->d_period, b->d_xo, b->d_pxo, b->d_wp, b->d_gz, b->d_inst_list, b->d_llg_hyp, b->d_llg_out, b->d_llg_inst};
     for (void *p : ptrs) if (p) cudaFree(p);
     for (cudaStream_t st : b->pipe) if (st) cudaStreamDestroy(st);
     if (b->h_flags) cudaFreeHost(b->h_flags);
@@ -187,15 +192,11 @@ void bqb_batch_destroy(bqb_batch *b) {
     delete b;
 }
 
-// Runs the setup kernel on the staged device inputs and fetches the per-instance headers and counts.
-static int run_setup(bqb_batch *b, int check_max, cudaStream_t s) {
+// Largest ns + nc and nc over the staged instances (they size the shared memory of the setup and gradient kernels).
+// The counts are fetched first when the device-side round kernels (add_observations, draw_candidates) changed them
+// without the host seeing it.
+static int staged_sizes(bqb_batch *b, cudaStream_t s, int *n_max_out, int *nc_max_out) {
     const int B = b->n_inst;
-    SetupArgs a;
-    a.ns = b->d_ns; a.nc = b->d_nc; a.x_s = b->d_xs; a.l_s = b->d_ls; a.x_c = b->d_xc; a.hyp = b->d_hyp; a.prior = b->d_prior;
-    a.in_stride = b->ns_cap; a.check_max = check_max; a.models = b->d_models; a.lay = b->lay;
-    a.work = b->d_work; a.work_stride = b->work_stride;
-    // counts on the host before the launch (they size the setup kernel's shared memory); the device-side
-    // round kernels (add_observations, draw_candidates) change them without the host seeing it
     if (!b->counts_fresh) {
         CU(cudaMemcpyAsync(b->h_ns.data(), b->d_ns, sizeof(int) * B, cudaMemcpyDeviceToHost, s));
         CU(cudaMemcpyAsync(b->h_nc.data(), b->d_nc, sizeof(int) * B, cudaMemcpyDeviceToHost, s));
@@ -209,6 +210,20 @@ static int run_setup(bqb_batch *b, int check_max, cudaStream_t s) {
         if (ns_i + nc_i > n_max) n_max = ns_i + nc_i;
         if (nc_i > nc_max) nc_max = nc_i;
     }
+    *n_max_out = n_max; *nc_max_out = nc_max;
+    return 0;
+}
+
+// Runs the setup kernel on the staged device inputs and fetches the per-instance headers and counts.
+static int run_setup(bqb_batch *b, int check_max, cudaStream_t s) {
+    const int B = b->n_inst;
+    SetupArgs a;
+    a.ns = b->d_ns; a.nc = b->d_nc; a.x_s = b->d_xs; a.l_s = b->d_ls; a.x_c = b->d_xc; a.hyp = b->d_hyp; a.prior = b->d_prior;
+    a.in_stride = b->ns_cap; a.check_max = check_max; a.models = b->d_models; a.lay = b->lay;
+    a.work = b->d_work; a.work_stride = b->work_stride;
+    int n_max, nc_max;
+    const int rc = staged_sizes(b, s, &n_max, &nc_max);
+    if (rc) return rc;
     a.n_max = n_max; a.nc_max = nc_max;
     a.kind = b->kind; a.period = b->d_period; a.xo = b->d_xo; a.pxo = b->d_pxo; a.n_xo = b->n_xo; a.xo_stride = b->xo_stride;
     a.wp = b->d_wp; a.gz = b->d_gz;
@@ -323,6 +338,50 @@ int bqb_batch_set_hypers(bqb_batch *b, const double *hyp, void *stream) {
     CU(cudaMemcpyAsync(b->d_hyp, hyp, sizeof(double) * (size_t)b->n_inst * 6, cudaMemcpyHostToDevice, s));
     CU(cudaStreamSynchronize(s));          // the host array may be pageable and is free to change after this call
     b->ready = false;
+    return 0;
+}
+
+int bqb_batch_log_lh_grad(bqb_batch *b, const double *hyp, const int *inst, int n_eval, int check_max, double *log_lh_out,
+                          double *grad_out, int *status_out, void *stream) {
+    if (!b) return fail(BQB_EINVAL, "bqb_batch_log_lh_grad: null batch");
+    if (!b->staged) return fail(BQB_ESTATE, "bqb_batch_log_lh_grad: nothing staged (bqb_batch_stage / bqb_batch_setup first)");
+    if (n_eval < 0 || (n_eval > 0 && (!hyp || !log_lh_out || !grad_out || !status_out)) || (!inst && n_eval > b->n_inst))
+        return fail(BQB_EINVAL, "bqb_batch_log_lh_grad: bad arguments");
+    for (int e = 0; inst && e < n_eval; ++e)
+        if (inst[e] < 0 || inst[e] >= b->n_inst) return fail(BQB_EINVAL, "bqb_batch_log_lh_grad: instance index out of range");
+    if (b->kind != 0) return fail(BQB_EUNSUPPORTED, "bqb_batch_log_lh_grad: only the Gaussian kernel is supported");
+    if (n_eval == 0) return 0;
+    CU(cudaSetDevice(b->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    LLGradArgs a;
+    int rc = staged_sizes(b, s, &a.n_max, &a.nc_max);
+    if (rc) return rc;
+    if ((size_t)n_eval > b->cap_llg) {
+        for (void *p : {(void *)b->d_llg_hyp, (void *)b->d_llg_out, (void *)b->d_llg_inst}) if (p) cudaFree(p);
+        b->d_llg_hyp = b->d_llg_out = nullptr; b->d_llg_inst = nullptr; b->cap_llg = 0;
+        CU(cudaMalloc(&b->d_llg_hyp, sizeof(double) * 6 * (size_t)n_eval));
+        CU(cudaMalloc(&b->d_llg_out, sizeof(double) * LLG_OUT * (size_t)n_eval));
+        CU(cudaMalloc(&b->d_llg_inst, sizeof(int) * (size_t)n_eval));
+        b->cap_llg = n_eval;
+    }
+    CU(cudaMemcpyAsync(b->d_llg_hyp, hyp, sizeof(double) * 6 * (size_t)n_eval, cudaMemcpyHostToDevice, s));
+    if (inst) CU(cudaMemcpyAsync(b->d_llg_inst, inst, sizeof(int) * (size_t)n_eval, cudaMemcpyHostToDevice, s));
+    a.ns = b->d_ns; a.nc = b->d_nc; a.x_s = b->d_xs; a.l_s = b->d_ls; a.x_c = b->d_xc; a.in_stride = b->ns_cap;
+    a.hyp = b->d_llg_hyp; a.inst = inst ? b->d_llg_inst : nullptr; a.e0 = 0; a.check_max = check_max;
+    a.work = b->d_work; a.work_stride = b->work_stride; a.out = b->d_llg_out;
+    int launches = 0;
+    const cudaError_t e = launch_llgrad(a, n_eval, b->work_inst, s, &launches);
+    b->launches += launches;
+    CU(e);
+    std::vector<double> h((size_t)n_eval * LLG_OUT);
+    CU(cudaMemcpyAsync(h.data(), b->d_llg_out, sizeof(double) * h.size(), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    for (int r = 0; r < n_eval; ++r) {
+        const double *o = &h[(size_t)r * LLG_OUT];
+        log_lh_out[r] = o[0];
+        memcpy(grad_out + (size_t)r * 6, o + 1, sizeof(double) * 6);
+        status_out[r] = (int)o[7];
+    }
     return 0;
 }
 

@@ -144,6 +144,24 @@ struct SetupArgs {
     double *gz;                // scratch [launch instances][n_xo]
 };
 
+// Arguments of one launch of the log-likelihood gradient kernel (bq_setup2.cu); shared with the C-ABI layer (bq_capi.cu).
+// It reads the staged inputs of a batch and writes nothing but `out`.
+constexpr int LLG_OUT = 8;     // doubles per output row: log_lh, d/d(h_tl, w_tl, s_tl, h_l, w_l, s_l), status
+struct LLGradArgs {
+    const int *ns, *nc;
+    const double *x_s, *l_s;   // [n_inst][in_stride] (in_stride = the batch's observation capacity)
+    const double *x_c;         // [n_inst][NC_MAX]
+    int in_stride;
+    const double *hyp;         // [n_eval][6]  h_tl, w_tl, s_tl, h_l, w_l, s_l of each row
+    const int *inst;           // [n_eval] instance of each row (null: row e is instance e)
+    int e0;                    // first row of this launch
+    int check_max;             // apply the bq.py:942-947 guard
+    int n_max, nc_max;         // largest ns + nc / nc over the batch's instances (size the shared memory)
+    double *work;              // scratch per CTA for instances too large for shared memory (setup2_scratch_stride)
+    size_t work_stride;
+    double *out;               // [n_eval][LLG_OUT]
+};
+
 #ifdef __CUDACC__
 
 // D(8x8) += A(8x4) * B(4x8), FP64 tensor path (SASS: DMMA.8x8x4).  Lane l holds

@@ -1004,4 +1004,336 @@ cudaError_t launch_setup2(const SetupArgs &a, int n_inst, cudaStream_t stream) {
     return launch_one<false, 512>(a, n_inst, bytes, stream);
 }
 
+// ============================================================================================================================
+// Value and gradient of the joint log marginal likelihood ll = ll_tl + ll_l (BQ._make_llh_params, bq.py:533-552) with
+// respect to the six hyper-parameters, one CTA per (instance, hyper-parameter row).  Gaussian kernel only.
+//
+//   ll_tl: gp_log_l on (x_s, log l_s), K_t = c_t E_t + s_t^2 I, c = h^2 / (sqrt(2 pi) w), E_ij = exp(-d_ij^2 / 2 w^2)
+//   ll_l:  gp_l on (x_sc, [l_s; l_c]), K_l = c_l E_l + s_l^2 I, l_c[j] = exp(m_j), m_j = k_j' a, a = K_t^-1 log l_s
+//   d ll / d theta_l = 1/2 alpha' Kd alpha - 1/2 tr(K_l^-1 Kd),   alpha = K_l^-1 l_sc
+//   d ll / d theta_t = 1/2 a' Kd a - 1/2 tr(K_t^-1 Kd) - sum_j gamma_j dm_j,   gamma_j = alpha[ns + j] l_c[j]
+//       dm_j = kd_j' a - k_j' K_t^-1 Kd a
+//   Kd_h = 2 G / h, Kd_w = G . D^2 / w^3 - G / w, Kd_s = 2 s I  (G = c E; kd_j the same for the cross-kernel, kd_s = 0)
+//   tr(K^-1 Kd_h) = 2 (n - s^2 tr K^-1) / h,  tr(K^-1 Kd_s) = 2 s tr K^-1,  tr K^-1 = |L^-1|_F^2
+//   tr(K^-1 Kd_w) = sum_ij (K^-1)_ij G_ij d_ij^2 / w^3 - (n - s^2 tr K^-1) / w
+//
+// Storage: one packed triangle serves both GPs, as in the setup kernel (the same carve-up, s2_carve, plus three vectors
+// and the 3 x nc derivatives dm_j).  tl phase: L_t -> L_t^-1 in place, a, l_c, the guard, the tl traces, and dm_j for
+// every candidate and tl parameter from the three vectors K_t^-1 G a, K_t^-1 (G . D^2) a and K_t^-1 a (so no ns x nc
+// matrix is kept).  l phase: L_l -> L_l^-1 in place, alpha, the l traces; then the -sum gamma_j dm_j terms.  The only
+// trace that needs entries of K^-1 (the w-trace) evaluates (K^-1)_ij = sum_{k >= i} X_ki X_kj (X = L^-1) for i > j, one
+// thread per entry, and never stores them.
+//
+// Observations are sorted as in the setup kernel, and the tl factor, a and l_c are computed by the same code, so l_c and
+// the guard are the setup's bit for bit.  Every reduction has a fixed order and the CTA shape is fixed (256 threads), so
+// a row's results do not depend on the other rows of the launch.  Status codes and the order of the checks are the
+// setup's: a K_l without the noise s_l^2 that is not positive definite is SETUP_KL_NOTPD even when s_l != 0.
+constexpr int LLG_NT = 256;
+constexpr int LLG_NVEC = 3;     // K_t^-1 G a, K_t^-1 (G . D^2) a, K_t^-1 a: live across the candidate pass (stage)
+
+__host__ __device__ inline int llg_smem_doubles(int nmax, int ncm, bool tsmem) {
+    const S2Carve c = s2_carve(nmax, ncm, tsmem);
+    return c.total + LLG_NVEC * c.nv + 3 * NC_MAX;
+}
+
+// sum over i > j of (K^-1)_ij G_ij d_ij^2 with K^-1 = X' X, X = L^-1 packed in T (partial sum of the calling thread)
+__device__ __forceinline__ double llg_wtrace_part(const double *T, int n, const double *x, double c, double nh) {
+    double p = 0.0;
+    for (int e = threadIdx.x; e < tri(n); e += LLG_NT) {
+        int i, j;
+        tri_decode(e, i, j);
+        if (j == i) continue;
+        double kij = 0.0;
+        for (int k = i, r = tri(i); k < n; r += ++k) kij = fma(T[r + i], T[r + j], kij);
+        const double d = x[i] - x[j], d2 = d * d;
+        p = fma(kij, c * kernel_exp(d, nh, 0, 0.0) * d2, p);
+    }
+    return p;
+}
+
+// g1 = G v, g2 = (G . D^2) v over the first n points of x, a thread per row (G = c E, without the noise)
+__device__ __forceinline__ void llg_gram_matvec(const double *x, int n, double c, double nh, const double *v, double *g1, double *g2) {
+    for (int i = threadIdx.x; i < n; i += LLG_NT) {
+        double s1 = 0.0, s2 = 0.0;
+        for (int j = 0; j < n; ++j) {
+            const double d = x[i] - x[j];
+            const double g = c * kernel_exp(d, nh, 0, 0.0);
+            s1 = fma(g, v[j], s1);
+            s2 = fma(g * (d * d), v[j], s2);
+        }
+        g1[i] = s1;
+        g2[i] = s2;
+    }
+    __syncthreads();
+}
+
+template <bool TSMEM>
+__global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
+    constexpr int NT = LLG_NT, NW = NT / 32;
+    __shared__ double red[NW];
+    __shared__ int s_fail, s_info;
+    extern __shared__ double s_dyn[];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int e = a.e0 + blockIdx.x;
+    const int inst = a.inst ? a.inst[e] : e;
+    double *out = a.out + (size_t)e * LLG_OUT;
+    const int ns = a.ns[inst], nc = a.nc[inst], n = ns + nc;
+
+    // carve-up: the setup kernel's, then [p1 p2 p3] [dm 3 x NC_MAX]
+    const S2Carve cv = s2_carve(a.n_max, a.nc_max, TSMEM);
+    const int lds = cv.lds, nv = cv.nv;
+    double *T = TSMEM ? s_dyn : a.work + (size_t)blockIdx.x * a.work_stride;
+    double *vec = s_dyn + cv.np;
+    double *tl_s = vec, *a_tl = vec + nv, *x_sc = vec + 2 * nv, *l_sc = vec + 3 * nv, *rdiag = vec + 4 * nv;
+    double *un = vec + S2_NVEC_FIXED * nv;
+    double *stage = un;
+    double *u0 = un, *u1 = un + nv, *u2 = un + 2 * nv, *u3 = un + 3 * nv;
+    double *blk = un + cv.un;
+    double *p1 = s_dyn + cv.total, *p2 = p1 + nv, *p3 = p2 + nv;
+    double *dm = p3 + nv;
+
+    auto fail = [&](int status) {
+        if (tid == 0) {
+            out[0] = -INFINITY;
+            for (int k = 1; k < 7; ++k) out[k] = NAN;
+            out[7] = status;
+        }
+    };
+    const double *hp = a.hyp + (size_t)e * 6;
+    const double h_tl = hp[0], w_tl = hp[1], s_tl = hp[2], h_l = hp[3], w_l = hp[4], s_l = hp[5];
+    if (!(ns >= 1 && ns <= a.in_stride && nc >= 0 && nc <= NC_MAX && nc <= a.nc_max && n <= a.n_max)) { fail(SETUP_BAD_INPUT); return; }
+    if (tid == 0) s_fail = SETUP_OK;
+    __syncthreads();
+    {
+        const double *x_s = a.x_s + (size_t)inst * a.in_stride;
+        const double *l_s = a.l_s + (size_t)inst * a.in_stride;
+        const double *x_c = a.x_c + (size_t)inst * NC_MAX;
+        int bad = 0;
+        for (int i = tid; i < ns; i += NT) {
+            const double x = x_s[i], l = l_s[i];
+            bad |= !(isfinite(x) && isfinite(l) && l > 0.0);
+            u0[i] = x;
+            u1[i] = l;
+        }
+        for (int i = tid; i < nc; i += NT) {
+            const double x = x_c[i];
+            bad |= !isfinite(x);
+            x_sc[ns + i] = x;
+        }
+        if (tid == 0) {
+            for (int k = 0; k < 6; ++k) bad |= !isfinite(hp[k]);
+            bad |= !(h_tl > 0 && w_tl > 0 && s_tl >= 0 && h_l > 0 && w_l > 0 && s_l >= 0);
+        }
+        if (bad) s_fail = SETUP_BAD_INPUT;
+    }
+    __syncthreads();
+    if (s_fail) { fail(s_fail); return; }
+    // observations in ascending order of x, stable (the setup kernel's order)
+    for (int i = tid; i < ns; i += NT) {
+        const double xi = u0[i];
+        int rank = 0;
+        for (int j = 0; j < ns; ++j) {
+            const double xj = u0[j];
+            rank += (xj < xi) || (xj == xi && j < i);
+        }
+        x_sc[rank] = xi;
+        l_sc[rank] = u1[i];
+    }
+    __syncthreads();
+
+    const double c_tl = (h_tl * h_tl) / (S2_SQRT_2PI * w_tl), nh_tl = -0.5 / (w_tl * w_tl);
+    const double c_l = (h_l * h_l) / (S2_SQRT_2PI * w_l), nh_l = -0.5 / (w_l * w_l);
+
+    // ---- tl phase: K_t -> L_t -> L_t^-1, a
+    for (int i = tid; i < ns; i += NT) tl_s[i] = log(l_sc[i]);
+    for (int q = tid; q < tri(ns); q += NT) {
+        int i, j;
+        tri_decode(q, i, j);
+        double v = c_tl * kernel_exp(x_sc[i] - x_sc[j], nh_tl, 0, 0.0);
+        if (i == j) v += s_tl * s_tl;
+        T[q] = v;
+    }
+    __syncthreads();
+    if (chol_packed<NT>(T, ns, blk, &s_info, rdiag)) { fail(SETUP_KTL_NOTPD); return; }
+    double sumlog_tl;
+    {
+        double p = 0.0;
+        for (int i = tid; i < ns; i += NT) p += log(T[tri(i) + i]);
+        sumlog_tl = block_sum2<NT>(p, red);
+    }
+    tri_inverse_packed<NT>(T, ns, stage, lds, rdiag);
+    lower_matvec_p<NT>(T, ns, tl_s, u0, nullptr, nullptr);
+    lower_matvec_t_p<NT>(T, ns, u0, a_tl, nullptr, nullptr);
+    // u0 = G a, u1 = (G . D^2) a; p1 = K_t^-1 u0, p2 = K_t^-1 u1, p3 = K_t^-1 a
+    llg_gram_matvec(x_sc, ns, c_tl, nh_tl, a_tl, u0, u1);
+    lower_matvec_p<NT>(T, ns, u0, u2, u1, u3);
+    lower_matvec_t_p<NT>(T, ns, u2, p1, u3, p2);
+    lower_matvec_p<NT>(T, ns, a_tl, u2, nullptr, nullptr);
+    lower_matvec_t_p<NT>(T, ns, u2, p3, nullptr, nullptr);
+    double g_tl[3], yKy_tl;
+    {
+        double pg1 = 0.0, pg2 = 0.0, paa = 0.0, py = 0.0, ptr = 0.0;
+        for (int i = tid; i < ns; i += NT) {
+            pg1 = fma(a_tl[i], u0[i], pg1);
+            pg2 = fma(a_tl[i], u1[i], pg2);
+            paa = fma(a_tl[i], a_tl[i], paa);
+        }
+        for (int i = tid; i < ns; i += NT) py = fma(tl_s[i], a_tl[i], py);
+        for (int q = tid; q < tri(ns); q += NT) ptr = fma(T[q], T[q], ptr);
+        const double aga = block_sum2<NT>(pg1, red), agda = block_sum2<NT>(pg2, red), aa = block_sum2<NT>(paa, red);
+        yKy_tl = block_sum2<NT>(py, red);
+        const double trK = block_sum2<NT>(ptr, red);
+        const double wtr = 2.0 * block_sum2<NT>(llg_wtrace_part(T, ns, x_sc, c_tl, nh_tl), red);
+        const double rest = ns - s_tl * s_tl * trK;
+        g_tl[0] = (aga - rest) / h_tl;
+        g_tl[1] = 0.5 * ((agda - wtr) / (w_tl * w_tl * w_tl) - (aga - rest) / w_tl);
+        g_tl[2] = s_tl * (aa - trK);
+    }
+    // l_c = exp(k_j' a), the guard and dm_j, four candidates per pass (the setup kernel's P6, plus the three dm_j):
+    // stage rows 0..3 = k_j, rows 4..7 = (L_t^-1 k_j)^2 element-wise (the guard only)
+    for (int j0 = 0; j0 < nc; j0 += 4) {
+        const int nbt = (nc - j0 < 4) ? nc - j0 : 4;
+        for (int q = tid; q < nbt * ns; q += NT) {
+            const int j = q / ns, k = q - j * ns;
+            stage[j * lds + k] = c_tl * kernel_exp(x_sc[ns + j0 + j] - x_sc[k], nh_tl, 0, 0.0);
+        }
+        __syncthreads();
+        if (a.check_max) {
+            for (int q = tid; q < nbt * ns; q += NT) {
+                const int j = q / ns, r = q - j * ns;
+                const double *row = T + tri(r), *kc = stage + j * lds;
+                double s0 = 0.0, s1 = 0.0;
+                int k = 0;
+                for (; k + 1 <= r; k += 2) {
+                    s0 = fma(row[k], kc[k], s0);
+                    s1 = fma(row[k + 1], kc[k + 1], s1);
+                }
+                if (k <= r) s0 = fma(row[k], kc[k], s0);
+                const double y = s0 + s1;
+                stage[(4 + j) * lds + r] = y * y;
+            }
+            __syncthreads();
+        }
+        if (warp < nbt) {
+            const int j = warp;
+            const double xc = x_sc[ns + j0 + j];
+            double m = 0.0, q = 0.0, r = 0.0, q1 = 0.0, q2 = 0.0, q3 = 0.0;
+            for (int k = lane; k < ns; k += 32) {
+                const double kv = stage[j * lds + k], d = xc - x_sc[k];
+                m = fma(kv, a_tl[k], m);
+                if (a.check_max) q += stage[(4 + j) * lds + k];
+                r = fma(kv * (d * d), a_tl[k], r);
+                q1 = fma(kv, p1[k], q1);
+                q2 = fma(kv, p2[k], q2);
+                q3 = fma(kv, p3[k], q3);
+            }
+            m = warp_sum(m);
+            q = warp_sum(q);
+            r = warp_sum(r);
+            q1 = warp_sum(q1);
+            q2 = warp_sum(q2);
+            q3 = warp_sum(q3);
+            if (lane == 0) {
+                if (a.check_max) {
+                    double V = c_tl - q;
+                    if (V < 0) V = 0;
+                    if (m + 2 * sqrt(V) > MAX_EXPONENT) s_fail = SETUP_MEAN_TOO_LARGE;
+                }
+                l_sc[ns + j0 + j] = exp(m);
+                dm[j0 + j] = 2.0 * (m - q1) / h_tl;
+                dm[NC_MAX + j0 + j] = (r - q2) / (w_tl * w_tl * w_tl) - (m - q1) / w_tl;
+                dm[2 * NC_MAX + j0 + j] = -2.0 * s_tl * q3;
+            }
+        }
+        __syncthreads();
+    }
+    __syncthreads();
+    if (s_fail) { fail(s_fail); return; }
+
+    // ---- l phase: K_l (the noise-free matrix first, as the setup kernel factorises it) -> L_l -> L_l^-1, alpha
+    for (int pass = 0; pass < (s_l != 0.0 ? 2 : 1); ++pass) {
+        for (int q = tid; q < tri(n); q += NT) {
+            int i, j;
+            tri_decode(q, i, j);
+            double v = c_l * kernel_exp(x_sc[i] - x_sc[j], nh_l, 0, 0.0);
+            if (pass && i == j) v += s_l * s_l;
+            T[q] = v;
+        }
+        __syncthreads();
+        if (chol_packed<NT>(T, n, blk, &s_info, rdiag)) { fail(SETUP_KL_NOTPD); return; }
+    }
+    double sumlog_l;
+    {
+        double p = 0.0;
+        for (int i = tid; i < n; i += NT) p += log(T[tri(i) + i]);
+        sumlog_l = block_sum2<NT>(p, red);
+    }
+    tri_inverse_packed<NT>(T, n, stage, lds, rdiag);
+    double *alpha = u1;
+    lower_matvec_p<NT>(T, n, l_sc, u0, nullptr, nullptr);
+    lower_matvec_t_p<NT>(T, n, u0, alpha, nullptr, nullptr);
+    llg_gram_matvec(x_sc, n, c_l, nh_l, alpha, u2, u3);
+    {
+        double pg1 = 0.0, pg2 = 0.0, paa = 0.0, py = 0.0, ptr = 0.0;
+        for (int i = tid; i < n; i += NT) {
+            pg1 = fma(alpha[i], u2[i], pg1);
+            pg2 = fma(alpha[i], u3[i], pg2);
+            paa = fma(alpha[i], alpha[i], paa);
+        }
+        for (int i = tid; i < n; i += NT) py = fma(l_sc[i], alpha[i], py);
+        for (int q = tid; q < tri(n); q += NT) ptr = fma(T[q], T[q], ptr);
+        const double aga = block_sum2<NT>(pg1, red), agda = block_sum2<NT>(pg2, red), aa = block_sum2<NT>(paa, red);
+        const double yKy = block_sum2<NT>(py, red), trK = block_sum2<NT>(ptr, red);
+        const double wtr = 2.0 * block_sum2<NT>(llg_wtrace_part(T, n, x_sc, c_l, nh_l), red);
+        if (tid == 0) {
+            const double rest = n - s_l * s_l * trK;
+            double ch = 0.0, cw = 0.0, cs = 0.0;                  // sum_j gamma_j dm_j, in candidate order
+            for (int j = 0; j < nc; ++j) {
+                const double gam = alpha[ns + j] * l_sc[ns + j];
+                ch = fma(gam, dm[j], ch);
+                cw = fma(gam, dm[NC_MAX + j], cw);
+                cs = fma(gam, dm[2 * NC_MAX + j], cs);
+            }
+            out[0] = (-0.5 * yKy_tl - sumlog_tl - 0.5 * ns * S2_LOG_2PI) + (-0.5 * yKy - sumlog_l - 0.5 * n * S2_LOG_2PI);
+            out[1] = g_tl[0] - ch;
+            out[2] = g_tl[1] - cw;
+            out[3] = g_tl[2] - cs;
+            out[4] = (aga - rest) / h_l;
+            out[5] = 0.5 * ((agda - wtr) / (w_l * w_l * w_l) - (aga - rest) / w_l);
+            out[6] = s_l * (aa - trK);
+            out[7] = SETUP_OK;
+        }
+    }
+}
+
+template <bool TSMEM>
+static cudaError_t launch_llgrad_one(const LLGradArgs &a, int n_rows, size_t bytes, cudaStream_t stream) {
+    cudaError_t e = cudaFuncSetAttribute(bq_llgrad_kernel<TSMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e != cudaSuccess) return e;
+    bq_llgrad_kernel<TSMEM><<<n_rows, LLG_NT, bytes, stream>>>(a);
+    return cudaGetLastError();
+}
+
+// Rows [a.e0, a.e0 + n_rows): one launch while the triangle fits shared memory, else launches of at most work_inst CTAs
+// on the global scratch a.work (work_inst triangles of a.work_stride doubles).  *launches counts the kernel launches.
+cudaError_t launch_llgrad(LLGradArgs a, int n_rows, int work_inst, cudaStream_t stream, int *launches) {
+    const size_t bytes_sm = sizeof(double) * (size_t)llg_smem_doubles(a.n_max, a.nc_max, true);
+    *launches = 0;
+    if (bytes_sm <= S2_CTA_SMEM_MAX) {
+        *launches = 1;
+        return launch_llgrad_one<true>(a, n_rows, bytes_sm, stream);
+    }
+    const int n_big = a.n_max;
+    if (!a.work || a.work_stride < (size_t)tri(n_big) || work_inst < 1) return cudaErrorInvalidValue;
+    const size_t bytes = sizeof(double) * (size_t)llg_smem_doubles(a.n_max, a.nc_max, false);
+    const int end = a.e0 + n_rows;
+    for (int e0 = a.e0; e0 < end; e0 += work_inst) {
+        a.e0 = e0;
+        cudaError_t e = launch_llgrad_one<false>(a, end - e0 < work_inst ? end - e0 : work_inst, bytes, stream);
+        ++*launches;
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
 }  // namespace bqb

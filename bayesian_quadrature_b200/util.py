@@ -242,6 +242,131 @@ def slice_sample_batch(logpdf, x0, n, w, keys, nburn=1, max_steps=None, stats=No
     return samples[:, nburn:]
 
 
+def _rowdot(a, b):
+    """Row-wise dot products of two [r, d] arrays, one column at a time (a row's arithmetic does not depend on r)."""
+    s = a[:, 0] * b[:, 0]
+    for c in range(1, a.shape[1]):
+        s = s + a[:, c] * b[:, c]
+    return s
+
+
+def lbfgs_batch(fg, x0, maxiter=200, m=10, gtol=1e-5, ftol=2.2e-9, max_backtrack=20):
+    """Maximise many independent smooth functions in lock-step with L-BFGS (memory ``m``) and a backtracking Armijo line
+    search.  Row p starts at x0[p] ([P, d]).
+
+    ``fg(X, rows)`` returns (f [r], g [r, d]), the values and gradients at the points X [r, d] of the rows ``rows`` (an
+    index array); it is called once per step with the rows that are still running, each at its own trial point.  A trial
+    whose value is -inf or NaN (or whose gradient is not finite) counts as a failed step: the step is halved.  The first
+    step of a row (and the first after its history was reset) has length at most 1.  When ``max_backtrack`` trials of
+    one step fail, the row forgets its history and searches once more along the steepest direction, as scipy's L-BFGS-B
+    restarts; the default of 20 trials per line search is scipy's ``maxls``.
+
+    A row stops, as scipy's L-BFGS-B does by default, when the largest gradient entry is at most ``gtol`` or when an
+    accepted step changed f by at most ``ftol * max(|f_old|, |f_new|, 1)``: it has then converged.  It also stops, not
+    converged, after ``maxiter`` iterations or when the line search fails along the steepest direction too.  Every row uses only its own values
+    and row-wise arithmetic, so its result does not depend on the other rows.
+
+    A start whose value is -inf or NaN raises RuntimeError with the attribute ``row``.  Returns a dict: x [P, d], f [P],
+    converged [P] (bool), iterations [P], evaluations (points evaluated, all rows together) and calls (calls of fg)."""
+    x = np.array(x0, dtype=DTYPE, ndmin=2)
+    P, d = x.shape
+    rows_all = np.arange(P)
+    f, g = fg(x.copy(), rows_all)
+    f, g = np.asarray(f, dtype=DTYPE).reshape(P), np.asarray(g, dtype=DTYPE).reshape(P, d)
+    bad = ~np.isfinite(f)
+    if bad.any():
+        err = RuntimeError("zero probability at the start of row %d" % int(np.argmax(bad)))
+        err.row = int(np.argmax(bad))
+        raise err
+    phi, G = -f, -g                                      # minimise phi = -f
+    S, Y = np.zeros((P, m, d)), np.zeros((P, m, d))
+    rho = np.zeros((P, m))
+    nh = np.zeros(P, dtype=np.int64)                     # stored pairs
+    head = np.zeros(P, dtype=np.int64)                   # slot of the next pair
+    iters = np.zeros(P, dtype=np.int64)
+    converged = np.abs(G).max(axis=1) <= gtol
+    active = np.isfinite(G).all(axis=1) & ~converged
+    p, t, slope, nbt = np.zeros((P, d)), np.zeros(P), np.zeros(P), np.zeros(P, dtype=np.int64)
+    evaluations, calls = P, 1
+
+    def direction(sel):
+        """-H G for the rows sel (two-loop recursion over each row's own history), the step length and the slope."""
+        r = sel.size
+        q = G[sel].copy()
+        al = np.zeros((r, m))
+        for age in range(m):
+            slot = (head[sel] - 1 - age) % m
+            v = age < nh[sel]
+            s_, y_ = S[sel, slot], Y[sel, slot]
+            a = np.where(v, rho[sel, slot] * _rowdot(s_, q), 0.0)
+            al[:, age] = a
+            q = q - a[:, None] * y_
+        newest = (head[sel] - 1) % m
+        sy, yy = _rowdot(S[sel, newest], Y[sel, newest]), _rowdot(Y[sel, newest], Y[sel, newest])
+        gam = np.where(nh[sel] > 0, sy / np.where(nh[sel] > 0, yy, 1.0), 1.0)
+        z = gam[:, None] * q
+        for age in reversed(range(m)):
+            slot = (head[sel] - 1 - age) % m
+            v = age < nh[sel]
+            s_, y_ = S[sel, slot], Y[sel, slot]
+            b = rho[sel, slot] * _rowdot(y_, z)
+            z = z + np.where(v, al[:, age] - b, 0.0)[:, None] * s_
+        pd_ = -z
+        sl = _rowdot(G[sel], pd_)
+        uphill = ~(sl < 0)                               # not a descent direction: forget the history
+        if uphill.any():
+            nh[sel[uphill]] = 0
+            pd_[uphill] = -G[sel[uphill]]
+            sl[uphill] = _rowdot(G[sel[uphill]], pd_[uphill])
+        p[sel], slope[sel], nbt[sel] = pd_, sl, 0
+        norm = np.sqrt(_rowdot(pd_, pd_))
+        t[sel] = np.where(nh[sel] == 0, np.minimum(1.0, 1.0 / norm), 1.0)
+
+    if active.any():
+        direction(np.nonzero(active)[0])
+    while active.any():
+        sel = np.nonzero(active)[0]
+        xt = x[sel] + t[sel, None] * p[sel]
+        ft, gt = fg(xt.copy(), sel)
+        ft, gt = np.asarray(ft, dtype=DTYPE).reshape(sel.size), np.asarray(gt, dtype=DTYPE).reshape(sel.size, d)
+        evaluations += sel.size
+        calls += 1
+        pt = -ft
+        with np.errstate(invalid="ignore"):
+            ok = np.isfinite(pt) & np.isfinite(gt).all(axis=1) & (pt <= phi[sel] + 1e-4 * t[sel] * slope[sel])
+        acc, rej = sel[ok], sel[~ok]
+        if rej.size:
+            t[rej] *= 0.5
+            nbt[rej] += 1
+            failed = rej[nbt[rej] >= max_backtrack]
+            retry = failed[nh[failed] > 0]                   # forget the history, search along -G once more
+            active[failed[nh[failed] == 0]] = False
+            if retry.size:
+                nh[retry] = 0
+                direction(retry)
+        if acc.size:
+            s_ = xt[ok] - x[acc]
+            y_ = -gt[ok] - G[acc]
+            phi_old = phi[acc]
+            x[acc], phi[acc], G[acc] = xt[ok], pt[ok], -gt[ok]
+            iters[acc] += 1
+            sy, yy = _rowdot(s_, y_), _rowdot(y_, y_)
+            keep = sy > 2.2e-16 * yy                     # curvature condition; otherwise the pair is skipped
+            ka = acc[keep]
+            S[ka, head[ka]], Y[ka, head[ka]], rho[ka, head[ka]] = s_[keep], y_[keep], 1.0 / sy[keep]
+            head[ka] = (head[ka] + 1) % m
+            nh[ka] = np.minimum(nh[ka] + 1, m)
+            done = ((np.abs(G[acc]).max(axis=1) <= gtol)
+                    | (phi_old - phi[acc] <= ftol * np.maximum(np.maximum(np.abs(phi_old), np.abs(phi[acc])), 1.0)))
+            converged[acc[done]] = True
+            active[acc[done | (iters[acc] >= maxiter)]] = False
+            nxt = acc[active[acc]]
+            if nxt.size:
+                direction(nxt)
+    return {"x": x, "f": -phi, "converged": converged, "iterations": iters, "evaluations": int(evaluations),
+            "calls": int(calls)}
+
+
 def find_good_parameters(logpdf, x0, method, ntry=10):
     """Maximise `logpdf` with scipy (util.py:151-169): up to `ntry` restarts, returns None when no
     restart reaches a log-density above MIN."""

@@ -96,6 +96,17 @@ int bqb_batch_stage(bqb_batch *b, const int *ns, const double *x_s, const double
  * the hyper-parameter log-density costs (BQ._make_llh_params, bq.py:533-552: _set_gp_log_l_params :933-957 +
  * _set_gp_l_params :959-965 + gp.log_lh) -- no buffer is reallocated, nothing but 48 bytes per instance is uploaded. */
 int bqb_batch_set_hypers(bqb_batch *b, const double *hyp, void *stream);
+/* Value and gradient of the joint log marginal likelihood that BQ._make_llh_params / BQ.fit_hypers maximise
+ * (bq.py:533-562: gp_log_l.log_lh + gp_l.log_lh after l_c is recomputed from the candidates) for n_eval rows, each an
+ * instance under its own hyper-parameters.  hyp [n_eval][6] (h, w, s of gp_log_l, then of gp_l), inst [n_eval] (instance
+ * of each row; NULL: row e is instance e, n_eval <= n_inst) and the outputs are HOST arrays: log_lh_out [n_eval],
+ * grad_out [n_eval][6] (d log_lh / d of the six hyper-parameters, in the order of hyp) and status_out [n_eval] (the setup
+ * status codes; a row that is not OK has log_lh -inf and a NaN gradient).  check_max applies the "GP mean is too large"
+ * guard (bq.py:942-947).  Reads the staged observations and candidates; leaves the model blocks and the batch's own
+ * hyper-parameters untouched, so the scoring model stays valid.  Gaussian kernel only (BQB_EUNSUPPORTED after
+ * bqb_batch_set_approx with the periodic kernel); BQB_ESTATE when nothing is staged.  Synchronises `stream`. */
+int bqb_batch_log_lh_grad(bqb_batch *b, const double *hyp, const int *inst, int n_eval, int check_max, double *log_lh_out,
+                          double *grad_out, int *status_out, void *stream);
 /* Non-Gaussian kernels and the trapezoid approximation.  Replaces gp.PeriodicKernel as used by bq.py:139-165 and
  * bq_c.approx_Z_mean (bq_c.pyx:216-261), approx_Z_var (:358-422), approx_expected_squared_mean_and_mean (:538-598),
  * i.e. what BQ does when options['use_approx'] is set (bq.py:251-252, :310-311, :498-510).
