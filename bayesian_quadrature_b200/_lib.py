@@ -33,12 +33,15 @@ SYMBOLS = {
     "bqb_batch_stage": (ctypes.c_int, [_vp, _ip, _dp, _dp, ctypes.c_int, _dp, _dp, _vp]),
     "bqb_batch_set_hypers": (ctypes.c_int, [_vp, _dp, _vp]),
     "bqb_batch_log_lh_grad": (ctypes.c_int, [_vp, _dp, _ip, ctypes.c_int, ctypes.c_int, _dp, _dp, _ip, _vp]),
+    "bqb_batch_log_lh_grad_periodic": (ctypes.c_int, [_vp, _dp, _dp, _ip, ctypes.c_int, ctypes.c_int, _dp, _dp, _ip, _vp]),
+    "bqb_batch_set_periods": (ctypes.c_int, [_vp, _dp, _vp]),
     "bqb_batch_set_approx": (ctypes.c_int, [_vp, ctypes.c_int, _dp, _dp, _dp, ctypes.c_int, _ll, ctypes.c_int]),
     "bqb_batch_setup_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp]),
     "bqb_batch_seed_candidates": (ctypes.c_int, [_vp, ctypes.POINTER(ctypes.c_uint), _vp]),
     "bqb_batch_rng_get": (ctypes.c_int, [_vp, ctypes.POINTER(ctypes.c_uint), _ip]),
     "bqb_batch_rng_set": (ctypes.c_int, [_vp, ctypes.POINTER(ctypes.c_uint), _ip]),
     "bqb_batch_draw_candidates": (ctypes.c_int, [_vp, ctypes.c_int, _vp]),
+    "bqb_batch_draw_candidates_wrapped": (ctypes.c_int, [_vp, ctypes.c_int, _vp]),
     "bqb_batch_add_observations": (ctypes.c_int, [_vp, _vp, _vp, _vp]),
     "bqb_batch_get_staged": (ctypes.c_int, [_vp, _ip, _ip, _dp, _dp, _dp]),
     "bqb_batch_capacity": (ctypes.c_int, [_vp]),
@@ -217,6 +220,30 @@ class Batch(object):
                                             _vp(stream) if stream else None), "bqb_batch_log_lh_grad")
         return llh, grad, st
 
+    def log_lh_grad_periodic(self, hyp, period, inst=None, check_max=True, stream=None):
+        """log_lh_grad for a batch of the periodic kernel: row r also has its periods period[r] = (p of gp_log_l, p of gp_l).
+        Returns (log_lh [n], grad [n, 8], status [n]), the gradient in the order h_tl, w_tl, s_tl, h_l, w_l, s_l, p_tl, p_l."""
+        hyp = _d(hyp).reshape(-1, 6)
+        n = hyp.shape[0]
+        period = _d(period).reshape(-1, 2)
+        if period.shape[0] != n:
+            raise ValueError("period must have one row per row of hyp")
+        if inst is not None:
+            inst = np.ascontiguousarray(inst, dtype=np.int32).reshape(-1)
+            if inst.shape[0] != n:
+                raise ValueError("inst must have one entry per row of hyp")
+        llh, grad, st = np.empty(n), np.empty((n, 8)), np.empty(n, dtype=np.int32)
+        _check(load().bqb_batch_log_lh_grad_periodic(self._h, _pd(hyp), _pd(period),
+                                                     inst.ctypes.data_as(_ip) if inst is not None else None, n, int(check_max),
+                                                     _pd(llh), _pd(grad), st.ctypes.data_as(_ip), _vp(stream) if stream else None),
+               "bqb_batch_log_lh_grad_periodic")
+        return llh, grad, st
+
+    def set_periods(self, period, stream=None):
+        """Replace the periods [n_inst, 2] of a batch of the periodic kernel (the next setup_device uses them)."""
+        period = _d(period).reshape(self.n_inst, 2)
+        _check(load().bqb_batch_set_periods(self._h, _pd(period), _vp(stream) if stream else None), "bqb_batch_set_periods")
+
     def set_approx(self, kernel_kind=0, period=None, xo=None, p_xo=None, force_generic=False):
         """Kernel kind (0 Gaussian, 1 periodic with period [n_inst, 2] = p of gp_log_l / gp_l) and, when ``xo`` / ``p_xo``
         are given ([n_xo] shared or [n_inst, n_xo]), the trapezoid approximation of the integrals over that grid
@@ -268,6 +295,11 @@ class Batch(object):
     def draw_candidates(self, n_candidate, stream=None):
         _check(load().bqb_batch_draw_candidates(self._h, int(n_candidate), _vp(stream) if stream else None),
                "bqb_batch_draw_candidates")
+
+    def draw_candidates_wrapped(self, n_candidate, stream=None):
+        """draw_candidates on [-pi p_tl, pi p_tl] (periodic kernel)."""
+        _check(load().bqb_batch_draw_candidates_wrapped(self._h, int(n_candidate), _vp(stream) if stream else None),
+               "bqb_batch_draw_candidates_wrapped")
 
     def add_observations(self, x_new, l_new, stream=None):
         """x_new, l_new: float64 CUDA tensors [n_inst]."""

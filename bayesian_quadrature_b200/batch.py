@@ -16,6 +16,11 @@ step (``log_lh``), and ``marginal_loss`` scores the P x S (problem, sample) inst
 draws from its own counter-based stream keyed by the pair (seed, p) (the reference's single global libc ``rand`` stream
 cannot be split per problem; SURVEY appendix A.4 documents the same choice for the candidate streams).
 
+``kernel=PeriodicKernel`` runs every problem with the periodic kernel, as ``BQ(kernel=PeriodicKernel)`` does: the
+parameters of a GP are (h, w, p, s), candidates are drawn on [-pi p_tl, pi p_tl] (bq.py:217-218), and the integrals are
+trapezoid sums over the 1000-point grid of that range with the von Mises prior density (``BQ._approx``), built at
+``init`` from the p_tl of that moment.
+
 All per-problem bookkeeping is numpy-vectorised over the batch; scoring, the per-problem argmin
 and the model setup run on the device through the C-ABI.
 """
@@ -26,10 +31,15 @@ import numpy as np
 
 from . import _lib
 from . import util
-from .bq import _SETUP_ERRORS
+from .bq import _SETUP_ERRORS, _vonmises_px
+from .gp import GaussianKernel, PeriodicKernel
 
 logger = logging.getLogger("bayesian_quadrature")
 _NAMES = ("h", "w", "s")                     # GaussianKernel parameters, then the noise: columns of one GP's (h, w, s)
+_NAMES_PERIODIC = ("h", "w", "p", "s")       # PeriodicKernel parameters, then the noise (BQ.init's params_tl / params_l)
+# columns (of gp_log_l, of gp_l) of a parameter in a row of hyper-parameters: hyp [6], then for the periodic kernel period [2]
+_COLS = {"h": (0, 3), "w": (1, 4), "s": (2, 5), "p": (6, 7)}
+N_GRID = 1000                                # points of the approximation grid (bq.py:167-171)
 
 
 def filter_candidates_batch(x_c, x_s, ns, thresh):
@@ -73,9 +83,13 @@ def filter_candidates_batch(x_c, x_s, ns, thresh):
 
 class BatchBQ(object):
     def __init__(self, x_s, l_s, params_tl, params_l, n_candidate, candidate_thresh, x_mean, x_var, seed=0,
-                 device=0, ns_reserve=0, device_resident=False):
+                 device=0, ns_reserve=0, device_resident=False, kernel=GaussianKernel):
         """x_s, l_s: [P, ns0] initial observations; params_*: (h, w, s) shared by all problems or [P, 3];
         x_mean / x_var scalars or [P].  ``ns_reserve`` extra observation slots are pre-allocated.
+
+        ``kernel`` is GaussianKernel or PeriodicKernel; with PeriodicKernel params_* are (h, w, p, s) or [P, 4], the
+        periods are kept in ``self.period`` [P, 2] (p of gp_log_l, of gp_l) next to ``self.hyp`` [P, 6], and x_mean /
+        x_var are the mean and the inverse concentration of the von Mises prior.
 
         ``device_resident=True`` keeps the observations, the candidate generators (one MT19937 stream per problem,
         bit-identical to ``np.random.RandomState(seed + p)``) and the candidate filter on the GPU: a round then moves
@@ -92,7 +106,16 @@ class BatchBQ(object):
         self.l_s = np.ones((self.P, self.cap)); self.l_s[:, :ns0] = l_s
         self.ns = np.full(self.P, ns0, dtype=np.int32)
         bc = lambda v, k: np.ascontiguousarray(np.broadcast_to(np.asarray(v, dtype=np.float64), (self.P, k)))
-        self.hyp = np.concatenate([bc(params_tl, 3), bc(params_l, 3)], axis=1)
+        if kernel not in (GaussianKernel, PeriodicKernel):
+            raise ValueError("kernel must be GaussianKernel or PeriodicKernel")
+        self.periodic = kernel is PeriodicKernel
+        self._names = _NAMES_PERIODIC if self.periodic else _NAMES
+        if self.periodic:
+            ptl, pl = bc(params_tl, 4), bc(params_l, 4)
+            self.hyp = np.ascontiguousarray(np.concatenate([ptl[:, [0, 1, 3]], pl[:, [0, 1, 3]]], axis=1))
+            self.period = np.ascontiguousarray(np.stack([ptl[:, 2], pl[:, 2]], axis=1))
+        else:
+            self.hyp = np.concatenate([bc(params_tl, 3), bc(params_l, 3)], axis=1)
         self.prior = np.stack([bc(x_mean, 1)[:, 0], bc(x_var, 1)[:, 0], np.full(self.P, float(candidate_thresh))], axis=1)
         self.n_candidate, self.thresh = int(n_candidate), float(candidate_thresh)
         if self.n_candidate > _lib.NC_MAX:
@@ -137,7 +160,11 @@ class BatchBQ(object):
             stride = min(self.cap, cap_class)
             self.batch.stage(self.ns, self.x_s[:, :stride], self.l_s[:, :stride], self.hyp, self.prior)
             self.batch.seed_candidates((self.seed + np.arange(self.P)) & 0xffffffff)
-        self.batch.draw_candidates(self.n_candidate)
+        if self.periodic:
+            self._apply_approx()
+            self.batch.draw_candidates_wrapped(self.n_candidate)
+        else:
+            self.batch.draw_candidates(self.n_candidate)
         info = self._check_info(self.batch.setup_device())
         self._host_stale = True
         return info
@@ -168,14 +195,31 @@ class BatchBQ(object):
         self._cap_class = cap_class
         self.batch.stage(st["ns"], st["x_s"], st["l_s"], self.hyp, self.prior)
         self.batch.rng_set(mt, pos)
+        if self.periodic:
+            self.batch.set_approx(1, period=self.period, xo=self.xo, p_xo=self.p_xo)
+
+    def _apply_approx(self):
+        """Periodic kernel: the grid of every problem from its current p_tl (``BQ._approx`` as of init: np.linspace of
+        [-pi p_tl, pi p_tl], the von Mises density on it) and its upload, with the periods, to the device batch."""
+        mu, var = self.prior[:, 0], self.prior[:, 1]
+        self.xo = np.empty((self.P, N_GRID))
+        self.p_xo = np.empty((self.P, N_GRID))
+        for p in range(self.P):                            # BQ's scalar expressions, so that the grids are the same bits
+            p_tl = float(self.period[p, 0])
+            self.xo[p] = np.linspace(-1 * np.pi * p_tl, +1 * np.pi * p_tl, N_GRID)
+            self.p_xo[p] = _vonmises_px(self.xo[p], float(mu[p]), float(var[p]))
+        self.batch.set_approx(1, period=self.period, xo=self.xo, p_xo=self.p_xo)
 
     def init(self):
         if self.device_resident:
             return self._init_device()
-        w_tl = self.hyp[:, 1]
-        idx = np.arange(self.cap)[None, :] < self.ns[:, None]
-        lo = np.where(idx, self.x_s, np.inf).min(axis=1) - w_tl
-        hi = np.where(idx, self.x_s, -np.inf).max(axis=1) + w_tl
+        if self.periodic:
+            lo, hi = -np.pi * self.period[:, 0], np.pi * self.period[:, 0]      # bq.py:217-218
+        else:
+            w_tl = self.hyp[:, 1]
+            idx = np.arange(self.cap)[None, :] < self.ns[:, None]
+            lo = np.where(idx, self.x_s, np.inf).min(axis=1) - w_tl
+            hi = np.where(idx, self.x_s, -np.inf).max(axis=1) + w_tl
         xc = np.stack([self.rngs[p].uniform(lo[p], hi[p], self.n_candidate) for p in range(self.P)])
         filter_candidates_batch(xc, self.x_s, self.ns, self.thresh)
         xc.sort(axis=1)                                   # NaNs sort last
@@ -189,6 +233,8 @@ class BatchBQ(object):
             self.close()
             self.batch = _lib.Batch(self.P, cap_class, device=self.device)
             self._cap_class = cap_class
+        if self.periodic:
+            self._apply_approx()
         stride = min(self.cap, cap_class)
         info = self.batch.setup(self.ns, self.nc, self.x_s[:, :stride], self.l_s[:, :stride], self.x_c, self.hyp, self.prior)
         return self._check_info(info)
@@ -200,27 +246,55 @@ class BatchBQ(object):
         return self.info["Z_var"]
 
     # ---------------------------------------------------------------- hyper-parameter samples (bq.py:533-598)
+    def _rows(self):
+        """The batch's hyper-parameter rows: hyp [P, 6], with the periodic kernel [P, 8] = (hyp, period)."""
+        return np.concatenate([self.hyp, self.period], axis=1) if self.periodic else self.hyp
+
+    def _set_rows(self, rows):
+        self.hyp[:] = rows[:, :6]
+        if self.periodic:
+            self.period[:] = rows[:, 6:]
+
+    def _upload_rows(self, rows):
+        """Hyper-parameter rows [P, 6 | 8] to the device batch (the next setup_device uses them)."""
+        self.batch.set_hypers(rows[:, :6])
+        if self.periodic:
+            self.batch.set_periods(rows[:, 6:])
+
+    def _cols(self, params):
+        """(columns of gp_log_l, columns of gp_l) of the named parameters in a hyper-parameter row."""
+        bad = [p for p in params if p not in self._names]
+        if not params or bad:
+            raise ValueError("unknown hyper-parameter in %s (BatchBQ has %s)" % (list(params), ", ".join(self._names)))
+        return [_COLS[p][0] for p in params], [_COLS[p][1] for p in params]
+
     def _hyp_rows(self, hypers_tl, hypers_l, params):
-        """[..., 6] hyper-parameter rows (h, w, s of gp_log_l, then of gp_l): the batch's own with the named entries
-        replaced by hypers_tl / hypers_l [P, ..., len(params)]."""
+        """[..., 6] hyper-parameter rows (h, w, s of gp_log_l, then of gp_l; with the periodic kernel [..., 8], the periods
+        p_tl, p_l last): the batch's own with the named entries replaced by hypers_tl / hypers_l [P, ..., len(params)]."""
         hypers_tl, hypers_l = np.asarray(hypers_tl, dtype=np.float64), np.asarray(hypers_l, dtype=np.float64)
         k = len(params)
         if hypers_tl.shape != hypers_l.shape or hypers_tl.shape[0] != self.P or hypers_tl.shape[-1] != k:
             raise ValueError("hypers_tl and hypers_l must be [P, ..., %d] arrays of the same shape" % k)
         mid = hypers_tl.shape[1:-1]
-        hyp = np.array(np.broadcast_to(self.hyp.reshape((self.P,) + (1,) * len(mid) + (6,)), (self.P,) + mid + (6,)))
+        base = self._rows()
+        w = base.shape[1]
+        hyp = np.array(np.broadcast_to(base.reshape((self.P,) + (1,) * len(mid) + (w,)), (self.P,) + mid + (w,)))
         for j, name in enumerate(params):
-            if name not in _NAMES:
-                raise ValueError("unknown hyper-parameter %r (BatchBQ has %s)" % (name, ", ".join(_NAMES)))
-            c = _NAMES.index(name)
-            hyp[..., c], hyp[..., 3 + c] = hypers_tl[..., j], hypers_l[..., j]
+            if name not in self._names:
+                raise ValueError("unknown hyper-parameter %r (BatchBQ has %s)" % (name, ", ".join(self._names)))
+            ct, cl = _COLS[name]
+            hyp[..., ct], hyp[..., cl] = hypers_tl[..., j], hypers_l[..., j]
         return hyp
 
     @staticmethod
     def _valid_hyp(hyp):
-        """The values GP.set_param accepts: finite, h and w positive, s non-negative."""
-        return (np.isfinite(hyp).all(axis=-1) & (hyp[..., [0, 1, 3, 4]] > 0).all(axis=-1)
-                & (hyp[..., [2, 5]] >= 0).all(axis=-1))
+        """The values GP.set_param accepts: finite, h and w positive, s non-negative (and the periods of [..., 8] rows
+        positive)."""
+        ok = (np.isfinite(hyp).all(axis=-1) & (hyp[..., [0, 1, 3, 4]] > 0).all(axis=-1)
+              & (hyp[..., [2, 5]] >= 0).all(axis=-1))
+        if hyp.shape[-1] == 8:
+            ok &= (hyp[..., 6:] > 0).all(axis=-1)
+        return ok
 
     def log_lh(self, hypers_tl, hypers_l, params):
         """Joint log marginal likelihood ``gp_log_l.log_lh + gp_l.log_lh`` of every problem under its own proposal
@@ -234,23 +308,26 @@ class BatchBQ(object):
         (the setup is deterministic, so the scoring model, Z_mean and Z_var are exactly what they were)."""
         hyp = self._hyp_rows(hypers_tl, hypers_l, params)
         ok = self._valid_hyp(hyp)
-        hyp[~ok] = self.hyp[~ok]                          # rows the device must not see; their result is -inf
+        hyp[~ok] = self._rows()[~ok]                      # rows the device must not see; their result is -inf
         try:
-            self.batch.set_hypers(hyp)
+            self._upload_rows(hyp)
             info = self.batch.setup_device(check_max=True)
         finally:
-            self.batch.set_hypers(self.hyp)
+            self._upload_rows(self._rows())
             self._check_info(self.batch.setup_device())
         return np.where(ok & (info["status"] == _lib.SETUP_OK) & np.isfinite(info["log_lh"]), info["log_lh"], -np.inf)
 
     def _log_lh_grad_rows(self, rows, hyp):
-        """(log_lh [r], grad [r, 6]) of the problems ``rows`` under the hyper-parameter rows hyp [r, 6], with the -inf
-        semantics of log_lh (the gradient is NaN there).  Only the valid rows reach the device."""
+        """(log_lh [r], grad [r, 6 | 8]) of the problems ``rows`` under the hyper-parameter rows hyp [r, 6 | 8], with the
+        -inf semantics of log_lh (the gradient is NaN there).  Only the valid rows reach the device."""
         rows = np.asarray(rows, dtype=np.int64)
-        ll, grad = np.full(rows.size, -np.inf), np.full((rows.size, 6), np.nan)
+        ll, grad = np.full(rows.size, -np.inf), np.full((rows.size, hyp.shape[1]), np.nan)
         ok = self._valid_hyp(hyp)
         if ok.any():
-            l, g, st = self.batch.log_lh_grad(hyp[ok], inst=rows[ok], check_max=True)
+            if self.periodic:
+                l, g, st = self.batch.log_lh_grad_periodic(hyp[ok, :6], hyp[ok, 6:], inst=rows[ok], check_max=True)
+            else:
+                l, g, st = self.batch.log_lh_grad(hyp[ok], inst=rows[ok], check_max=True)
             good = (st == _lib.SETUP_OK) & np.isfinite(l)
             idx = np.nonzero(ok)[0][good]
             ll[idx], grad[idx] = l[good], g[good]
@@ -266,8 +343,8 @@ class BatchBQ(object):
         if hyp.ndim != 2:
             raise ValueError("hypers_tl and hypers_l must be [P, %d]" % len(params))
         ll, g = self._log_lh_grad_rows(np.arange(self.P), hyp)
-        cols = [_NAMES.index(p) for p in params]
-        return ll, g[:, cols], g[:, [3 + c for c in cols]]
+        ct, cl = self._cols(params)
+        return ll, g[:, ct], g[:, cl]
 
     def fit_hypers(self, params, maxiter=200):
         """Maximise every problem's joint log marginal likelihood over the named parameters of both GPs
@@ -279,26 +356,27 @@ class BatchBQ(object):
         A problem whose start has zero probability raises RuntimeError naming it, before anything changes.  Fitting "s"
         needs s > 0 at the start for both GPs of every problem (ValueError otherwise).  Returns a dict: log_lh [P] at the
         fitted point, converged [P], iterations [P] and evaluations (problem evaluations in total)."""
-        cols = [_NAMES.index(p) if p in _NAMES else -1 for p in params]
-        if not params or min(cols) < 0:
-            raise ValueError("unknown hyper-parameter in %s (BatchBQ has %s)" % (params, ", ".join(_NAMES)))
-        cols6 = cols + [3 + c for c in cols]
-        if not (self.hyp[:, cols6] > 0).all():
+        ct, cl = self._cols(params)
+        cols6 = ct + cl
+        start = self._rows()
+        if not (start[:, cols6] > 0).all():
             raise ValueError("fitting %s needs positive starting values (it works with their logarithms)" % list(params))
 
         def fg(X, rows):
-            hyp = self.hyp[rows].copy()
+            hyp = start[rows].copy()
             hyp[:, cols6] = np.exp(X)
             ll, g = self._log_lh_grad_rows(rows, hyp)
             return ll, g[:, cols6] * hyp[:, cols6]           # d ll / d log(theta)
         try:
-            res = util.lbfgs_batch(fg, np.log(self.hyp[:, cols6]), maxiter=maxiter)
+            res = util.lbfgs_batch(fg, np.log(start[:, cols6]), maxiter=maxiter)
         except RuntimeError as e:
             if getattr(e, "row", None) is None:
                 raise
             raise RuntimeError("problem %d: zero probability at the starting hyper-parameters" % e.row) from e
-        self.hyp[:, cols6] = np.exp(res["x"])
-        self.batch.set_hypers(self.hyp)
+        fitted = start.copy()
+        fitted[:, cols6] = np.exp(res["x"])
+        self._set_rows(fitted)
+        self._upload_rows(self._rows())
         self._check_info(self.batch.setup_device())
         return {"log_lh": res["f"], "converged": res["converged"], "iterations": res["iterations"],
                 "evaluations": res["evaluations"]}
@@ -314,10 +392,9 @@ class BatchBQ(object):
         whose start has zero probability raises RuntimeError (the reference would search for better starting parameters
         instead)."""
         k = len(params)
-        cols = [_NAMES.index(p) if p in _NAMES else -1 for p in params]
-        if min(cols + [0]) < 0:
-            raise ValueError("unknown hyper-parameter in %s (BatchBQ has %s)" % (params, ", ".join(_NAMES)))
-        x0 = np.concatenate([self.hyp[:, cols], self.hyp[:, [3 + c for c in cols]]], axis=1)
+        ct, cl = self._cols(params) if k else ([], [])
+        rows = self._rows()
+        x0 = np.concatenate([rows[:, ct], rows[:, cl]], axis=1)
         f = lambda X: self.log_lh(X[:, :k], X[:, k:], params)
         keys = util.stream_keys(seed, int(first_problem) + np.arange(self.P))
         try:
@@ -346,6 +423,8 @@ class BatchBQ(object):
     def _chunks(self, S, na):
         """(problems per setup chunk, problems per scoring launch) under MODEL_CHUNK_BYTES / LOSS_CHUNK_BYTES."""
         model_bytes = 8 * _lib.load().bqb_model_doubles(self.batch._h)
+        if self.periodic:
+            model_bytes += 8 * (3 * N_GRID + 2)           # grid, prior density, trapezoid weights and periods per instance
         per_score = max(1, min(self.P, self.LOSS_CHUNK_BYTES // max(8 * S * max(na, 1), 1)))
         per_setup = max(1, min(self.P, self.MODEL_CHUNK_BYTES // (S * model_bytes)))
         if per_setup >= per_score:
@@ -404,8 +483,11 @@ class BatchBQ(object):
             rep = lambda a: np.repeat(a[p0:p0 + cp], S, axis=0)
             batch = self._sample_batch(cp * S)
             t0 = time.perf_counter()
+            hrows = hyp[p0:p0 + cp].reshape(cp * S, hyp.shape[-1])
+            if self.periodic:                             # each sample's periods, its problem's grid
+                batch.set_approx(1, period=hrows[:, 6:], xo=rep(self.xo), p_xo=rep(self.p_xo))
             info = batch.setup(rep(self.ns), rep(self.nc), rep(self.x_s[:, :stride]), rep(self.l_s[:, :stride]), rep(self.x_c),
-                               hyp[p0:p0 + cp].reshape(cp * S, 6), rep(self.prior), check_max=True)
+                               hrows[:, :6], rep(self.prior), check_max=True)
             bad = np.nonzero(info["status"])[0]
             if bad.size:
                 p, i = divmod(int(bad[0]), S)

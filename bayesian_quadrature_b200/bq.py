@@ -53,6 +53,15 @@ def _raise_setup(status):
     raise exc(msg)
 
 
+def _vonmises_px(x, mu, var):
+    """Prior density of the wrapped (periodic) mode on the grid x: bq_c.p_x_vonmises / vonmises_logpdf (bq_c.pyx:31-60)
+    with kappa = 1 / var.  The reference normalises with libc's j0 (the Bessel function of the FIRST kind), not I0: kept,
+    so that results stay identical."""
+    from scipy.special import j0
+    kappa = 1.0 / var
+    return np.exp(-np.log(2 * np.pi * j0(kappa)) + kappa * np.cos(np.asarray(x, dtype=DTYPE) - mu))
+
+
 class _DeviceModel(object):
     """The device-resident factors of ONE BQ object: a single-instance batch handle that lives as long as the
     observation capacity class does.  ``refresh`` re-stages the data only when observations / candidates / prior
@@ -715,11 +724,7 @@ class BQ(object):
         mu = float(self.options["x_mean"][0])
         var = float(self.options["x_cov"][0, 0])
         if self.options["wrapped"]:
-            # bq_c.p_x_vonmises / vonmises_logpdf (bq_c.pyx:31-60) with kappa = 1 / x_cov; the reference normalises with
-            # libc's j0 (the Bessel function of the FIRST kind), not I0: kept, so that results stay identical
-            from scipy.special import j0
-            kappa = 1.0 / var
-            return np.exp(-np.log(2 * np.pi * j0(kappa)) + kappa * np.cos(np.asarray(x, dtype=DTYPE) - mu))
+            return _vonmises_px(x, mu, var)
         return np.exp(-0.5 * (np.log(2 * np.pi) + np.log(var) + (x - mu) ** 2 / var))
 
     # ------------------------------------------------------------------ plotting (host, optional matplotlib)

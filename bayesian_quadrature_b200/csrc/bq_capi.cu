@@ -15,7 +15,7 @@
 
 namespace bqb {
 cudaError_t launch_setup2(const SetupArgs &a, int n_inst, cudaStream_t stream);
-cudaError_t launch_llgrad(LLGradArgs a, int n_rows, int work_inst, cudaStream_t stream, int *launches);
+cudaError_t launch_llgrad(LLGradArgs a, int n_rows, int work_inst, cudaStream_t stream, int *launches, int kind);
 int setup2_two_cta_limit(int nc_max);
 size_t setup2_scratch_stride(int cap);
 cudaError_t launch_score(const ScoreArgs &a, int n_inst, int sm_count, cudaStream_t stream, int *grid_x = nullptr);
@@ -41,6 +41,8 @@ cudaError_t launch_add_observations(double *x_s, double *l_s, int *ns, int strid
                                     const double *l_new, int P, int *overflow, cudaStream_t s);
 cudaError_t launch_draw_candidates(const double *x_s, const int *ns, int stride, const double *hyp, const double *prior,
                                    unsigned *mt, int *mti, int n_candidate, double *x_c, int *nc, int P, cudaStream_t s);
+cudaError_t launch_draw_candidates_wrapped(const double *x_s, const int *ns, int stride, const double *period, const double *prior,
+                                           unsigned *mt, int *mti, int n_candidate, double *x_c, int *nc, int P, cudaStream_t s);
 }  // namespace bqb
 
 using namespace bqb;
@@ -70,8 +72,8 @@ struct bqb_batch {
     bool big_class = false;            // capacity 512: no tensor-core scoring kernels
     double *d_period = nullptr, *d_xo = nullptr, *d_pxo = nullptr, *d_wp = nullptr, *d_gz = nullptr;
     int *d_inst_list = nullptr;        // setup launch groups (instances ordered by size class)
-    // bqb_batch_log_lh_grad: hyper-parameter rows, instance list and output rows (grown on demand)
-    double *d_llg_hyp = nullptr, *d_llg_out = nullptr;
+    // bqb_batch_log_lh_grad(_periodic): hyper-parameter rows, periods, instance list and output rows (grown on demand)
+    double *d_llg_hyp = nullptr, *d_llg_out = nullptr, *d_llg_period = nullptr;
     int *d_llg_inst = nullptr;
     size_t cap_llg = 0;
     // scoring: relevance cut-off (bq_score.cu, CUT_ARG; +inf = dense) and the optional executed-work counter
@@ -182,7 +184,8 @@ void bqb_batch_destroy(bqb_batch *b) {
     cudaSetDevice(b->device);
     void *ptrs[] = {b->d_models, b->d_tab, b->d_work, b->d_ns, b->d_nc, b->d_xs, b->d_ls, b->d_xc, b->d_hyp, b->d_prior,
                     b->d_xa, b->d_esm, b->d_em, b->d_st, b->d_red_val, b->d_red_idx, b->d_flags, b->d_mt, b->d_mti, b->d_overflow, b->d_work_ctr, b->d_xsorted, b->d_perm, b->d_iota, b->d_sort_tmp,
-                    b->d_period, b->d_xo, b->d_pxo, b->d_wp, b->d_gz, b->d_inst_list, b->d_llg_hyp, b->d_llg_out, b->d_llg_inst};
+                    b->d_period, b->d_xo, b->d_pxo, b->d_wp, b->d_gz, b->d_inst_list, b->d_llg_hyp, b->d_llg_out, b->d_llg_inst,
+                    b->d_llg_period};
     for (void *p : ptrs) if (p) cudaFree(p);
     for (cudaStream_t st : b->pipe) if (st) cudaStreamDestroy(st);
     if (b->h_flags) cudaFreeHost(b->h_flags);
@@ -341,15 +344,20 @@ int bqb_batch_set_hypers(bqb_batch *b, const double *hyp, void *stream) {
     return 0;
 }
 
-int bqb_batch_log_lh_grad(bqb_batch *b, const double *hyp, const int *inst, int n_eval, int check_max, double *log_lh_out,
-                          double *grad_out, int *status_out, void *stream) {
-    if (!b) return fail(BQB_EINVAL, "bqb_batch_log_lh_grad: null batch");
-    if (!b->staged) return fail(BQB_ESTATE, "bqb_batch_log_lh_grad: nothing staged (bqb_batch_stage / bqb_batch_setup first)");
-    if (n_eval < 0 || (n_eval > 0 && (!hyp || !log_lh_out || !grad_out || !status_out)) || (!inst && n_eval > b->n_inst))
-        return fail(BQB_EINVAL, "bqb_batch_log_lh_grad: bad arguments");
+// The gradient kernel on rows of (instance, hyper-parameters [, periods]): kind 0 writes grad [n][6], kind 1 grad [n][8]
+static int run_llgrad(bqb_batch *b, int kind, const char *who, const double *hyp, const double *period, const int *inst,
+                      int n_eval, int check_max, double *log_lh_out, double *grad_out, int *status_out, void *stream) {
+    const std::string name(who);
+    if (!b) return fail(BQB_EINVAL, name + ": null batch");
+    if (!b->staged) return fail(BQB_ESTATE, name + ": nothing staged (bqb_batch_stage / bqb_batch_setup first)");
+    if (n_eval < 0 || (n_eval > 0 && (!hyp || (kind && !period) || !log_lh_out || !grad_out || !status_out)) ||
+        (!inst && n_eval > b->n_inst))
+        return fail(BQB_EINVAL, name + ": bad arguments");
     for (int e = 0; inst && e < n_eval; ++e)
-        if (inst[e] < 0 || inst[e] >= b->n_inst) return fail(BQB_EINVAL, "bqb_batch_log_lh_grad: instance index out of range");
-    if (b->kind != 0) return fail(BQB_EUNSUPPORTED, "bqb_batch_log_lh_grad: only the Gaussian kernel is supported");
+        if (inst[e] < 0 || inst[e] >= b->n_inst) return fail(BQB_EINVAL, name + ": instance index out of range");
+    if (b->kind != kind)
+        return fail(BQB_EUNSUPPORTED, name + (kind ? ": the batch does not use the periodic kernel (bqb_batch_set_approx)"
+                                                   : ": only the Gaussian kernel is supported"));
     if (n_eval == 0) return 0;
     CU(cudaSetDevice(b->device));
     cudaStream_t s = (cudaStream_t)stream;
@@ -357,31 +365,59 @@ int bqb_batch_log_lh_grad(bqb_batch *b, const double *hyp, const int *inst, int 
     int rc = staged_sizes(b, s, &a.n_max, &a.nc_max);
     if (rc) return rc;
     if ((size_t)n_eval > b->cap_llg) {
-        for (void *p : {(void *)b->d_llg_hyp, (void *)b->d_llg_out, (void *)b->d_llg_inst}) if (p) cudaFree(p);
-        b->d_llg_hyp = b->d_llg_out = nullptr; b->d_llg_inst = nullptr; b->cap_llg = 0;
+        for (void *p : {(void *)b->d_llg_hyp, (void *)b->d_llg_out, (void *)b->d_llg_inst, (void *)b->d_llg_period}) if (p) cudaFree(p);
+        b->d_llg_hyp = b->d_llg_out = b->d_llg_period = nullptr; b->d_llg_inst = nullptr; b->cap_llg = 0;
         CU(cudaMalloc(&b->d_llg_hyp, sizeof(double) * 6 * (size_t)n_eval));
-        CU(cudaMalloc(&b->d_llg_out, sizeof(double) * LLG_OUT * (size_t)n_eval));
+        CU(cudaMalloc(&b->d_llg_out, sizeof(double) * LLG_OUT_PERIODIC * (size_t)n_eval));
+        CU(cudaMalloc(&b->d_llg_period, sizeof(double) * 2 * (size_t)n_eval));
         CU(cudaMalloc(&b->d_llg_inst, sizeof(int) * (size_t)n_eval));
         b->cap_llg = n_eval;
     }
     CU(cudaMemcpyAsync(b->d_llg_hyp, hyp, sizeof(double) * 6 * (size_t)n_eval, cudaMemcpyHostToDevice, s));
+    if (kind) CU(cudaMemcpyAsync(b->d_llg_period, period, sizeof(double) * 2 * (size_t)n_eval, cudaMemcpyHostToDevice, s));
     if (inst) CU(cudaMemcpyAsync(b->d_llg_inst, inst, sizeof(int) * (size_t)n_eval, cudaMemcpyHostToDevice, s));
     a.ns = b->d_ns; a.nc = b->d_nc; a.x_s = b->d_xs; a.l_s = b->d_ls; a.x_c = b->d_xc; a.in_stride = b->ns_cap;
     a.hyp = b->d_llg_hyp; a.inst = inst ? b->d_llg_inst : nullptr; a.e0 = 0; a.check_max = check_max;
     a.work = b->d_work; a.work_stride = b->work_stride; a.out = b->d_llg_out;
+    a.period = kind ? b->d_llg_period : nullptr;
     int launches = 0;
-    const cudaError_t e = launch_llgrad(a, n_eval, b->work_inst, s, &launches);
+    const cudaError_t e = launch_llgrad(a, n_eval, b->work_inst, s, &launches, kind);
     b->launches += launches;
     CU(e);
-    std::vector<double> h((size_t)n_eval * LLG_OUT);
+    const int nout = kind ? LLG_OUT_PERIODIC : LLG_OUT, ngrad = nout - 2;
+    std::vector<double> h((size_t)n_eval * nout);
     CU(cudaMemcpyAsync(h.data(), b->d_llg_out, sizeof(double) * h.size(), cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     for (int r = 0; r < n_eval; ++r) {
-        const double *o = &h[(size_t)r * LLG_OUT];
+        const double *o = &h[(size_t)r * nout];
         log_lh_out[r] = o[0];
-        memcpy(grad_out + (size_t)r * 6, o + 1, sizeof(double) * 6);
-        status_out[r] = (int)o[7];
+        memcpy(grad_out + (size_t)r * ngrad, o + 1, sizeof(double) * ngrad);
+        status_out[r] = (int)o[nout - 1];
     }
+    return 0;
+}
+
+int bqb_batch_log_lh_grad(bqb_batch *b, const double *hyp, const int *inst, int n_eval, int check_max, double *log_lh_out,
+                          double *grad_out, int *status_out, void *stream) {
+    return run_llgrad(b, 0, "bqb_batch_log_lh_grad", hyp, nullptr, inst, n_eval, check_max, log_lh_out, grad_out, status_out,
+                      stream);
+}
+
+int bqb_batch_log_lh_grad_periodic(bqb_batch *b, const double *hyp, const double *period, const int *inst, int n_eval,
+                                   int check_max, double *log_lh_out, double *grad_out, int *status_out, void *stream) {
+    return run_llgrad(b, 1, "bqb_batch_log_lh_grad_periodic", hyp, period, inst, n_eval, check_max, log_lh_out, grad_out,
+                      status_out, stream);
+}
+
+int bqb_batch_set_periods(bqb_batch *b, const double *period, void *stream) {
+    if (!b || !period) return fail(BQB_EINVAL, "bqb_batch_set_periods: null argument");
+    if (b->kind != 1 || !b->d_period)
+        return fail(BQB_ESTATE, "bqb_batch_set_periods: the batch does not use the periodic kernel (bqb_batch_set_approx first)");
+    CU(cudaSetDevice(b->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    CU(cudaMemcpyAsync(b->d_period, period, sizeof(double) * (size_t)b->n_inst * 2, cudaMemcpyHostToDevice, s));
+    CU(cudaStreamSynchronize(s));          // the host array may be pageable and is free to change after this call
+    b->ready = false;
     return 0;
 }
 
@@ -462,6 +498,22 @@ int bqb_batch_draw_candidates(bqb_batch *b, int n_candidate, void *stream) {
     CU(cudaSetDevice(b->device));
     CU(launch_draw_candidates(b->d_xs, b->d_ns, b->ns_cap, b->d_hyp, b->d_prior, b->d_mt, b->d_mti, n_candidate, b->d_xc,
                               b->d_nc, b->n_inst, (cudaStream_t)stream));
+    b->launches++;
+    b->ready = false;
+    b->counts_fresh = false;
+    return 0;
+}
+
+int bqb_batch_draw_candidates_wrapped(bqb_batch *b, int n_candidate, void *stream) {
+    if (!b || !b->staged) return fail(BQB_ESTATE, "bqb_batch_draw_candidates_wrapped: nothing staged");
+    if (!b->d_mt) return fail(BQB_ESTATE, "bqb_batch_draw_candidates_wrapped: generators were not seeded");
+    if (b->kind != 1 || !b->d_period)
+        return fail(BQB_ESTATE, "bqb_batch_draw_candidates_wrapped: the batch does not use the periodic kernel (bqb_batch_set_approx first)");
+    if (n_candidate < 0 || n_candidate > NC_MAX)
+        return fail(BQB_EUNSUPPORTED, "bqb_batch_draw_candidates_wrapped: more than 16 candidates");
+    CU(cudaSetDevice(b->device));
+    CU(launch_draw_candidates_wrapped(b->d_xs, b->d_ns, b->ns_cap, b->d_period, b->d_prior, b->d_mt, b->d_mti, n_candidate,
+                                      b->d_xc, b->d_nc, b->n_inst, (cudaStream_t)stream));
     b->launches++;
     b->ready = false;
     b->counts_fresh = false;

@@ -147,6 +147,7 @@ struct SetupArgs {
 // Arguments of one launch of the log-likelihood gradient kernel (bq_setup2.cu); shared with the C-ABI layer (bq_capi.cu).
 // It reads the staged inputs of a batch and writes nothing but `out`.
 constexpr int LLG_OUT = 8;     // doubles per output row: log_lh, d/d(h_tl, w_tl, s_tl, h_l, w_l, s_l), status
+constexpr int LLG_OUT_PERIODIC = 10;   // periodic kernel: log_lh, d/d(h_tl, w_tl, s_tl, h_l, w_l, s_l, p_tl, p_l), status
 struct LLGradArgs {
     const int *ns, *nc;
     const double *x_s, *l_s;   // [n_inst][in_stride] (in_stride = the batch's observation capacity)
@@ -159,7 +160,9 @@ struct LLGradArgs {
     int n_max, nc_max;         // largest ns + nc / nc over the batch's instances (size the shared memory)
     double *work;              // scratch per CTA for instances too large for shared memory (setup2_scratch_stride)
     size_t work_stride;
-    double *out;               // [n_eval][LLG_OUT]
+    double *out;               // [n_eval][LLG_OUT], periodic kernel [n_eval][LLG_OUT_PERIODIC]
+    const double *period;      // periodic kernel: [n_eval][2] p of gp_log_l's and gp_l's kernel of each row (last member:
+                               // the Gaussian instantiations keep their parameter offsets)
 };
 
 #ifdef __CUDACC__

@@ -6,7 +6,8 @@
 //   mt_seed_kernel            np.random.RandomState(seed) for a 32-bit integer seed (MT19937 init_genrand)
 //   draw_candidates_kernel    BQ._choose_candidates (bq.py:967-991): n_candidate draws of
 //                             np.random.uniform(x_s.min() - w_tl, x_s.max() + w_tl), bq_c.filter_candidates
-//                             (bq_c.pyx:601-650), np.sort of the survivors
+//                             (bq_c.pyx:601-650), np.sort of the survivors; draw_candidates_wrapped_kernel draws
+//                             on [-pi p_tl, pi p_tl] instead (the periodic kernel, bq.py:217-218)
 //
 // One thread per problem: each of these is a few thousand scalar operations per problem and runs once per round,
 // next to a scoring launch of ~10^8 FP64 operations per problem.  The Mersenne-Twister state is stored word-major
@@ -83,19 +84,32 @@ __global__ void add_observations_kernel(double *__restrict__ x_s, double *__rest
     }
 }
 
-__global__ void draw_candidates_kernel(const double *__restrict__ x_s, const int *__restrict__ ns, int stride,
-                                       const double *__restrict__ hyp, const double *__restrict__ prior,
-                                       unsigned *__restrict__ mt, int *__restrict__ mti, int n_candidate,
-                                       double *__restrict__ x_c, int *__restrict__ nc, int P) {
+// WRAPPED: the periodic kernel's draw on [-pi p_tl, pi p_tl] (bq.py:217-218), p_tl = period[2 p]; otherwise on
+// [min x_s - w_tl, max x_s + w_tl]
+template <bool WRAPPED>
+__device__ __forceinline__ void draw_candidates_body(const double *__restrict__ x_s, const int *__restrict__ ns, int stride,
+                                                     const double *__restrict__ hyp, const double *__restrict__ period,
+                                                     const double *__restrict__ prior, unsigned *__restrict__ mt,
+                                                     int *__restrict__ mti, int n_candidate, double *__restrict__ x_c,
+                                                     int *__restrict__ nc, int P) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= P) return;
     const double *xs = x_s + (size_t)p * stride;
     const int n = ns[p];
-    const double w_tl = hyp[6 * p + 1], thresh = prior[3 * p + 2];
-    double lo = INFINITY, hi = -INFINITY;
-    for (int j = 0; j < n; ++j) { lo = fmin(lo, xs[j]); hi = fmax(hi, xs[j]); }
-    lo = __dsub_rn(lo, w_tl);                                    // bq.py:974-975
-    hi = __dadd_rn(hi, w_tl);
+    double lo, hi, thresh;
+    if (WRAPPED) {
+        const double p_tl = period[2 * p];
+        thresh = prior[3 * p + 2];
+        lo = __dmul_rn(-M_PI, p_tl);                             // -np.pi * p, np.pi * p
+        hi = __dmul_rn(M_PI, p_tl);
+    } else {
+        const double w_tl = hyp[6 * p + 1];
+        thresh = prior[3 * p + 2];
+        lo = INFINITY; hi = -INFINITY;
+        for (int j = 0; j < n; ++j) { lo = fmin(lo, xs[j]); hi = fmax(hi, xs[j]); }
+        lo = __dsub_rn(lo, w_tl);                                // bq.py:974-975
+        hi = __dadd_rn(hi, w_tl);
+    }
     const double range = __dsub_rn(hi, lo);
     double xc[NC_MAX];
     int idx = mti[p];
@@ -141,6 +155,20 @@ __global__ void draw_candidates_kernel(const double *__restrict__ x_s, const int
     nc[p] = m;
 }
 
+__global__ void draw_candidates_kernel(const double *__restrict__ x_s, const int *__restrict__ ns, int stride,
+                                       const double *__restrict__ hyp, const double *__restrict__ prior,
+                                       unsigned *__restrict__ mt, int *__restrict__ mti, int n_candidate,
+                                       double *__restrict__ x_c, int *__restrict__ nc, int P) {
+    draw_candidates_body<false>(x_s, ns, stride, hyp, nullptr, prior, mt, mti, n_candidate, x_c, nc, P);
+}
+
+__global__ void draw_candidates_wrapped_kernel(const double *__restrict__ x_s, const int *__restrict__ ns, int stride,
+                                               const double *__restrict__ period, const double *__restrict__ prior,
+                                               unsigned *__restrict__ mt, int *__restrict__ mti, int n_candidate,
+                                               double *__restrict__ x_c, int *__restrict__ nc, int P) {
+    draw_candidates_body<true>(x_s, ns, stride, nullptr, period, prior, mt, mti, n_candidate, x_c, nc, P);
+}
+
 cudaError_t launch_mt_seed(const unsigned *seeds, unsigned *mt, int *mti, int P, cudaStream_t s) {
     mt_seed_kernel<<<(P + 127) / 128, 128, 0, s>>>(seeds, mt, mti, P);
     return cudaGetLastError();
@@ -155,6 +183,12 @@ cudaError_t launch_add_observations(double *x_s, double *l_s, int *ns, int strid
 cudaError_t launch_draw_candidates(const double *x_s, const int *ns, int stride, const double *hyp, const double *prior,
                                    unsigned *mt, int *mti, int n_candidate, double *x_c, int *nc, int P, cudaStream_t s) {
     draw_candidates_kernel<<<(P + 127) / 128, 128, 0, s>>>(x_s, ns, stride, hyp, prior, mt, mti, n_candidate, x_c, nc, P);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_draw_candidates_wrapped(const double *x_s, const int *ns, int stride, const double *period, const double *prior,
+                                           unsigned *mt, int *mti, int n_candidate, double *x_c, int *nc, int P, cudaStream_t s) {
+    draw_candidates_wrapped_kernel<<<(P + 127) / 128, 128, 0, s>>>(x_s, ns, stride, period, prior, mt, mti, n_candidate, x_c, nc, P);
     return cudaGetLastError();
 }
 

@@ -1006,7 +1006,8 @@ cudaError_t launch_setup2(const SetupArgs &a, int n_inst, cudaStream_t stream) {
 
 // ============================================================================================================================
 // Value and gradient of the joint log marginal likelihood ll = ll_tl + ll_l (BQ._make_llh_params, bq.py:533-552) with
-// respect to the six hyper-parameters, one CTA per (instance, hyper-parameter row).  Gaussian kernel only.
+// respect to the hyper-parameters, one CTA per (instance, hyper-parameter row).  KIND 0: gp.GaussianKernel, six
+// derivatives; KIND 1: gp.PeriodicKernel, eight (the periods p_tl and p_l last).
 //
 //   ll_tl: gp_log_l on (x_s, log l_s), K_t = c_t E_t + s_t^2 I, c = h^2 / (sqrt(2 pi) w), E_ij = exp(-d_ij^2 / 2 w^2)
 //   ll_l:  gp_l on (x_sc, [l_s; l_c]), K_l = c_l E_l + s_l^2 I, l_c[j] = exp(m_j), m_j = k_j' a, a = K_t^-1 log l_s
@@ -1024,6 +1025,13 @@ cudaError_t launch_setup2(const SetupArgs &a, int n_inst, cudaStream_t stream) {
 // trace that needs entries of K^-1 (the w-trace) evaluates (K^-1)_ij = sum_{k >= i} X_ki X_kj (X = L^-1) for i > j, one
 // thread per entry, and never stores them.
 //
+// Periodic kernel (KIND 1): K = c exp(nh D^2) with c = h^2 (independent of w), nh = -1 / (2 w^2), D = 2 sin(d / 2p), and
+// F_ij = d_ij sin(d_ij / p) / (w^2 p^2):
+//   Kd_h = 2 G / h, Kd_w = G . D^2 / w^3 (no -G / w term), Kd_p = G . F (one per GP), Kd_s = 2 s I
+//   tr(K^-1 Kd_p) = sum_ij (K^-1)_ij G_ij F_ij, accumulated in the pass of the w-trace from the same (K^-1)_ij
+//   dm_j / dp_tl = (k_j . F(x_c[j] - x_s))' a - k_j' K_t^-1 (G . F) a
+// which needs a fourth live vector K_t^-1 (G . F) a and a fourth row of dm_j.
+//
 // Observations are sorted as in the setup kernel, and the tl factor, a and l_c are computed by the same code, so l_c and
 // the guard are the setup's bit for bit.  Every reduction has a fixed order and the CTA shape is fixed (256 threads), so
 // a row's results do not depend on the other rows of the launch.  Status codes and the order of the checks are the
@@ -1031,55 +1039,88 @@ cudaError_t launch_setup2(const SetupArgs &a, int n_inst, cudaStream_t stream) {
 constexpr int LLG_NT = 256;
 constexpr int LLG_NVEC = 3;     // K_t^-1 G a, K_t^-1 (G . D^2) a, K_t^-1 a: live across the candidate pass (stage)
 
-__host__ __device__ inline int llg_smem_doubles(int nmax, int ncm, bool tsmem) {
+// kind 1 adds the vector K_t^-1 (G . F) a and the row dm_j / dp_tl
+__host__ __device__ inline int llg_smem_doubles(int nmax, int ncm, bool tsmem, int kind) {
     const S2Carve c = s2_carve(nmax, ncm, tsmem);
-    return c.total + LLG_NVEC * c.nv + 3 * NC_MAX;
+    return c.total + (LLG_NVEC + kind) * c.nv + (3 + kind) * NC_MAX;
 }
 
-// sum over i > j of (K^-1)_ij G_ij d_ij^2 with K^-1 = X' X, X = L^-1 packed in T (partial sum of the calling thread)
-__device__ __forceinline__ double llg_wtrace_part(const double *T, int n, const double *x, double c, double nh) {
-    double p = 0.0;
+// D^2 = (2 sin(d hp))^2 and F = d sin(d / p) / (w^2 p^2) of the periodic kernel (hp = 1 / (2 p), nh = -1 / (2 w^2))
+__device__ __forceinline__ void llg_periodic_terms(double d, double nh, double hp, double &D2, double &F) {
+    double sn, cs;
+    sincos(d * hp, &sn, &cs);
+    D2 = (2.0 * sn) * (2.0 * sn);
+    F = d * (2.0 * sn * cs) * (-2.0 * nh) * (4.0 * hp * hp);
+}
+
+// sum over i > j of (K^-1)_ij G_ij D_ij^2 with K^-1 = X' X, X = L^-1 packed in T (partial sum of the calling thread);
+// KIND 1 also sums (K^-1)_ij G_ij F_ij into *pp
+template <int KIND>
+__device__ __forceinline__ double llg_wtrace_part(const double *T, int n, const double *x, double c, double nh, double hp, double *pp) {
+    double p = 0.0, q = 0.0;
     for (int e = threadIdx.x; e < tri(n); e += LLG_NT) {
         int i, j;
         tri_decode(e, i, j);
         if (j == i) continue;
         double kij = 0.0;
         for (int k = i, r = tri(i); k < n; r += ++k) kij = fma(T[r + i], T[r + j], kij);
-        const double d = x[i] - x[j], d2 = d * d;
-        p = fma(kij, c * kernel_exp(d, nh, 0, 0.0) * d2, p);
+        const double d = x[i] - x[j];
+        if (KIND) {
+            double D2, F;
+            llg_periodic_terms(d, nh, hp, D2, F);
+            const double g = c * kernel_exp(d, nh, 1, hp);
+            p = fma(kij, g * D2, p);
+            q = fma(kij, g * F, q);
+        } else {
+            const double d2 = d * d;
+            p = fma(kij, c * kernel_exp(d, nh, 0, 0.0) * d2, p);
+        }
     }
+    if (KIND) *pp = q;
     return p;
 }
 
-// g1 = G v, g2 = (G . D^2) v over the first n points of x, a thread per row (G = c E, without the noise)
-__device__ __forceinline__ void llg_gram_matvec(const double *x, int n, double c, double nh, const double *v, double *g1, double *g2) {
+// g1 = G v, g2 = (G . D^2) v (and for KIND 1 g3 = (G . F) v) over the first n points of x, a thread per row (G = c E,
+// without the noise)
+template <int KIND>
+__device__ __forceinline__ void llg_gram_matvec(const double *x, int n, double c, double nh, double hp, const double *v, double *g1,
+                                                double *g2, double *g3) {
     for (int i = threadIdx.x; i < n; i += LLG_NT) {
-        double s1 = 0.0, s2 = 0.0;
+        double s1 = 0.0, s2 = 0.0, s3 = 0.0;
         for (int j = 0; j < n; ++j) {
             const double d = x[i] - x[j];
-            const double g = c * kernel_exp(d, nh, 0, 0.0);
+            const double g = c * kernel_exp(d, nh, KIND, hp);
             s1 = fma(g, v[j], s1);
-            s2 = fma(g * (d * d), v[j], s2);
+            if (KIND) {
+                double D2, F;
+                llg_periodic_terms(d, nh, hp, D2, F);
+                s2 = fma(g * D2, v[j], s2);
+                s3 = fma(g * F, v[j], s3);
+            } else {
+                s2 = fma(g * (d * d), v[j], s2);
+            }
         }
         g1[i] = s1;
         g2[i] = s2;
+        if (KIND) g3[i] = s3;
     }
     __syncthreads();
 }
 
-template <bool TSMEM>
+template <bool TSMEM, int KIND>
 __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
     constexpr int NT = LLG_NT, NW = NT / 32;
+    constexpr int NOUT = KIND ? LLG_OUT_PERIODIC : LLG_OUT;
     __shared__ double red[NW];
     __shared__ int s_fail, s_info;
     extern __shared__ double s_dyn[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int e = a.e0 + blockIdx.x;
     const int inst = a.inst ? a.inst[e] : e;
-    double *out = a.out + (size_t)e * LLG_OUT;
+    double *out = a.out + (size_t)e * NOUT;
     const int ns = a.ns[inst], nc = a.nc[inst], n = ns + nc;
 
-    // carve-up: the setup kernel's, then [p1 p2 p3] [dm 3 x NC_MAX]
+    // carve-up: the setup kernel's, then [p1 p2 p3 (p4)] [dm (3 | 4) x NC_MAX]
     const S2Carve cv = s2_carve(a.n_max, a.nc_max, TSMEM);
     const int lds = cv.lds, nv = cv.nv;
     double *T = TSMEM ? s_dyn : a.work + (size_t)blockIdx.x * a.work_stride;
@@ -1088,19 +1129,22 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
     double *un = vec + S2_NVEC_FIXED * nv;
     double *stage = un;
     double *u0 = un, *u1 = un + nv, *u2 = un + 2 * nv, *u3 = un + 3 * nv;
+    double *u4 = un + 4 * nv, *u5 = un + 5 * nv;       // KIND 1 only
     double *blk = un + cv.un;
     double *p1 = s_dyn + cv.total, *p2 = p1 + nv, *p3 = p2 + nv;
-    double *dm = p3 + nv;
+    double *p4 = p3 + nv;                               // KIND 1 only: K_t^-1 (G . F) a
+    double *dm = p3 + (KIND ? 2 : 1) * nv;
 
     auto fail = [&](int status) {
         if (tid == 0) {
             out[0] = -INFINITY;
-            for (int k = 1; k < 7; ++k) out[k] = NAN;
-            out[7] = status;
+            for (int k = 1; k < NOUT - 1; ++k) out[k] = NAN;
+            out[NOUT - 1] = status;
         }
     };
     const double *hp = a.hyp + (size_t)e * 6;
     const double h_tl = hp[0], w_tl = hp[1], s_tl = hp[2], h_l = hp[3], w_l = hp[4], s_l = hp[5];
+    const double p_tl = KIND ? a.period[(size_t)e * 2] : 0.0, p_l = KIND ? a.period[(size_t)e * 2 + 1] : 0.0;
     if (!(ns >= 1 && ns <= a.in_stride && nc >= 0 && nc <= NC_MAX && nc <= a.nc_max && n <= a.n_max)) { fail(SETUP_BAD_INPUT); return; }
     if (tid == 0) s_fail = SETUP_OK;
     __syncthreads();
@@ -1123,6 +1167,7 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
         if (tid == 0) {
             for (int k = 0; k < 6; ++k) bad |= !isfinite(hp[k]);
             bad |= !(h_tl > 0 && w_tl > 0 && s_tl >= 0 && h_l > 0 && w_l > 0 && s_l >= 0);
+            if (KIND) bad |= !(isfinite(p_tl) && isfinite(p_l) && p_tl > 0 && p_l > 0);
         }
         if (bad) s_fail = SETUP_BAD_INPUT;
     }
@@ -1141,15 +1186,17 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
     }
     __syncthreads();
 
-    const double c_tl = (h_tl * h_tl) / (S2_SQRT_2PI * w_tl), nh_tl = -0.5 / (w_tl * w_tl);
-    const double c_l = (h_l * h_l) / (S2_SQRT_2PI * w_l), nh_l = -0.5 / (w_l * w_l);
+    // the setup kernel's expressions (bit for bit the same l_c and guard)
+    const double hp_tl = KIND ? 0.5 / p_tl : 0.0, hp_l = KIND ? 0.5 / p_l : 0.0;
+    const double c_tl = KIND ? h_tl * h_tl : (h_tl * h_tl) / (S2_SQRT_2PI * w_tl), nh_tl = -0.5 / (w_tl * w_tl);
+    const double c_l = KIND ? h_l * h_l : (h_l * h_l) / (S2_SQRT_2PI * w_l), nh_l = -0.5 / (w_l * w_l);
 
     // ---- tl phase: K_t -> L_t -> L_t^-1, a
     for (int i = tid; i < ns; i += NT) tl_s[i] = log(l_sc[i]);
     for (int q = tid; q < tri(ns); q += NT) {
         int i, j;
         tri_decode(q, i, j);
-        double v = c_tl * kernel_exp(x_sc[i] - x_sc[j], nh_tl, 0, 0.0);
+        double v = c_tl * kernel_exp(x_sc[i] - x_sc[j], nh_tl, KIND, hp_tl);
         if (i == j) v += s_tl * s_tl;
         T[q] = v;
     }
@@ -1164,29 +1211,36 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
     tri_inverse_packed<NT>(T, ns, stage, lds, rdiag);
     lower_matvec_p<NT>(T, ns, tl_s, u0, nullptr, nullptr);
     lower_matvec_t_p<NT>(T, ns, u0, a_tl, nullptr, nullptr);
-    // u0 = G a, u1 = (G . D^2) a; p1 = K_t^-1 u0, p2 = K_t^-1 u1, p3 = K_t^-1 a
-    llg_gram_matvec(x_sc, ns, c_tl, nh_tl, a_tl, u0, u1);
+    // u0 = G a, u1 = (G . D^2) a (u4 = (G . F) a); p1 = K_t^-1 u0, p2 = K_t^-1 u1, p3 = K_t^-1 a (p4 = K_t^-1 u4)
+    llg_gram_matvec<KIND>(x_sc, ns, c_tl, nh_tl, hp_tl, a_tl, u0, u1, u4);
     lower_matvec_p<NT>(T, ns, u0, u2, u1, u3);
     lower_matvec_t_p<NT>(T, ns, u2, p1, u3, p2);
-    lower_matvec_p<NT>(T, ns, a_tl, u2, nullptr, nullptr);
-    lower_matvec_t_p<NT>(T, ns, u2, p3, nullptr, nullptr);
-    double g_tl[3], yKy_tl;
+    lower_matvec_p<NT>(T, ns, a_tl, u2, KIND ? u4 : nullptr, KIND ? u5 : nullptr);
+    lower_matvec_t_p<NT>(T, ns, u2, p3, KIND ? u5 : nullptr, KIND ? p4 : nullptr);
+    double g_tl[4], yKy_tl;
     {
-        double pg1 = 0.0, pg2 = 0.0, paa = 0.0, py = 0.0, ptr = 0.0;
+        double pg1 = 0.0, pg2 = 0.0, paa = 0.0, py = 0.0, ptr = 0.0, pg3 = 0.0, pp = 0.0;
         for (int i = tid; i < ns; i += NT) {
             pg1 = fma(a_tl[i], u0[i], pg1);
             pg2 = fma(a_tl[i], u1[i], pg2);
             paa = fma(a_tl[i], a_tl[i], paa);
+            if (KIND) pg3 = fma(a_tl[i], u4[i], pg3);
         }
         for (int i = tid; i < ns; i += NT) py = fma(tl_s[i], a_tl[i], py);
         for (int q = tid; q < tri(ns); q += NT) ptr = fma(T[q], T[q], ptr);
         const double aga = block_sum2<NT>(pg1, red), agda = block_sum2<NT>(pg2, red), aa = block_sum2<NT>(paa, red);
         yKy_tl = block_sum2<NT>(py, red);
         const double trK = block_sum2<NT>(ptr, red);
-        const double wtr = 2.0 * block_sum2<NT>(llg_wtrace_part(T, ns, x_sc, c_tl, nh_tl), red);
+        const double wtr = 2.0 * block_sum2<NT>(llg_wtrace_part<KIND>(T, ns, x_sc, c_tl, nh_tl, hp_tl, &pp), red);
         const double rest = ns - s_tl * s_tl * trK;
         g_tl[0] = (aga - rest) / h_tl;
-        g_tl[1] = 0.5 * ((agda - wtr) / (w_tl * w_tl * w_tl) - (aga - rest) / w_tl);
+        if (KIND) {
+            g_tl[1] = 0.5 * (agda - wtr) / (w_tl * w_tl * w_tl);
+            const double agfa = block_sum2<NT>(pg3, red), ptrace = 2.0 * block_sum2<NT>(pp, red);
+            g_tl[3] = 0.5 * (agfa - ptrace);
+        } else {
+            g_tl[1] = 0.5 * ((agda - wtr) / (w_tl * w_tl * w_tl) - (aga - rest) / w_tl);
+        }
         g_tl[2] = s_tl * (aa - trK);
     }
     // l_c = exp(k_j' a), the guard and dm_j, four candidates per pass (the setup kernel's P6, plus the three dm_j):
@@ -1195,7 +1249,7 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
         const int nbt = (nc - j0 < 4) ? nc - j0 : 4;
         for (int q = tid; q < nbt * ns; q += NT) {
             const int j = q / ns, k = q - j * ns;
-            stage[j * lds + k] = c_tl * kernel_exp(x_sc[ns + j0 + j] - x_sc[k], nh_tl, 0, 0.0);
+            stage[j * lds + k] = c_tl * kernel_exp(x_sc[ns + j0 + j] - x_sc[k], nh_tl, KIND, hp_tl);
         }
         __syncthreads();
         if (a.check_max) {
@@ -1217,12 +1271,20 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
         if (warp < nbt) {
             const int j = warp;
             const double xc = x_sc[ns + j0 + j];
-            double m = 0.0, q = 0.0, r = 0.0, q1 = 0.0, q2 = 0.0, q3 = 0.0;
+            double m = 0.0, q = 0.0, r = 0.0, q1 = 0.0, q2 = 0.0, q3 = 0.0, rp = 0.0, q4 = 0.0;
             for (int k = lane; k < ns; k += 32) {
                 const double kv = stage[j * lds + k], d = xc - x_sc[k];
                 m = fma(kv, a_tl[k], m);
                 if (a.check_max) q += stage[(4 + j) * lds + k];
-                r = fma(kv * (d * d), a_tl[k], r);
+                if (KIND) {
+                    double D2, F;
+                    llg_periodic_terms(d, nh_tl, hp_tl, D2, F);
+                    r = fma(kv * D2, a_tl[k], r);
+                    rp = fma(kv * F, a_tl[k], rp);
+                    q4 = fma(kv, p4[k], q4);
+                } else {
+                    r = fma(kv * (d * d), a_tl[k], r);
+                }
                 q1 = fma(kv, p1[k], q1);
                 q2 = fma(kv, p2[k], q2);
                 q3 = fma(kv, p3[k], q3);
@@ -1233,6 +1295,10 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
             q1 = warp_sum(q1);
             q2 = warp_sum(q2);
             q3 = warp_sum(q3);
+            if (KIND) {
+                rp = warp_sum(rp);
+                q4 = warp_sum(q4);
+            }
             if (lane == 0) {
                 if (a.check_max) {
                     double V = c_tl - q;
@@ -1241,7 +1307,12 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
                 }
                 l_sc[ns + j0 + j] = exp(m);
                 dm[j0 + j] = 2.0 * (m - q1) / h_tl;
-                dm[NC_MAX + j0 + j] = (r - q2) / (w_tl * w_tl * w_tl) - (m - q1) / w_tl;
+                if (KIND) {
+                    dm[NC_MAX + j0 + j] = (r - q2) / (w_tl * w_tl * w_tl);
+                    dm[3 * NC_MAX + j0 + j] = rp - q4;
+                } else {
+                    dm[NC_MAX + j0 + j] = (r - q2) / (w_tl * w_tl * w_tl) - (m - q1) / w_tl;
+                }
                 dm[2 * NC_MAX + j0 + j] = -2.0 * s_tl * q3;
             }
         }
@@ -1255,7 +1326,7 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
         for (int q = tid; q < tri(n); q += NT) {
             int i, j;
             tri_decode(q, i, j);
-            double v = c_l * kernel_exp(x_sc[i] - x_sc[j], nh_l, 0, 0.0);
+            double v = c_l * kernel_exp(x_sc[i] - x_sc[j], nh_l, KIND, hp_l);
             if (pass && i == j) v += s_l * s_l;
             T[q] = v;
         }
@@ -1272,68 +1343,89 @@ __global__ void __launch_bounds__(LLG_NT) bq_llgrad_kernel(LLGradArgs a) {
     double *alpha = u1;
     lower_matvec_p<NT>(T, n, l_sc, u0, nullptr, nullptr);
     lower_matvec_t_p<NT>(T, n, u0, alpha, nullptr, nullptr);
-    llg_gram_matvec(x_sc, n, c_l, nh_l, alpha, u2, u3);
+    llg_gram_matvec<KIND>(x_sc, n, c_l, nh_l, hp_l, alpha, u2, u3, u4);
     {
-        double pg1 = 0.0, pg2 = 0.0, paa = 0.0, py = 0.0, ptr = 0.0;
+        double pg1 = 0.0, pg2 = 0.0, paa = 0.0, py = 0.0, ptr = 0.0, pg3 = 0.0, pp = 0.0;
         for (int i = tid; i < n; i += NT) {
             pg1 = fma(alpha[i], u2[i], pg1);
             pg2 = fma(alpha[i], u3[i], pg2);
             paa = fma(alpha[i], alpha[i], paa);
+            if (KIND) pg3 = fma(alpha[i], u4[i], pg3);
         }
         for (int i = tid; i < n; i += NT) py = fma(l_sc[i], alpha[i], py);
         for (int q = tid; q < tri(n); q += NT) ptr = fma(T[q], T[q], ptr);
         const double aga = block_sum2<NT>(pg1, red), agda = block_sum2<NT>(pg2, red), aa = block_sum2<NT>(paa, red);
         const double yKy = block_sum2<NT>(py, red), trK = block_sum2<NT>(ptr, red);
-        const double wtr = 2.0 * block_sum2<NT>(llg_wtrace_part(T, n, x_sc, c_l, nh_l), red);
+        const double wtr = 2.0 * block_sum2<NT>(llg_wtrace_part<KIND>(T, n, x_sc, c_l, nh_l, hp_l, &pp), red);
+        double agfa = 0.0, ptrace = 0.0;
+        if (KIND) {
+            agfa = block_sum2<NT>(pg3, red);
+            ptrace = 2.0 * block_sum2<NT>(pp, red);
+        }
         if (tid == 0) {
             const double rest = n - s_l * s_l * trK;
-            double ch = 0.0, cw = 0.0, cs = 0.0;                  // sum_j gamma_j dm_j, in candidate order
+            double ch = 0.0, cw = 0.0, cs = 0.0, cp = 0.0;        // sum_j gamma_j dm_j, in candidate order
             for (int j = 0; j < nc; ++j) {
                 const double gam = alpha[ns + j] * l_sc[ns + j];
                 ch = fma(gam, dm[j], ch);
                 cw = fma(gam, dm[NC_MAX + j], cw);
                 cs = fma(gam, dm[2 * NC_MAX + j], cs);
+                if (KIND) cp = fma(gam, dm[3 * NC_MAX + j], cp);
             }
             out[0] = (-0.5 * yKy_tl - sumlog_tl - 0.5 * ns * S2_LOG_2PI) + (-0.5 * yKy - sumlog_l - 0.5 * n * S2_LOG_2PI);
             out[1] = g_tl[0] - ch;
             out[2] = g_tl[1] - cw;
             out[3] = g_tl[2] - cs;
             out[4] = (aga - rest) / h_l;
-            out[5] = 0.5 * ((agda - wtr) / (w_l * w_l * w_l) - (aga - rest) / w_l);
-            out[6] = s_l * (aa - trK);
-            out[7] = SETUP_OK;
+            if (KIND) {
+                out[5] = 0.5 * (agda - wtr) / (w_l * w_l * w_l);
+                out[6] = s_l * (aa - trK);
+                out[7] = g_tl[3] - cp;
+                out[8] = 0.5 * (agfa - ptrace);
+            } else {
+                out[5] = 0.5 * ((agda - wtr) / (w_l * w_l * w_l) - (aga - rest) / w_l);
+                out[6] = s_l * (aa - trK);
+            }
+            out[NOUT - 1] = SETUP_OK;
         }
     }
 }
 
-template <bool TSMEM>
+template <bool TSMEM, int KIND>
 static cudaError_t launch_llgrad_one(const LLGradArgs &a, int n_rows, size_t bytes, cudaStream_t stream) {
-    cudaError_t e = cudaFuncSetAttribute(bq_llgrad_kernel<TSMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cudaError_t e = cudaFuncSetAttribute(bq_llgrad_kernel<TSMEM, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
-    bq_llgrad_kernel<TSMEM><<<n_rows, LLG_NT, bytes, stream>>>(a);
+    bq_llgrad_kernel<TSMEM, KIND><<<n_rows, LLG_NT, bytes, stream>>>(a);
     return cudaGetLastError();
 }
 
-// Rows [a.e0, a.e0 + n_rows): one launch while the triangle fits shared memory, else launches of at most work_inst CTAs
-// on the global scratch a.work (work_inst triangles of a.work_stride doubles).  *launches counts the kernel launches.
-cudaError_t launch_llgrad(LLGradArgs a, int n_rows, int work_inst, cudaStream_t stream, int *launches) {
-    const size_t bytes_sm = sizeof(double) * (size_t)llg_smem_doubles(a.n_max, a.nc_max, true);
+template <int KIND>
+static cudaError_t launch_llgrad_kind(LLGradArgs a, int n_rows, int work_inst, cudaStream_t stream, int *launches) {
+    const size_t bytes_sm = sizeof(double) * (size_t)llg_smem_doubles(a.n_max, a.nc_max, true, KIND);
     *launches = 0;
     if (bytes_sm <= S2_CTA_SMEM_MAX) {
         *launches = 1;
-        return launch_llgrad_one<true>(a, n_rows, bytes_sm, stream);
+        return launch_llgrad_one<true, KIND>(a, n_rows, bytes_sm, stream);
     }
     const int n_big = a.n_max;
     if (!a.work || a.work_stride < (size_t)tri(n_big) || work_inst < 1) return cudaErrorInvalidValue;
-    const size_t bytes = sizeof(double) * (size_t)llg_smem_doubles(a.n_max, a.nc_max, false);
+    const size_t bytes = sizeof(double) * (size_t)llg_smem_doubles(a.n_max, a.nc_max, false, KIND);
     const int end = a.e0 + n_rows;
     for (int e0 = a.e0; e0 < end; e0 += work_inst) {
         a.e0 = e0;
-        cudaError_t e = launch_llgrad_one<false>(a, end - e0 < work_inst ? end - e0 : work_inst, bytes, stream);
+        cudaError_t e = launch_llgrad_one<false, KIND>(a, end - e0 < work_inst ? end - e0 : work_inst, bytes, stream);
         ++*launches;
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;
+}
+
+// Rows [a.e0, a.e0 + n_rows) of kernel kind 0 (Gaussian) or 1 (periodic, a.period set): one launch while the triangle fits
+// shared memory, else launches of at most work_inst CTAs on the global scratch a.work (work_inst triangles of a.work_stride
+// doubles).  *launches counts the kernel launches.
+cudaError_t launch_llgrad(LLGradArgs a, int n_rows, int work_inst, cudaStream_t stream, int *launches, int kind) {
+    return kind ? launch_llgrad_kind<1>(a, n_rows, work_inst, stream, launches)
+                : launch_llgrad_kind<0>(a, n_rows, work_inst, stream, launches);
 }
 
 }  // namespace bqb

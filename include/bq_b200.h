@@ -107,6 +107,16 @@ int bqb_batch_set_hypers(bqb_batch *b, const double *hyp, void *stream);
  * bqb_batch_set_approx with the periodic kernel); BQB_ESTATE when nothing is staged.  Synchronises `stream`. */
 int bqb_batch_log_lh_grad(bqb_batch *b, const double *hyp, const int *inst, int n_eval, int check_max, double *log_lh_out,
                           double *grad_out, int *status_out, void *stream);
+/* bqb_batch_log_lh_grad for a batch of the periodic kernel (bqb_batch_set_approx with kernel_kind 1): each row also has
+ * its periods, period [n_eval][2] (p of gp_log_l, then of gp_l; HOST array), and grad_out is [n_eval][8]: d log_lh / d
+ * (h_tl, w_tl, s_tl, h_l, w_l, s_l, p_tl, p_l).  BQB_EUNSUPPORTED unless the batch uses the periodic kernel; BQB_ESTATE
+ * when nothing is staged.  Synchronises `stream`. */
+int bqb_batch_log_lh_grad_periodic(bqb_batch *b, const double *hyp, const double *period, const int *inst, int n_eval,
+                                   int check_max, double *log_lh_out, double *grad_out, int *status_out, void *stream);
+/* The periodic twin of bqb_batch_set_hypers: replaces the periods period [n_inst][2] (HOST pointer) of a batch of the
+ * periodic kernel and nothing else (the grids of bqb_batch_set_approx stay as they are).  BQB_ESTATE when the batch does
+ * not use the periodic kernel. */
+int bqb_batch_set_periods(bqb_batch *b, const double *period, void *stream);
 /* Non-Gaussian kernels and the trapezoid approximation.  Replaces gp.PeriodicKernel as used by bq.py:139-165 and
  * bq_c.approx_Z_mean (bq_c.pyx:216-261), approx_Z_var (:358-422), approx_expected_squared_mean_and_mean (:538-598),
  * i.e. what BQ does when options['use_approx'] is set (bq.py:251-252, :310-311, :498-510).
@@ -132,6 +142,10 @@ int bqb_batch_rng_set(bqb_batch *b, const unsigned *mt, const int *pos);
  * np.random.uniform(x_s.min() - w_tl, x_s.max() + w_tl) from the instance's generator (bit-identical to numpy),
  * bq_c.filter_candidates (bq_c.pyx:601-650) with the instance's candidate_thresh, np.sort of the survivors. */
 int bqb_batch_draw_candidates(bqb_batch *b, int n_candidate, void *stream);
+/* bqb_batch_draw_candidates with the periodic kernel's wrapped range (bq.py:217-218): the draws are
+ * np.random.uniform(-pi p_tl, pi p_tl) with p_tl the instance's period of gp_log_l; the filter and sort are the same.
+ * BQB_ESTATE when the batch does not use the periodic kernel. */
+int bqb_batch_draw_candidates_wrapped(bqb_batch *b, int n_candidate, void *stream);
 /* BQ.add_observation (bq.py:683-701) for every instance: DEVICE arrays d_x_new / d_l_new [n_inst]; the new point
  * is averaged into the nearest observation when closer than candidate_thresh, appended otherwise.  Returns
  * BQB_EUNSUPPORTED if an instance is already at bqb_batch_capacity() observations.  Synchronises `stream`. */
