@@ -565,10 +565,14 @@ int bqb_batch_info(bqb_batch *b, double *Z_mean, double *Z_var, double *log_lh, 
     return 0;
 }
 
-// the tensor-core kernels (Gaussian kernel, closed-form integrals) or the generic kernel (bqb_batch_set_approx)
-static cudaError_t score_dispatch(bqb_batch *b, ScoreArgs &a, int n_inst, cudaStream_t s, int *grid_x = nullptr) {
+// the tensor-core kernels (Gaussian kernel, closed-form integrals) or the generic kernel (bqb_batch_set_approx).
+// `first`: the instance at which a.models begins.  The single-instance entry points pass that instance's own model block
+// with inst0 = 0, so the generic kernel's per-instance grid and trapezoid weights must begin at the same instance.
+static cudaError_t score_dispatch(bqb_batch *b, ScoreArgs &a, int n_inst, cudaStream_t s, int *grid_x = nullptr, int first = 0) {
     if (b->generic) {
-        a.xo = b->d_xo; a.wp = b->d_wp; a.n_xo = b->n_xo; a.xo_stride = b->xo_stride;
+        a.xo = b->d_xo ? b->d_xo + (size_t)first * b->xo_stride : nullptr;
+        a.wp = b->d_wp ? b->d_wp + (size_t)first * b->n_xo : nullptr;
+        a.n_xo = b->n_xo; a.xo_stride = b->xo_stride;
         return launch_score_generic(a, n_inst, s, grid_x);
     }
     return launch_score(a, n_inst, b->sm_count, s, grid_x);
@@ -835,11 +839,11 @@ int bqb_expected_var_host(bqb_batch *b, int inst, const double *x_a, int na, dou
             // fused epilogue: Zm^2 + Zv - esm written straight into the caller's page-locked array
             a.esm = nullptr; a.ev = (double *)dout + lo;
             a.part_val = b->d_red_val + 2048 * (c & 1); a.part_idx = b->d_red_idx + 2048 * (c & 1);
-            CU(score_dispatch(b, a, 1, s, &zc_grid));
+            CU(score_dispatch(b, a, 1, s, &zc_grid, inst));
             b->launches += 1;
         } else {
             a.esm = b->d_esm + lo; a.ev = nullptr;
-            CU(score_dispatch(b, a, 1, s));
+            CU(score_dispatch(b, a, 1, s, nullptr, inst));
             CU(launch_expected_var(b->d_esm + lo, n, msm, b->d_em + lo, s));
             b->launches += 2;
             CU(cudaMemcpyAsync(out + lo, b->d_em + lo, sizeof(double) * n, cudaMemcpyDeviceToHost, s));
@@ -936,7 +940,7 @@ int bqb_choose_step_device(bqb_batch *b, int inst, const double *d_x_a, int na, 
     a.inst0 = 0; a.ndb_max = b->ndb_max;
     a.ev = d_ev; a.part_val = b->d_red_val; a.part_idx = b->d_red_idx;
     int grid_x = 0;
-    CU(score_dispatch(b, a, 1, s, &grid_x));
+    CU(score_dispatch(b, a, 1, s, &grid_x, inst));
     CU(launch_argmin_partials(b->d_red_val, b->d_red_idx, grid_x, offset, d_pair, s));
     b->launches += 2;
     return 0;
@@ -959,7 +963,7 @@ int bqb_choose_step_exchange(bqb_batch *b, int inst, const double *d_x_a, int na
     a.inst0 = 0; a.ndb_max = b->ndb_max;
     a.ev = d_ev; a.part_val = b->d_red_val; a.part_idx = b->d_red_idx;
     int grid_x = 0;
-    CU(score_dispatch(b, a, 1, s, &grid_x));
+    CU(score_dispatch(b, a, 1, s, &grid_x, inst));
     CU(launch_argmin_exchange(b->d_red_val, b->d_red_idx, grid_x, offset, cyclic_block, peer_slots, world, rank, seq, out4, s));
     b->launches += 2;
     return 0;

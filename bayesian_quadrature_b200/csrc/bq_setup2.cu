@@ -64,6 +64,11 @@ __device__ __forceinline__ void tri_decode(int e, int &i, int &j) {
     j = e - tri(r);
 }
 
+// Tolerance of np.isclose(x_a, x_s, atol=1e-4) (bq.py:456): atol + rtol |x_s| rounded after the product and after the
+// sum, as numpy evaluates it.  Contracted to one fma it differs by an ulp for about a fifth of all x_s, and a point at
+// that distance would take the shortcut where the reference does not (or the other way round).
+__device__ __forceinline__ double isclose_tol(double xs) { return __dadd_rn(1e-4, __dmul_rn(1e-5, fabs(xs))); }
+
 template <int NT>
 __device__ double block_sum2(double v, double *red) {
     v = warp_sum(v);
@@ -902,7 +907,7 @@ __global__ void __launch_bounds__(NT, 512 / NT) bq_setup2_kernel(SetupArgs a) {
     PH(21);
     // ---- P15/P16: header and vectors
     double t2 = 0.0;
-    for (int i = tid; i < ns; i += NT) { const double t = 1e-4 + 1e-5 * fabs(x_sc[i]); t2 = fmax(t2, t * t); }
+    for (int i = tid; i < ns; i += NT) { const double t = isclose_tol(x_sc[i]); t2 = fmax(t2, t * t); }
     t2 = block_max2<NT>(t2, red);
     if (tid == 0) {
         M[H_NS] = ns; M[H_NC] = nc; M[H_NSP] = nsp; M[H_STATUS] = SETUP_OK; M[H_NDB] = ndb;
@@ -924,7 +929,7 @@ __global__ void __launch_bounds__(NT, 512 / NT) bq_setup2_kernel(SetupArgs a) {
     for (int i = tid; i < lay.nsp_cap; i += NT) {
         const bool in = i < ns;
         M[lay.off_xs + i] = in ? x_sc[i] : 1e150;
-        M[lay.off_tol + i] = in ? 1e-4 + 1e-5 * fabs(x_sc[i]) : -1.0;
+        M[lay.off_tol + i] = in ? isclose_tol(x_sc[i]) : -1.0;
         M[lay.off_atl + i] = in ? c_tl * a_tl[i] : 0.0;
     }
     for (int i = tid; i < nc; i += NT) M[lay.off_xc + i] = x_sc[ns + i];
