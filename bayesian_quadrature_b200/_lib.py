@@ -57,6 +57,7 @@ SYMBOLS = {
     "bqb_expected_var_host": (ctypes.c_int, [_vp, ctypes.c_int, _dp, ctypes.c_int, _dp, _ip]),
     "bqb_score_host": (ctypes.c_int, [_vp, _dp, _ll, ctypes.c_int, _dp, _dp, _ip]),
     "bqb_expected_var_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _ll, _vp, _vp]),
+    "bqb_expected_var_rows_device": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, _ll, _ll, _vp, _ll, _vp]),
     "bqb_mean_neg_device": (ctypes.c_int, [_vp, _vp, _ll, _ll, _vp, _vp]),
     "bqb_argmin_device": (ctypes.c_int, [_vp, _vp, _ll, _dp, ctypes.POINTER(_ll), _vp]),
     "bqb_argmin_pair_device": (ctypes.c_int, [_vp, _vp, _ll, _ll, _vp, _vp]),
@@ -416,6 +417,17 @@ class Batch(object):
     def expected_var_device(self, inst, esm, out, stream=None):
         _check(load().bqb_expected_var_device(self._h, int(inst), _ptr(esm), esm.numel(), _ptr(out),
                                               _vp(stream) if stream else None), "bqb_expected_var_device")
+
+    def expected_var_rows_device(self, inst0, n_inst, esm, out, stream=None):
+        """out[r] = Z_mean^2 + Z_var - esm[r] for instances inst0 + r, r < n_inst: float64 CUDA tensors [>= n_inst, na] with
+        unit column stride (strided rows are fine; esm and out may be the same tensor)."""
+        if esm.dim() != 2 or out.dim() != 2 or esm.shape[1] != out.shape[1] or min(esm.shape[0], out.shape[0]) < int(n_inst):
+            raise ValueError("esm and out must be [>= n_inst, na] tensors with the same na")
+        if (esm.shape[1] > 1 and esm.stride(1) != 1) or (out.shape[1] > 1 and out.stride(1) != 1):
+            raise ValueError("esm and out must have contiguous rows")
+        _check(load().bqb_expected_var_rows_device(self._h, int(inst0), int(n_inst), _ptr(esm), esm.stride(0), esm.shape[1],
+                                                   _ptr(out), out.stride(0), _vp(stream) if stream else None),
+               "bqb_expected_var_rows_device")
 
     def mean_neg_device(self, esm, loss, stream=None):
         _check(load().bqb_mean_neg_device(self._h, _ptr(esm), esm.stride(0), esm.shape[1], _ptr(loss),

@@ -26,13 +26,14 @@ and the model setup run on the device through the C-ABI.
 """
 import logging
 import time
+import warnings
 
 import numpy as np
 
 from . import _lib
 from . import util
-from .bq import _SETUP_ERRORS, _vonmises_px
-from .gp import GaussianKernel, PeriodicKernel
+from .bq import BQ, _SETUP_ERRORS, _looks_sorted, _vonmises_px
+from .gp import GP, GaussianKernel, PeriodicKernel
 
 logger = logging.getLogger("bayesian_quadrature")
 _NAMES = ("h", "w", "s")                     # GaussianKernel parameters, then the noise: columns of one GP's (h, w, s)
@@ -627,3 +628,181 @@ class BatchBQ(object):
         self.l_s[rows, self.ns[rows]] = l_new[rows]
         self.ns[rows] += 1
         return self.init()
+
+    # ---------------------------------------------------------------- per-point read-outs (bq.py:177-231, :354-445)
+    # Row p of every result is what the BQ object of problem p returns.  x_a is a shared grid [na] or per-problem grids
+    # [P, na], numpy or a float64 CUDA tensor; results are numpy arrays, or CUDA tensors with on_device=True.  None of these
+    # methods touches the model.
+    def _grid(self, x_a):
+        x_h, x_d = self._query(x_a)
+        if x_d.dim() not in (1, 2) or (x_d.dim() == 2 and x_d.shape[0] != self.P):
+            raise ValueError("x_a must be [na] or [P, na]")
+        return x_h, x_d
+
+    def _presort(self, x_h, x_d):
+        """The automatic pre-sort of the host scoring entry points that BQ goes through (``want_presort`` of bq_capi.cu): a
+        shared grid of at least 8192 points that does not look sorted is scored in ascending order on a batch of capacity
+        128 or more, where band skipping would otherwise lose most of its effect.  Returns (points to score, perm): the
+        result at sorted position j belongs to the caller's point perm[j] (perm is None when nothing is sorted)."""
+        import torch
+        if x_d.dim() != 1 or x_d.shape[0] < 8192 or self._cap_class < 128:
+            return x_d, None
+        if _looks_sorted(x_d.cpu().numpy() if x_h is None else x_h):
+            return x_d, None
+        return torch.sort(x_d)
+
+    @staticmethod
+    def _unsort(t, perm, on_device):
+        """Rows of t (scored in sorted order) in the caller's order, as a CUDA tensor or a numpy array."""
+        if perm is None:
+            return t if on_device else t.cpu().numpy()
+        if on_device:
+            import torch
+            return torch.empty_like(t).index_copy_(1, perm, t)
+        h = t.cpu().numpy()
+        out = np.empty_like(h)
+        out[:, perm.cpu().numpy()] = h
+        return out
+
+    def _check_flags(self, x_h, x_d, xs, perm, flags):
+        """BQ's post-checks from the per-problem OR of the status bits: ValueError for a non-finite point (bq.py:451-452);
+        per-point status is fetched only for problems with a bit other than ST_SHORTCUT | ST_NOTPD, which then get
+        ``BQ._report`` (bq.py:514-525: RuntimeError, or logged warnings for infinities) with the problem named."""
+        import torch
+        fl = flags.cpu().numpy()
+        if not (fl & ~(_lib.ST_SHORTCUT | _lib.ST_NOTPD)).any():
+            return
+        if x_h is None:
+            x_h = x_d.cpu().numpy()
+        bad = np.nonzero(fl & _lib.ST_XA_BAD)[0]
+        if bad.size:
+            p = int(bad[0])
+            row = x_h if x_h.ndim == 1 else x_h[p]
+            raise ValueError("invalid value for x_a of problem %d: %s" % (p, row[np.argmax(~np.isfinite(row))]))
+        na = x_d.shape[-1]
+        for p in np.nonzero(fl & ~(_lib.ST_SHORTCUT | _lib.ST_NOTPD))[0]:
+            p = int(p)
+            esm = torch.empty(1, na, dtype=torch.float64, device=x_d.device)
+            em, st = torch.empty_like(esm), torch.empty(1, na, dtype=torch.int32, device=x_d.device)
+            self.batch.score_device_range(p, 1, xs if xs.dim() == 1 else xs[p:p + 1], esm, em, st)
+            esm, em, st = (self._unsort(t, perm, False)[0] for t in (esm, em, st))
+            BQ._report(x_h if x_h.ndim == 1 else x_h[p], esm, em, st, where=" (problem %d)" % p)
+
+    def _score_all(self, x_a, want_em, on_device):
+        """(esm, em or None) [P, na] of every problem in one scoring pass over the batch."""
+        import torch
+        x_h, x_d = self._grid(x_a)
+        xs, perm = self._presort(x_h, x_d)
+        shape = (self.P, x_d.shape[-1])
+        esm = torch.empty(shape, dtype=torch.float64, device=x_d.device)
+        em = torch.empty_like(esm) if want_em else None
+        flags = torch.zeros(self.P, dtype=torch.int32, device=x_d.device)
+        if shape[1]:
+            self.batch.score_device(xs, esm, em, None, flags)
+        self._check_flags(x_h, x_d, xs, perm, flags)
+        return self._unsort(esm, perm, on_device), None if em is None else self._unsort(em, perm, on_device)
+
+    def expected_squared_mean(self, x_a, on_device=False):
+        """E[ E[Z|l_s,l_a]^2 ] of every problem at every point [P, na] (``BQ.expected_squared_mean``, bq.py:379-402)."""
+        return self._score_all(x_a, False, on_device)[0]
+
+    def expected_mean(self, x_a, on_device=False):
+        """E[ E[Z|l_s,l_a] ] of every problem at every point [P, na] (``BQ.expected_mean``, bq.py:404-423)."""
+        return self._score_all(x_a, True, on_device)[1]
+
+    def expected_squared_mean_and_mean(self, x_a, on_device=False):
+        """[P, na, 2] of (expected squared mean, expected mean) (``BQ.expected_squared_mean_and_mean``, bq.py:425-445)."""
+        esm, em = self._score_all(x_a, True, on_device)
+        if on_device:
+            import torch
+            return torch.stack([esm, em], dim=-1)
+        return np.stack([esm, em], axis=-1)
+
+    def expected_Z_var(self, x_a, on_device=False):
+        """E[V(Z) | l_s, l_a] = Z_mean^2 + Z_var - expected_squared_mean of every problem at every point [P, na]
+        (``BQ.expected_Z_var``, bq.py:354-377), bit for bit what ``bqb_expected_var_host`` gives each problem.
+
+        The problems are scored in chunks of whole problems through one LOSS_CHUNK_BYTES score buffer, and each chunk goes
+        through the expected-variance kernel while it is still in L2 (in place; on_device=True and no pre-sort: straight
+        into the result's rows).  Host results are copied back chunk by chunk, so besides an on_device result nothing
+        of size [P, na] is allocated on the device.  Problems with Z_mean <= 0 or Z_var <= 0 get one warning per call."""
+        import torch
+        x_h, x_d = self._grid(x_a)
+        for name, v in (("m_Z", self.info["Z_mean"]), ("V_Z", self.info["Z_var"])):       # bq_c.pyx:210-211, :352-353
+            bad = np.nonzero(v <= 0)[0]
+            if bad.size:
+                warnings.warn("%s = %s in problems %s" % (name, v[bad], bad.tolist()))
+        xs, perm = self._presort(x_h, x_d)
+        dev, P, na = x_d.device, self.P, x_d.shape[-1]
+        out = torch.empty(P, na, dtype=torch.float64, device=dev) if on_device else np.empty((P, na))
+        flags = torch.zeros(P, dtype=torch.int32, device=dev)
+        per = max(1, min(P, self.LOSS_CHUNK_BYTES // max(8 * na, 1)))
+        esm = torch.empty(per, na, dtype=torch.float64, device=dev) if na else None
+        perm_h = None if perm is None or on_device else perm.cpu().numpy()
+        for q0 in range(0, P if na else 0, per):
+            cq = min(per, P - q0)
+            self.batch.score_device_range(q0, cq, xs if xs.dim() == 1 else xs[q0:q0 + cq], esm, None, None, flags[q0:q0 + cq])
+            if on_device and perm is None:
+                self.batch.expected_var_rows_device(q0, cq, esm, out[q0:q0 + cq])
+                continue
+            self.batch.expected_var_rows_device(q0, cq, esm, esm)
+            if on_device:
+                out[q0:q0 + cq].index_copy_(1, perm, esm[:cq])
+            elif perm is None:
+                torch.from_numpy(out[q0:q0 + cq]).copy_(esm[:cq])
+            else:
+                out[q0:q0 + cq, perm_h] = esm[:cq].cpu().numpy()
+        self._check_flags(x_h, x_d, xs, perm, flags)
+        return out
+
+    def _host_gps(self, p):
+        """``BQ.init``'s two GPs of problem p (bq.py:132-171) from the batch's state: gp_log_l over (x_s, log l_s), gp_l over
+        the observations and the candidates with their values l_c from the setup."""
+        n, c = int(self.ns[p]), int(self.nc[p])
+        h = self.hyp[p]
+        if self.periodic:
+            k_tl, k_l = PeriodicKernel(h[0], h[1], self.period[p, 0]), PeriodicKernel(h[3], h[4], self.period[p, 1])
+        else:
+            k_tl, k_l = GaussianKernel(h[0], h[1]), GaussianKernel(h[3], h[4])
+        x_s, l_s = self.x_s[p, :n], self.l_s[p, :n]
+        gp_log_l = GP(k_tl, x_s, np.log(l_s), s=h[2])
+        gp_l = GP(k_l, np.concatenate([x_s, self.x_c[p, :c]]), np.concatenate([l_s, self.info["l_c"][p, :c]]), s=h[5])
+        return gp_log_l, gp_l
+
+    def _predict(self, x):
+        """(gp_l.mean(x), diag gp_log_l.cov(x)) [P, na] as CUDA tensors, each problem by ``BQ._predict``'s route: one
+        prediction launch for the whole batch serves the Gaussian kernel in capacity classes up to 256 where s_l = 0 and
+        the problem's points are finite; host GP objects answer every other row (noisy gp_l, the periodic kernel, the 512
+        class: the factors on the device are those of the noise-free bordered matrix, and the generic kernel has no
+        prediction mode)."""
+        import torch
+        self.sync_host()
+        x_h, x_d = self._grid(x)
+        if x_h is None:
+            x_h = x_d.cpu().numpy()
+        finite = np.isfinite(x_h).all(axis=-1)
+        on_dev = (not self.periodic and self._cap_class <= 256) & (self.hyp[:, 5] == 0) & finite
+        m = torch.empty(self.P, x_d.shape[-1], dtype=torch.float64, device=x_d.device)
+        v = torch.empty_like(m)
+        if on_dev.any() and x_d.shape[-1]:
+            self.batch.predict_device(x_d, m, v)
+        for p in np.nonzero(~on_dev)[0]:
+            gp_log_l, gp_l = self._host_gps(p)
+            row = x_h if x_h.ndim == 1 else x_h[p]
+            m[p] = torch.from_numpy(gp_l.mean(row))
+            v[p] = torch.from_numpy(np.diag(gp_log_l.cov(row)).copy())
+        return m, v
+
+    def l_mean(self, x, on_device=False):
+        """Mean of the final approximation to l of every problem [P, na] (``BQ.l_mean``, bq.py:177-200)."""
+        m, _ = self._predict(x)
+        return m if on_device else m.cpu().numpy()
+
+    def l_var(self, x, on_device=False):
+        """Marginal variance of the final approximation of every problem [P, na] (``BQ.l_var``, bq.py:202-231):
+        v_log_l * m_l^2, negative values set to 0."""
+        import torch
+        m, v = self._predict(x)
+        lv = v * (m * m)
+        lv = torch.where(lv < 0, torch.zeros_like(lv), lv)
+        return lv if on_device else lv.cpu().numpy()

@@ -354,24 +354,26 @@ class BQ(object):
         if bad.any():
             raise ValueError("invalid value for x_a: %s", x_a[np.argmax(bad)])
 
-    def _report(self, x_a, esm, em, status):
-        """The reference's post-checks (bq.py:514-525) on a vector of results."""
+    @staticmethod
+    def _report(x_a, esm, em, status, where=""):
+        """The reference's post-checks (bq.py:514-525) on a vector of results; ``where`` is appended to every message
+        (BatchBQ names the problem there)."""
         if status is None:
             return
         bad = (status & _lib.ST_ESM_BAD) != 0
         if bad.any():
             i = int(np.argmax(bad))
-            raise RuntimeError("invalid expected squared mean for x_a=%s: %s" % (x_a[[i]], esm[i]))
+            raise RuntimeError("invalid expected squared mean for x_a=%s: %s%s" % (x_a[[i]], esm[i], where))
         bad = (status & _lib.ST_EM_BAD) != 0
         if bad.any():
             i = int(np.argmax(bad))
-            raise RuntimeError("invalid expected mean for x_a=%s: %s" % (x_a[[i]], None if em is None else em[i]))
+            raise RuntimeError("invalid expected mean for x_a=%s: %s%s" % (x_a[[i]], None if em is None else em[i], where))
         for bit, name in ((_lib.ST_ESM_INF, "expected squared mean"), (_lib.ST_EM_INF, "expected mean")):
             idx = np.nonzero(status & bit)[0]
             for i in idx[:5]:
-                logger.warning("%s for x_a=%s is infinity!", name, x_a[[i]])
+                logger.warning("%s for x_a=%s is infinity!%s", name, x_a[[i]], where)
             if idx.size > 5:
-                logger.warning("%s is infinity for %d more points", name, idx.size - 5)
+                logger.warning("%s is infinity for %d more points%s", name, idx.size - 5, where)
 
     def _score(self, x_a, want_em=True):
         x_a = self._check_x_a(x_a)

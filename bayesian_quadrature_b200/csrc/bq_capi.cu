@@ -27,6 +27,8 @@ cudaError_t launch_sum_neg_accum(const double *esm, long long stride, int n_rows
 cudaError_t launch_sum_neg_groups(const double *esm, long long stride, int n_groups, int group_size, long long na, double *acc,
                                   long long acc_stride, cudaStream_t s);
 cudaError_t launch_expected_var(const double *esm, long long na, double msm, double *out, cudaStream_t s);
+cudaError_t launch_expected_var_rows(const double *models, long long model_stride, int inst0, int n_rows, const double *esm,
+                                     long long esm_stride, long long na, double *out, long long out_stride, cudaStream_t s);
 cudaError_t launch_argmin(const double *v, long long n, double *scratch_val, long long *scratch_idx, int sm_count,
                           cudaStream_t s);
 cudaError_t launch_argmin_rows(const double *v, long long stride, long long n, int rows, double *mins, long long *idxs,
@@ -899,6 +901,22 @@ int bqb_expected_var_device(bqb_batch *b, int inst, const double *d_esm, long lo
     const double *h = &b->h_hdr[(size_t)inst * H_COUNT];
     CU(cudaSetDevice(b->device));
     CU(launch_expected_var(d_esm, na, h[H_ZM] * h[H_ZM] + h[H_ZV], d_out, (cudaStream_t)stream));   // bq.py:374-377
+    b->launches++;
+    return 0;
+}
+
+int bqb_expected_var_rows_device(bqb_batch *b, int inst0, int n_inst, const double *d_esm, long long esm_stride, long long na,
+                                 double *d_out, long long out_stride, void *stream) {
+    if (!b || inst0 < 0 || n_inst < 0 || inst0 > b->n_inst - n_inst)
+        return fail(BQB_EINVAL, "bqb_expected_var_rows_device: bad instance range");
+    if (na < 0 || esm_stride < na || out_stride < na) return fail(BQB_EINVAL, "bqb_expected_var_rows_device: bad arguments");
+    if (na == 0 || n_inst == 0) return 0;
+    int rc = check_ready(b, "bqb_expected_var_rows_device");
+    if (rc) return rc;
+    if (!d_esm || !d_out) return fail(BQB_EINVAL, "bqb_expected_var_rows_device: bad arguments");
+    CU(cudaSetDevice(b->device));
+    CU(launch_expected_var_rows(b->d_models, b->lay.total, inst0, n_inst, d_esm, esm_stride, na, d_out, out_stride,
+                                (cudaStream_t)stream));
     b->launches++;
     return 0;
 }

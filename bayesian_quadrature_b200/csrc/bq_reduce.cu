@@ -48,6 +48,22 @@ __global__ void expected_var_kernel(const double *__restrict__ esm, long long na
         out[p] = msm - esm[p];
 }
 
+// Row-wise expected variance of instances [inst0, inst0 + n_rows): out[r][p] = (Zm^2 + Zv) - esm[r][p] with Zm / Zv read
+// from each instance's model header on the device (so that a device-resident setup needs no host round trip).  The
+// rounding steps are those of the host entry point (Zm * Zm + Zv on the host, then one subtraction) and of the fused
+// epilogue of the scoring kernels, spelled out so that no FMA contraction can change the bits.  esm and out may alias.
+__global__ void expected_var_rows_kernel(const double *models, long long model_stride, int inst0, int n_rows, const double *esm,
+                                         long long esm_stride, long long na, double *out, long long out_stride) {
+    for (int r = blockIdx.y; r < n_rows; r += gridDim.y) {
+        const double *M = models + (size_t)(inst0 + r) * model_stride;
+        const double msm = __dadd_rn(__dmul_rn(M[H_ZM], M[H_ZM]), M[H_ZV]);          // bq.py:374
+        const double *e = esm + (size_t)r * esm_stride;
+        double *o = out + (size_t)r * out_stride;
+        for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < na; p += (long long)gridDim.x * blockDim.x)
+            o[p] = __dsub_rn(msm, e[p]);
+    }
+}
+
 __device__ __forceinline__ void better(double &v, long long &i, double v2, long long i2) {
     // NaN never wins; ties keep the smaller index (np.argmin semantics for finite data)
     if (v2 < v || (v2 == v && i2 < i)) { v = v2; i = i2; }
@@ -159,6 +175,15 @@ cudaError_t launch_sum_neg_groups(const double *esm, long long stride, int n_gro
 cudaError_t launch_expected_var(const double *esm, long long na, double msm, double *out, cudaStream_t s) {
     const int blocks = (int)((na + 255) / 256 < 2368 ? (na + 255) / 256 : 2368);
     expected_var_kernel<<<blocks > 0 ? blocks : 1, 256, 0, s>>>(esm, na, msm, out);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_expected_var_rows(const double *models, long long model_stride, int inst0, int n_rows, const double *esm,
+                                     long long esm_stride, long long na, double *out, long long out_stride, cudaStream_t s) {
+    const int bx = (int)((na + 255) / 256 < 2368 ? (na + 255) / 256 : 2368);
+    const int by = n_rows < 65535 ? n_rows : 65535;
+    expected_var_rows_kernel<<<dim3(bx > 0 ? bx : 1, by > 0 ? by : 1), 256, 0, s>>>(models, model_stride, inst0, n_rows, esm,
+                                                                                  esm_stride, na, out, out_stride);
     return cudaGetLastError();
 }
 

@@ -201,6 +201,14 @@ int bqb_predict_host(bqb_batch *b, const double *x, long long x_stride, int na, 
 int bqb_expected_var_device(bqb_batch *b, int inst, const double *d_esm, long long na, double *d_out,
                             void *stream);
 
+/* out[r][p] = Z_mean^2 + Z_var - esm[r][p] for the instances [inst0, inst0 + n_inst), row r of esm (at r * esm_stride) and of
+ * out (at r * out_stride) belonging to instance inst0 + r: BQ.expected_Z_var of many problems (bq.py:374-377).  Z_mean and
+ * Z_var are read from the model blocks on the device; every row has the bits of bqb_expected_var_host for its instance.
+ * esm and out may be the same buffer.  BQB_EINVAL for a bad range or strides < na, BQB_ESTATE when the batch was not set
+ * up; na = 0 or n_inst = 0 does nothing.  DEVICE pointers, asynchronous on `stream`. */
+int bqb_expected_var_rows_device(bqb_batch *b, int inst0, int n_inst, const double *d_esm, long long esm_stride, long long na,
+                                 double *d_out, long long out_stride, void *stream);
+
 /* BQ.expected_Z_var(x_a) (bq.py:354-377) end to end for instance `inst`: HOST x_a in, HOST
  * out[p] = Z_mean^2 + Z_var - esm[p]; *flags_out = OR of the points' status bits.  Synchronous. */
 int bqb_expected_var_host(bqb_batch *b, int inst, const double *x_a, int na, double *out, int *flags_out);
