@@ -142,6 +142,21 @@ def _ptr(t):
     return ctypes.c_void_p(t.data_ptr())
 
 
+def _stream(stream):
+    """A CUDA stream handle as the C-ABI takes it (None: the legacy default stream)."""
+    return _vp(stream) if stream else None
+
+
+def _query(x, n_inst=None, name="x_a"):
+    """(row stride, na) of query points x: [na] shared by every instance (stride 0) or [B, na], a numpy array or a torch
+    tensor.  With ``n_inst`` a 2-D x must have that many rows."""
+    if x.ndim == 1:
+        return 0, x.shape[0]
+    if n_inst is not None and x.shape[0] != n_inst:
+        raise ValueError("%s must be [na] or [n_inst, na]" % name)
+    return (x.shape[1] if isinstance(x, np.ndarray) else x.stride(0)), x.shape[1]
+
+
 class Batch(object):
     """B model instances (one BQ problem under one hyper-parameter set each) resident on one GPU."""
 
@@ -174,7 +189,7 @@ class Batch(object):
         hyp, prior = _d(hyp).reshape(B, 6), _d(prior).reshape(B, 3)
         _check(load().bqb_batch_setup(self._h, ns.ctypes.data_as(_ip), nc.ctypes.data_as(_ip), _pd(x_s), _pd(l_s),
                                       x_s.shape[1], _pd(xc), _pd(hyp), _pd(prior), int(check_max),
-                                      _vp(stream) if stream else None), "bqb_batch_setup")
+                                      _stream(stream)), "bqb_batch_setup")
         self.ns, self.nc = ns, nc
         return self.info()
 
@@ -197,53 +212,47 @@ class Batch(object):
         x_s, l_s = _d(x_s).reshape(B, -1), _d(l_s).reshape(B, -1)
         hyp, prior = _d(hyp).reshape(B, 6), _d(prior).reshape(B, 3)
         _check(load().bqb_batch_stage(self._h, ns.ctypes.data_as(_ip), _pd(x_s), _pd(l_s), x_s.shape[1], _pd(hyp), _pd(prior),
-                                      _vp(stream) if stream else None), "bqb_batch_stage")
+                                      _stream(stream)), "bqb_batch_stage")
 
     def set_hypers(self, hyp, stream=None):
         """Replace the hyper-parameters [n_inst, 6] of the staged instances (the next setup_device uses them)."""
         hyp = _d(hyp).reshape(self.n_inst, 6)
-        _check(load().bqb_batch_set_hypers(self._h, _pd(hyp), _vp(stream) if stream else None), "bqb_batch_set_hypers")
+        _check(load().bqb_batch_set_hypers(self._h, _pd(hyp), _stream(stream)), "bqb_batch_set_hypers")
 
-    def log_lh_grad(self, hyp, inst=None, check_max=True, stream=None):
+    def log_lh_grad(self, hyp, inst=None, check_max=True, stream=None, period=None):
         """Joint log marginal likelihood and its gradient for rows of hyper-parameters hyp [n, 6] (h, w, s of gp_log_l,
         then of gp_l); row r is instance inst[r] (default: instance r).  Evaluated on the staged observations and
         candidates; the set-up model is left untouched.  Returns (log_lh [n], grad [n, 6], status [n]); a row whose status
-        is not SETUP_OK has log_lh -inf and a NaN gradient."""
+        is not SETUP_OK has log_lh -inf and a NaN gradient.  A batch of the periodic kernel takes the periods of every row,
+        period [n, 2] = (p of gp_log_l, p of gp_l), and returns grad [n, 8] in the order h_tl, w_tl, s_tl, h_l, w_l, s_l,
+        p_tl, p_l."""
         hyp = _d(hyp).reshape(-1, 6)
         n = hyp.shape[0]
+        if period is not None:
+            period = _d(period).reshape(-1, 2)
+            if period.shape[0] != n:
+                raise ValueError("period must have one row per row of hyp")
         if inst is not None:
             inst = np.ascontiguousarray(inst, dtype=np.int32).reshape(-1)
             if inst.shape[0] != n:
                 raise ValueError("inst must have one entry per row of hyp")
-        llh, grad, st = np.empty(n), np.empty((n, 6)), np.empty(n, dtype=np.int32)
-        _check(load().bqb_batch_log_lh_grad(self._h, _pd(hyp), inst.ctypes.data_as(_ip) if inst is not None else None, n,
-                                            int(check_max), _pd(llh), _pd(grad), st.ctypes.data_as(_ip),
-                                            _vp(stream) if stream else None), "bqb_batch_log_lh_grad")
+        llh, grad, st = np.empty(n), np.empty((n, 6 if period is None else 8)), np.empty(n, dtype=np.int32)
+        rows = (inst.ctypes.data_as(_ip) if inst is not None else None, n, int(check_max), _pd(llh), _pd(grad),
+                st.ctypes.data_as(_ip), _stream(stream))
+        if period is None:
+            _check(load().bqb_batch_log_lh_grad(self._h, _pd(hyp), *rows), "bqb_batch_log_lh_grad")
+        else:
+            _check(load().bqb_batch_log_lh_grad_periodic(self._h, _pd(hyp), _pd(period), *rows), "bqb_batch_log_lh_grad_periodic")
         return llh, grad, st
 
     def log_lh_grad_periodic(self, hyp, period, inst=None, check_max=True, stream=None):
-        """log_lh_grad for a batch of the periodic kernel: row r also has its periods period[r] = (p of gp_log_l, p of gp_l).
-        Returns (log_lh [n], grad [n, 8], status [n]), the gradient in the order h_tl, w_tl, s_tl, h_l, w_l, s_l, p_tl, p_l."""
-        hyp = _d(hyp).reshape(-1, 6)
-        n = hyp.shape[0]
-        period = _d(period).reshape(-1, 2)
-        if period.shape[0] != n:
-            raise ValueError("period must have one row per row of hyp")
-        if inst is not None:
-            inst = np.ascontiguousarray(inst, dtype=np.int32).reshape(-1)
-            if inst.shape[0] != n:
-                raise ValueError("inst must have one entry per row of hyp")
-        llh, grad, st = np.empty(n), np.empty((n, 8)), np.empty(n, dtype=np.int32)
-        _check(load().bqb_batch_log_lh_grad_periodic(self._h, _pd(hyp), _pd(period),
-                                                     inst.ctypes.data_as(_ip) if inst is not None else None, n, int(check_max),
-                                                     _pd(llh), _pd(grad), st.ctypes.data_as(_ip), _vp(stream) if stream else None),
-               "bqb_batch_log_lh_grad_periodic")
-        return llh, grad, st
+        """log_lh_grad(hyp, inst, check_max, stream, period=period): the periodic kernel's form under its own name."""
+        return self.log_lh_grad(hyp, inst, check_max, stream, period=period)
 
     def set_periods(self, period, stream=None):
         """Replace the periods [n_inst, 2] of a batch of the periodic kernel (the next setup_device uses them)."""
         period = _d(period).reshape(self.n_inst, 2)
-        _check(load().bqb_batch_set_periods(self._h, _pd(period), _vp(stream) if stream else None), "bqb_batch_set_periods")
+        _check(load().bqb_batch_set_periods(self._h, _pd(period), _stream(stream)), "bqb_batch_set_periods")
 
     def set_approx(self, kernel_kind=0, period=None, xo=None, p_xo=None, force_generic=False):
         """Kernel kind (0 Gaussian, 1 periodic with period [n_inst, 2] = p of gp_log_l / gp_l) and, when ``xo`` / ``p_xo``
@@ -267,7 +276,7 @@ class Batch(object):
                                            int(n_xo), int(stride), int(bool(force_generic))), "bqb_batch_set_approx")
 
     def setup_device(self, check_max=False, stream=None):
-        _check(load().bqb_batch_setup_device(self._h, int(check_max), _vp(stream) if stream else None), "bqb_batch_setup_device")
+        _check(load().bqb_batch_setup_device(self._h, int(check_max), _stream(stream)), "bqb_batch_setup_device")
         return self.info()
 
     def seed_candidates(self, seeds, stream=None):
@@ -275,7 +284,7 @@ class Batch(object):
         if seeds.shape != (self.n_inst,):
             raise ValueError("one 32-bit seed per instance")
         _check(load().bqb_batch_seed_candidates(self._h, seeds.ctypes.data_as(ctypes.POINTER(ctypes.c_uint)),
-                                                _vp(stream) if stream else None), "bqb_batch_seed_candidates")
+                                                _stream(stream)), "bqb_batch_seed_candidates")
 
     def rng_get(self):
         """(words [624, n_inst] uint32, positions [n_inst] int32) of the per-instance MT19937 generators."""
@@ -294,17 +303,17 @@ class Batch(object):
                "bqb_batch_rng_set")
 
     def draw_candidates(self, n_candidate, stream=None):
-        _check(load().bqb_batch_draw_candidates(self._h, int(n_candidate), _vp(stream) if stream else None),
+        _check(load().bqb_batch_draw_candidates(self._h, int(n_candidate), _stream(stream)),
                "bqb_batch_draw_candidates")
 
     def draw_candidates_wrapped(self, n_candidate, stream=None):
         """draw_candidates on [-pi p_tl, pi p_tl] (periodic kernel)."""
-        _check(load().bqb_batch_draw_candidates_wrapped(self._h, int(n_candidate), _vp(stream) if stream else None),
+        _check(load().bqb_batch_draw_candidates_wrapped(self._h, int(n_candidate), _stream(stream)),
                "bqb_batch_draw_candidates_wrapped")
 
     def add_observations(self, x_new, l_new, stream=None):
         """x_new, l_new: float64 CUDA tensors [n_inst]."""
-        _check(load().bqb_batch_add_observations(self._h, _ptr(x_new), _ptr(l_new), _vp(stream) if stream else None),
+        _check(load().bqb_batch_add_observations(self._h, _ptr(x_new), _ptr(l_new), _stream(stream)),
                "bqb_batch_add_observations")
 
     def get_staged(self):
@@ -319,12 +328,7 @@ class Batch(object):
         """x_a: [na] shared by all instances, or [B, na].  Returns (esm, em, status) as [B, na] numpy arrays."""
         x_a = _d(x_a)
         B = self.n_inst
-        if x_a.ndim == 1:
-            stride, na = 0, x_a.shape[0]
-        else:
-            if x_a.shape[0] != B:
-                raise ValueError("x_a must be [na] or [n_inst, na]")
-            stride, na = x_a.shape[1], x_a.shape[1]
+        stride, na = _query(x_a, B)
         esm = np.empty((B, na))
         em = np.empty((B, na)) if want_em else None
         st = np.empty((B, na), dtype=np.int32) if want_status else None
@@ -336,24 +340,16 @@ class Batch(object):
         """(l_mean, v_log_l) as [B, na] numpy arrays for x [na] (shared) or [B, na]: gp_l.mean(x), diag gp_log_l.cov(x)."""
         x = _d(x)
         B = self.n_inst
-        if x.ndim == 1:
-            stride, na = 0, x.shape[0]
-        else:
-            if x.shape[0] != B:
-                raise ValueError("x must be [na] or [n_inst, na]")
-            stride, na = x.shape[1], x.shape[1]
+        stride, na = _query(x, B, "x")
         m, v = np.empty((B, na)), np.empty((B, na))
         _check(load().bqb_predict_host(self._h, _pd(x), stride, na, _pd(m), _pd(v)), "bqb_predict_host")
         return m, v
 
     def predict_device(self, x, l_mean, v_log_l, stream=None):
         """torch CUDA tensors: x float64 [na] or [B, na]; outputs float64 [B, na]."""
-        if x.dim() == 1:
-            stride, na = 0, x.shape[0]
-        else:
-            stride, na = x.stride(0), x.shape[1]
+        stride, na = _query(x)
         _check(load().bqb_predict_device(self._h, _ptr(x), stride, na, _ptr(l_mean), _ptr(v_log_l), l_mean.stride(0),
-                                         _vp(stream) if stream else None), "bqb_predict_device")
+                                         _stream(stream)), "bqb_predict_device")
 
     def expected_var_host(self, x_a, inst=0, out=None):
         """BQ.expected_Z_var for one instance: numpy in, numpy out, plus the OR of the status bits.
@@ -368,55 +364,46 @@ class Batch(object):
 
     def score_device(self, x_a, esm, em=None, status=None, flags=None, stream=None):
         """torch CUDA tensors: x_a float64 [na] or [B, na]; esm/em float64 [B, na]; status int32 [B, na]."""
-        if x_a.dim() == 1:
-            stride, na = 0, x_a.shape[0]
-        else:
-            stride, na = x_a.stride(0), x_a.shape[1]
+        stride, na = _query(x_a)
         out_stride = esm.stride(0) if esm.dim() == 2 else esm.shape[0]
         _check(load().bqb_score_device(self._h, _ptr(x_a), stride, na, _ptr(esm), _ptr(em), _ptr(status), out_stride,
-                                       _ptr(flags), _vp(stream) if stream else None), "bqb_score_device")
+                                       _ptr(flags), _stream(stream)), "bqb_score_device")
 
     def score_device_range(self, inst0, n_inst, x_a, esm, em=None, status=None, flags=None, stream=None):
         """score_device for instances [inst0, inst0 + n_inst); row 0 of esm / em / status / flags belongs to inst0."""
-        if x_a.dim() == 1:
-            stride, na = 0, x_a.shape[0]
-        else:
-            stride, na = x_a.stride(0), x_a.shape[1]
+        stride, na = _query(x_a)
         out_stride = esm.stride(0) if esm.dim() == 2 else esm.shape[0]
         _check(load().bqb_score_device_range(self._h, int(inst0), int(n_inst), _ptr(x_a), stride, na, _ptr(esm), _ptr(em),
-                                             _ptr(status), out_stride, _ptr(flags), _vp(stream) if stream else None),
+                                             _ptr(status), out_stride, _ptr(flags), _stream(stream)),
                "bqb_score_device_range")
 
     def score_device_grouped(self, inst0, n_inst, x_a, xa_group, esm, em=None, status=None, flags=None, stream=None):
         """score_device_range where instance inst0 + i reads row i // xa_group of x_a [n_inst / xa_group, na] (or the shared
         [na]); inst0 must be a multiple of xa_group."""
-        if x_a.dim() == 1:
-            stride, na = 0, x_a.shape[0]
-        else:
-            stride, na = x_a.stride(0), x_a.shape[1]
-            if xa_group >= 1 and x_a.shape[0] < -(-int(n_inst) // int(xa_group)):
-                raise ValueError("x_a has %d rows; %d instances in groups of %d read %d" % (
-                    x_a.shape[0], n_inst, xa_group, -(-int(n_inst) // int(xa_group))))
+        stride, na = _query(x_a)
+        if x_a.dim() != 1 and xa_group >= 1 and x_a.shape[0] < -(-int(n_inst) // int(xa_group)):
+            raise ValueError("x_a has %d rows; %d instances in groups of %d read %d" % (
+                x_a.shape[0], n_inst, xa_group, -(-int(n_inst) // int(xa_group))))
         out_stride = esm.stride(0) if esm.dim() == 2 else esm.shape[0]
         _check(load().bqb_score_device_grouped(self._h, int(inst0), int(n_inst), _ptr(x_a), stride, int(xa_group), na, _ptr(esm),
-                                               _ptr(em), _ptr(status), out_stride, _ptr(flags), _vp(stream) if stream else None),
+                                               _ptr(em), _ptr(status), out_stride, _ptr(flags), _stream(stream)),
                "bqb_score_device_grouped")
 
     def sum_neg_accum_groups_device(self, esm, n_groups, group_size, acc, stream=None):
         """acc[g] += sum over rows g*group_size ... (g+1)*group_size - 1 of -esm, in row order, for g < n_groups."""
         acc_stride = acc.stride(0) if acc.dim() == 2 else acc.shape[0]
         _check(load().bqb_sum_neg_accum_groups_device(self._h, _ptr(esm), esm.stride(0), int(n_groups), int(group_size), esm.shape[1],
-                                                      _ptr(acc), acc_stride, _vp(stream) if stream else None),
+                                                      _ptr(acc), acc_stride, _stream(stream)),
                "bqb_sum_neg_accum_groups_device")
 
     def sum_neg_accum_device(self, esm, n_rows, acc, stream=None):
         """acc[p] += sum over the first n_rows rows of -esm[:, p], in row order (running form of mean_neg_device)."""
         _check(load().bqb_sum_neg_accum_device(self._h, _ptr(esm), esm.stride(0), int(n_rows), esm.shape[1], _ptr(acc),
-                                               _vp(stream) if stream else None), "bqb_sum_neg_accum_device")
+                                               _stream(stream)), "bqb_sum_neg_accum_device")
 
     def expected_var_device(self, inst, esm, out, stream=None):
         _check(load().bqb_expected_var_device(self._h, int(inst), _ptr(esm), esm.numel(), _ptr(out),
-                                              _vp(stream) if stream else None), "bqb_expected_var_device")
+                                              _stream(stream)), "bqb_expected_var_device")
 
     def expected_var_rows_device(self, inst0, n_inst, esm, out, stream=None):
         """out[r] = Z_mean^2 + Z_var - esm[r] for instances inst0 + r, r < n_inst: float64 CUDA tensors [>= n_inst, na] with
@@ -426,39 +413,39 @@ class Batch(object):
         if (esm.shape[1] > 1 and esm.stride(1) != 1) or (out.shape[1] > 1 and out.stride(1) != 1):
             raise ValueError("esm and out must have contiguous rows")
         _check(load().bqb_expected_var_rows_device(self._h, int(inst0), int(n_inst), _ptr(esm), esm.stride(0), esm.shape[1],
-                                                   _ptr(out), out.stride(0), _vp(stream) if stream else None),
+                                                   _ptr(out), out.stride(0), _stream(stream)),
                "bqb_expected_var_rows_device")
 
     def mean_neg_device(self, esm, loss, stream=None):
         _check(load().bqb_mean_neg_device(self._h, _ptr(esm), esm.stride(0), esm.shape[1], _ptr(loss),
-                                          _vp(stream) if stream else None), "bqb_mean_neg_device")
+                                          _stream(stream)), "bqb_mean_neg_device")
 
     def argmin_device(self, v, stream=None):
         mn, idx = ctypes.c_double(0), _ll(0)
         _check(load().bqb_argmin_device(self._h, _ptr(v), v.numel(), ctypes.byref(mn), ctypes.byref(idx),
-                                        _vp(stream) if stream else None), "bqb_argmin_device")
+                                        _stream(stream)), "bqb_argmin_device")
         return mn.value, idx.value
 
     def argmin_pair_device(self, v, offset, pair, stream=None):
         """(min, first index + offset) of `v` written to the 2-element float64 CUDA tensor `pair`; no host sync."""
         _check(load().bqb_argmin_pair_device(self._h, _ptr(v), v.numel(), int(offset), _ptr(pair),
-                                             _vp(stream) if stream else None), "bqb_argmin_pair_device")
+                                             _stream(stream)), "bqb_argmin_pair_device")
 
     def choose_step_device(self, x_a, esm, ev, pair, offset=0, inst=0, stream=None):
         """Fused esm + expected variance + (min, first index + offset) for one instance; CUDA tensors, no host sync."""
         _check(load().bqb_choose_step_device(self._h, int(inst), _ptr(x_a), x_a.numel(), _ptr(esm), _ptr(ev), int(offset),
-                                             _ptr(pair), _vp(stream) if stream else None), "bqb_choose_step_device")
+                                             _ptr(pair), _stream(stream)), "bqb_choose_step_device")
 
     def choose_step_exchange(self, x_a, esm, ev, offset, peer_ptrs, world, rank, seq, out_ptr, inst=0, stream=None, cyclic_block=0):
         """choose_step_device + cross-rank exchange in the reduction kernel (see dist.PairExchange); no host sync."""
         _check(load().bqb_choose_step_exchange(self._h, int(inst), _ptr(x_a), x_a.numel(), _ptr(esm), _ptr(ev), int(offset),
                                                int(cyclic_block), peer_ptrs, int(world), int(rank), int(seq), _vp(out_ptr),
-                                               _vp(stream) if stream else None), "bqb_choose_step_exchange")
+                                               _stream(stream)), "bqb_choose_step_exchange")
 
     def argmin_rows_device(self, v, mins, idxs, stream=None):
         """Per-instance (min, first index) of the CUDA tensor v [n_inst, n] into mins (float64) / idxs (int64)."""
         _check(load().bqb_argmin_rows_device(self._h, _ptr(v), v.stride(0), v.shape[1], _ptr(mins), _ptr(idxs),
-                                             _vp(stream) if stream else None), "bqb_argmin_rows_device")
+                                             _stream(stream)), "bqb_argmin_rows_device")
 
     def set_cutoff(self, cut_arg):
         """Relevance cut-off of the band skipping (default 72; float('inf') = dense algorithm)."""

@@ -325,10 +325,8 @@ class BatchBQ(object):
         ll, grad = np.full(rows.size, -np.inf), np.full((rows.size, hyp.shape[1]), np.nan)
         ok = self._valid_hyp(hyp)
         if ok.any():
-            if self.periodic:
-                l, g, st = self.batch.log_lh_grad_periodic(hyp[ok, :6], hyp[ok, 6:], inst=rows[ok], check_max=True)
-            else:
-                l, g, st = self.batch.log_lh_grad(hyp[ok], inst=rows[ok], check_max=True)
+            l, g, st = self.batch.log_lh_grad(hyp[ok, :6], inst=rows[ok], check_max=True,
+                                              period=hyp[ok, 6:] if self.periodic else None)
             good = (st == _lib.SETUP_OK) & np.isfinite(l)
             idx = np.nonzero(ok)[0][good]
             ll[idx], grad[idx] = l[good], g[good]

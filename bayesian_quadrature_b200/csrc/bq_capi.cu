@@ -21,19 +21,15 @@ size_t setup2_scratch_stride(int cap);
 cudaError_t launch_score(const ScoreArgs &a, int n_inst, int sm_count, cudaStream_t stream, int *grid_x = nullptr);
 cudaError_t launch_score_generic(const ScoreArgs &a, int n_inst, cudaStream_t stream, int *grid_x);
 cudaError_t launch_argmin_partials(double *bv, long long *bi, int nblocks, long long offset, double *pair, cudaStream_t s);
-cudaError_t launch_mean_neg(const double *esm, long long stride, int n_inst, long long na, double *loss, cudaStream_t s);
 cudaError_t launch_pack_info(const double *models, long long model_stride, int off_lc, int n_inst, double *out, cudaStream_t s);
-cudaError_t launch_sum_neg_accum(const double *esm, long long stride, int n_rows, long long na, double *acc, cudaStream_t s);
 cudaError_t launch_sum_neg_groups(const double *esm, long long stride, int n_groups, int group_size, long long na, double *acc,
-                                  long long acc_stride, cudaStream_t s);
-cudaError_t launch_expected_var(const double *esm, long long na, double msm, double *out, cudaStream_t s);
+                                  long long acc_stride, bool mean, cudaStream_t s);
 cudaError_t launch_expected_var_rows(const double *models, long long model_stride, int inst0, int n_rows, const double *esm,
                                      long long esm_stride, long long na, double *out, long long out_stride, cudaStream_t s);
-cudaError_t launch_argmin(const double *v, long long n, double *scratch_val, long long *scratch_idx, int sm_count,
+cudaError_t launch_argmin(const double *v, long long n, double *bv, long long *bi, int sm_count, long long offset, double *pair,
                           cudaStream_t s);
 cudaError_t launch_argmin_rows(const double *v, long long stride, long long n, int rows, double *mins, long long *idxs,
                                cudaStream_t s);
-cudaError_t launch_argmin_pair(const double *bv, const long long *bi, long long offset, double *pair, cudaStream_t s);
 cudaError_t launch_argmin_exchange(const double *bv, const long long *bi, int nblocks, long long offset, long long cyc_block,
                                    void *const *peer_slots, int world, int rank, unsigned long long seq, double *out, cudaStream_t s);
 cudaError_t sort_points(const double *d_x, int n, double *d_x_sorted, int *d_iota, int *d_perm, void *temp, size_t *temp_bytes,
@@ -580,6 +576,26 @@ static cudaError_t score_dispatch(bqb_batch *b, ScoreArgs &a, int n_inst, cudaSt
     return launch_score(a, n_inst, b->sm_count, s, grid_x);
 }
 
+// The scoring arguments that come from the batch, with a.models beginning at instance `first`
+static ScoreArgs score_args(const bqb_batch *b, int first = 0) {
+    ScoreArgs a;
+    a.models = b->d_models + (size_t)first * b->lay.total; a.lay = b->lay; a.exp_tab = b->d_tab;
+    a.cut_arg = b->cut_arg; a.work = b->d_work_ctr;
+    a.nb_max = b->nb_max; a.nrow_max = b->nrow_max; a.ndb_max = b->ndb_max;
+    return a;
+}
+
+// Instances [first, first + count) of a batch-wide launch (a.models at instance 0), in launches of at most 32768
+// instances: gridDim.y is limited to 65535
+static int score_chunks(bqb_batch *b, ScoreArgs &a, int first, int count, cudaStream_t s) {
+    for (int i0 = first; i0 < first + count; i0 += 32768) {
+        a.inst0 = i0;
+        CU(score_dispatch(b, a, std::min(first + count - i0, 32768), s));
+        b->launches++;
+    }
+    return 0;
+}
+
 static int check_ready(bqb_batch *b, const char *who) {
     if (!b || !b->ready) return fail(BQB_ESTATE, std::string(who) + ": batch was not set up");
     for (int i = 0; i < b->n_inst; ++i)
@@ -665,22 +681,13 @@ static int score_device_impl(bqb_batch *b, const double *d_x_a, long long xa_str
     if (na == 0) return 0;
     if (count < 0) count = b->n_inst - first;
     CU(cudaSetDevice(b->device));
-    ScoreArgs a;
-    a.cut_arg = b->cut_arg; a.work = b->d_work_ctr; a.nb_max = b->nb_max; a.nrow_max = b->nrow_max;
-    a.models = b->d_models; a.lay = b->lay; a.x_a = d_x_a - (size_t)(first / xa_group) * xa_stride; a.xa_stride = xa_stride;
-    a.xa_group = xa_group; a.na = na;
+    ScoreArgs a = score_args(b);
+    a.x_a = d_x_a - (size_t)(first / xa_group) * xa_stride; a.xa_stride = xa_stride; a.xa_group = xa_group; a.na = na;
     a.esm = d_esm - (size_t)first * out_stride; a.em = d_em ? d_em - (size_t)first * out_stride : nullptr;
-    a.status = d_status ? d_status - (size_t)first * out_stride : nullptr; a.out_stride = out_stride; a.exp_tab = b->d_tab;
-    a.flags = d_flags ? d_flags - first : nullptr; a.ndb_max = b->ndb_max; a.perm = d_perm;
+    a.status = d_status ? d_status - (size_t)first * out_stride : nullptr; a.out_stride = out_stride;
+    a.flags = d_flags ? d_flags - first : nullptr; a.perm = d_perm;
     if (d_flags) CU(cudaMemsetAsync(d_flags, 0, sizeof(int) * count, (cudaStream_t)stream));
-    // gridDim.y is limited to 65535
-    for (int i0 = first; i0 < first + count; i0 += 32768) {
-        const int cnt = (first + count - i0 < 32768) ? first + count - i0 : 32768;
-        a.inst0 = i0;
-        CU(score_dispatch(b, a, cnt, (cudaStream_t)stream));
-        b->launches++;
-    }
-    return 0;
+    return score_chunks(b, a, first, count, (cudaStream_t)stream);
 }
 
 int bqb_predict_device(bqb_batch *b, const double *d_x, long long x_stride, int na, double *d_l_mean, double *d_v_log_l,
@@ -691,18 +698,10 @@ int bqb_predict_device(bqb_batch *b, const double *d_x, long long x_stride, int 
     if (!d_x || !d_l_mean || !d_v_log_l || na < 0 || out_stride < na) return fail(BQB_EINVAL, "bqb_predict_device: bad arguments");
     if (na == 0) return 0;
     CU(cudaSetDevice(b->device));
-    ScoreArgs a;
-    a.cut_arg = b->cut_arg; a.work = b->d_work_ctr; a.nb_max = b->nb_max; a.nrow_max = b->nrow_max;
-    a.models = b->d_models; a.lay = b->lay; a.x_a = d_x; a.xa_stride = x_stride; a.na = na;
-    a.esm = d_l_mean; a.em = d_v_log_l; a.status = nullptr; a.out_stride = out_stride; a.exp_tab = b->d_tab;
-    a.flags = nullptr; a.ndb_max = b->ndb_max; a.predict = 1;
-    for (int i0 = 0; i0 < b->n_inst; i0 += 32768) {
-        const int cnt = (b->n_inst - i0 < 32768) ? b->n_inst - i0 : 32768;
-        a.inst0 = i0;
-        CU(score_dispatch(b, a, cnt, (cudaStream_t)stream));
-        b->launches++;
-    }
-    return 0;
+    ScoreArgs a = score_args(b);
+    a.x_a = d_x; a.xa_stride = x_stride; a.na = na;
+    a.esm = d_l_mean; a.em = d_v_log_l; a.out_stride = out_stride; a.predict = 1;
+    return score_chunks(b, a, 0, b->n_inst, (cudaStream_t)stream);
 }
 
 static int grow(bqb_batch *b, size_t n_xa, size_t n_out) {
@@ -802,8 +801,6 @@ int bqb_expected_var_host(bqb_batch *b, int inst, const double *x_a, int na, dou
     if (!b->d_flags) CU(cudaMalloc(&b->d_flags, sizeof(int) * b->n_inst));
     if (!b->h_flags) CU(cudaMallocHost(&b->h_flags, sizeof(int)));
     for (cudaStream_t &st : b->pipe) if (!st) CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    const double *h = &b->h_hdr[(size_t)inst * H_COUNT];
-    const double msm = h[H_ZM] * h[H_ZM] + h[H_ZV];                                    // bq.py:374
     // Buffers that are not page-locked go through device staging in chunks that alternate between two streams, so
     // that the H2D copy of one chunk, the kernels of another and the D2H copy of a third overlap.
     static const int min_chunk = getenv("BQB_PIPE_CHUNK") ? atoi(getenv("BQB_PIPE_CHUNK")) : (1 << 18);
@@ -816,11 +813,8 @@ int bqb_expected_var_host(bqb_batch *b, int inst, const double *x_a, int na, dou
     if (!zc) CU(cudaMemsetAsync(b->d_flags, 0, sizeof(int) * b->n_inst, b->pipe[0]));
     if (nchunk > 1) CU(cudaStreamSynchronize(b->pipe[0]));
     int zc_grid = 0;
-    ScoreArgs a;
-    a.cut_arg = b->cut_arg; a.work = b->d_work_ctr; a.nb_max = b->nb_max; a.nrow_max = b->nrow_max;
-    a.models = b->d_models + (size_t)inst * b->lay.total; a.lay = b->lay; a.xa_stride = 0;
-    a.em = nullptr; a.status = nullptr; a.exp_tab = b->d_tab; a.flags = zc ? nullptr : b->d_flags; a.inst0 = 0; a.ndb_max = b->ndb_max;
-    a.cta_flags = zc ? b->h_cta_flags : nullptr;
+    ScoreArgs a = score_args(b, inst);
+    a.flags = zc ? nullptr : b->d_flags; a.cta_flags = zc ? b->h_cta_flags : nullptr;
     int c = 0;
     for (int lo = 0; lo < na; lo += per, ++c) {
         const int n = (na - lo < per) ? na - lo : per;
@@ -846,7 +840,7 @@ int bqb_expected_var_host(bqb_batch *b, int inst, const double *x_a, int na, dou
         } else {
             a.esm = b->d_esm + lo; a.ev = nullptr;
             CU(score_dispatch(b, a, 1, s, nullptr, inst));
-            CU(launch_expected_var(b->d_esm + lo, n, msm, b->d_em + lo, s));
+            CU(launch_expected_var_rows(b->d_models, b->lay.total, inst, 1, b->d_esm + lo, n, n, b->d_em + lo, n, s));
             b->launches += 2;
             CU(cudaMemcpyAsync(out + lo, b->d_em + lo, sizeof(double) * n, cudaMemcpyDeviceToHost, s));
         }
@@ -868,7 +862,7 @@ int bqb_expected_var_host(bqb_batch *b, int inst, const double *x_a, int na, dou
 int bqb_mean_neg_device(bqb_batch *b, const double *d_esm, long long stride, long long na, double *d_loss, void *stream) {
     if (!b || !d_esm || !d_loss || na < 0) return fail(BQB_EINVAL, "bqb_mean_neg_device: bad arguments");
     CU(cudaSetDevice(b->device));
-    CU(launch_mean_neg(d_esm, stride, b->n_inst, na, d_loss, (cudaStream_t)stream));
+    CU(launch_sum_neg_groups(d_esm, stride, 1, b->n_inst, na, d_loss, 0, true, (cudaStream_t)stream));
     b->launches++;
     return 0;
 }
@@ -877,7 +871,7 @@ int bqb_sum_neg_accum_device(bqb_batch *b, const double *d_esm, long long stride
     if (!b || !d_esm || !d_acc || na < 0 || n_rows < 0 || stride < na) return fail(BQB_EINVAL, "bqb_sum_neg_accum_device: bad arguments");
     if (na == 0 || n_rows == 0) return 0;
     CU(cudaSetDevice(b->device));
-    CU(launch_sum_neg_accum(d_esm, stride, n_rows, na, d_acc, (cudaStream_t)stream));
+    CU(launch_sum_neg_groups(d_esm, stride, 1, n_rows, na, d_acc, 0, false, (cudaStream_t)stream));
     b->launches++;
     return 0;
 }
@@ -889,7 +883,7 @@ int bqb_sum_neg_accum_groups_device(bqb_batch *b, const double *d_esm, long long
     if (!d_esm || !d_acc || stride < na || (n_groups > 1 && acc_stride < na))
         return fail(BQB_EINVAL, "bqb_sum_neg_accum_groups_device: bad arguments");
     CU(cudaSetDevice(b->device));
-    CU(launch_sum_neg_groups(d_esm, stride, n_groups, group_size, na, d_acc, acc_stride, (cudaStream_t)stream));
+    CU(launch_sum_neg_groups(d_esm, stride, n_groups, group_size, na, d_acc, acc_stride, false, (cudaStream_t)stream));
     b->launches++;
     return 0;
 }
@@ -898,9 +892,8 @@ int bqb_expected_var_device(bqb_batch *b, int inst, const double *d_esm, long lo
     int rc = check_ready(b, "bqb_expected_var_device");
     if (rc) return rc;
     if (inst < 0 || inst >= b->n_inst || !d_esm || !d_out) return fail(BQB_EINVAL, "bqb_expected_var_device: bad arguments");
-    const double *h = &b->h_hdr[(size_t)inst * H_COUNT];
     CU(cudaSetDevice(b->device));
-    CU(launch_expected_var(d_esm, na, h[H_ZM] * h[H_ZM] + h[H_ZV], d_out, (cudaStream_t)stream));   // bq.py:374-377
+    CU(launch_expected_var_rows(b->d_models, b->lay.total, inst, 1, d_esm, na, na, d_out, na, (cudaStream_t)stream));
     b->launches++;
     return 0;
 }
@@ -925,7 +918,7 @@ int bqb_argmin_device(bqb_batch *b, const double *d_v, long long n, double *min_
     if (!b || !d_v || n < 1 || !min_out || !idx_out) return fail(BQB_EINVAL, "bqb_argmin_device: bad arguments");
     CU(cudaSetDevice(b->device));
     cudaStream_t s = (cudaStream_t)stream;
-    CU(launch_argmin(d_v, n, b->d_red_val, b->d_red_idx, b->sm_count, s));
+    CU(launch_argmin(d_v, n, b->d_red_val, b->d_red_idx, b->sm_count, 0, nullptr, s));
     b->launches += 2;
     CU(cudaMemcpyAsync(min_out, b->d_red_val, sizeof(double), cudaMemcpyDeviceToHost, s));
     CU(cudaMemcpyAsync(idx_out, b->d_red_idx, sizeof(long long), cudaMemcpyDeviceToHost, s));
@@ -936,10 +929,20 @@ int bqb_argmin_device(bqb_batch *b, const double *d_v, long long n, double *min_
 int bqb_argmin_pair_device(bqb_batch *b, const double *d_v, long long n, long long offset, double *d_pair, void *stream) {
     if (!b || !d_v || n < 1 || !d_pair) return fail(BQB_EINVAL, "bqb_argmin_pair_device: bad arguments");
     CU(cudaSetDevice(b->device));
-    cudaStream_t s = (cudaStream_t)stream;
-    CU(launch_argmin(d_v, n, b->d_red_val, b->d_red_idx, b->sm_count, s));
-    CU(launch_argmin_pair(b->d_red_val, b->d_red_idx, offset, d_pair, s));
-    b->launches += 3;
+    CU(launch_argmin(d_v, n, b->d_red_val, b->d_red_idx, b->sm_count, offset, d_pair, (cudaStream_t)stream));
+    b->launches += 2;
+    return 0;
+}
+
+// The scoring launch of a choose_next step: esm and the fused expected variance of instance `inst`, with the per-CTA
+// (min, first index) partials of the expected variance in b->d_red_val / b->d_red_idx and their number in *grid_x
+static int choose_step_score(bqb_batch *b, int inst, const double *d_x_a, int na, double *d_esm, double *d_ev, cudaStream_t s,
+                             int *grid_x) {
+    CU(cudaSetDevice(b->device));
+    ScoreArgs a = score_args(b, inst);
+    a.x_a = d_x_a; a.na = na; a.esm = d_esm; a.out_stride = na;
+    a.ev = d_ev; a.part_val = b->d_red_val; a.part_idx = b->d_red_idx;
+    CU(score_dispatch(b, a, 1, s, grid_x, inst));
     return 0;
 }
 
@@ -949,16 +952,10 @@ int bqb_choose_step_device(bqb_batch *b, int inst, const double *d_x_a, int na, 
     if (rc) return rc;
     if (inst < 0 || inst >= b->n_inst || !d_x_a || !d_esm || !d_ev || !d_pair || na < 1)
         return fail(BQB_EINVAL, "bqb_choose_step_device: bad arguments");
-    CU(cudaSetDevice(b->device));
     cudaStream_t s = (cudaStream_t)stream;
-    ScoreArgs a;
-    a.cut_arg = b->cut_arg; a.work = b->d_work_ctr; a.nb_max = b->nb_max; a.nrow_max = b->nrow_max;
-    a.models = b->d_models + (size_t)inst * b->lay.total; a.lay = b->lay; a.x_a = d_x_a; a.xa_stride = 0; a.na = na;
-    a.esm = d_esm; a.em = nullptr; a.status = nullptr; a.out_stride = na; a.exp_tab = b->d_tab; a.flags = nullptr;
-    a.inst0 = 0; a.ndb_max = b->ndb_max;
-    a.ev = d_ev; a.part_val = b->d_red_val; a.part_idx = b->d_red_idx;
     int grid_x = 0;
-    CU(score_dispatch(b, a, 1, s, &grid_x, inst));
+    rc = choose_step_score(b, inst, d_x_a, na, d_esm, d_ev, s, &grid_x);
+    if (rc) return rc;
     CU(launch_argmin_partials(b->d_red_val, b->d_red_idx, grid_x, offset, d_pair, s));
     b->launches += 2;
     return 0;
@@ -972,16 +969,10 @@ int bqb_choose_step_exchange(bqb_batch *b, int inst, const double *d_x_a, int na
     if (inst < 0 || inst >= b->n_inst || !d_x_a || !d_ev || !peer_slots || !out4 || na < 1 || world < 1 || world > 16 || rank < 0 ||
         rank >= world || seq == 0 || cyclic_block < 0)
         return fail(BQB_EINVAL, "bqb_choose_step_exchange: bad arguments");
-    CU(cudaSetDevice(b->device));
     cudaStream_t s = (cudaStream_t)stream;
-    ScoreArgs a;
-    a.cut_arg = b->cut_arg; a.work = b->d_work_ctr; a.nb_max = b->nb_max; a.nrow_max = b->nrow_max;
-    a.models = b->d_models + (size_t)inst * b->lay.total; a.lay = b->lay; a.x_a = d_x_a; a.xa_stride = 0; a.na = na;
-    a.esm = d_esm; a.em = nullptr; a.status = nullptr; a.out_stride = na; a.exp_tab = b->d_tab; a.flags = nullptr;
-    a.inst0 = 0; a.ndb_max = b->ndb_max;
-    a.ev = d_ev; a.part_val = b->d_red_val; a.part_idx = b->d_red_idx;
     int grid_x = 0;
-    CU(score_dispatch(b, a, 1, s, &grid_x, inst));
+    rc = choose_step_score(b, inst, d_x_a, na, d_esm, d_ev, s, &grid_x);
+    if (rc) return rc;
     CU(launch_argmin_exchange(b->d_red_val, b->d_red_idx, grid_x, offset, cyclic_block, peer_slots, world, rank, seq, out4, s));
     b->launches += 2;
     return 0;

@@ -6,46 +6,32 @@
 
 namespace bqb {
 
-__global__ void mean_neg_kernel(const double *__restrict__ esm, long long stride, int n_inst, long long na,
-                                double *__restrict__ loss) {
-    for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < na; p += (long long)gridDim.x * blockDim.x) {
-        double s = 0;
-        for (int b = 0; b < n_inst; ++b) s += -esm[(size_t)b * stride + p];   // pairwise-free: sample order
-        loss[p] = s / n_inst;
-    }
+// CTAs of 256 threads for a grid-stride loop over n elements: one element per thread, at most `cap` CTAs, at least one
+static int grid_1d(long long n, long long cap = 2368) {
+    const long long blocks = (n + 255) / 256 < cap ? (n + 255) / 256 : cap;
+    return blocks > 0 ? (int)blocks : 1;
 }
 
-// acc[p] += -esm[0][p] - esm[1][p] - ... in row order, starting from acc[p]: walking a batch of hyper-parameter samples
-// through a chunk-sized score buffer performs exactly the additions of mean_neg_kernel (and of numpy's mean(axis=0)), in the
-// same order, without ever holding the [n_samples, na] matrix (819 MB at BASELINE configs[3]).
-__global__ void sum_neg_accum_kernel(const double *__restrict__ esm, long long stride, int n_rows, long long na, double *__restrict__ acc) {
-    for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < na; p += (long long)gridDim.x * blockDim.x) {
-        double s = acc[p];
-        for (int b = 0; b < n_rows; ++b) s += -esm[(size_t)b * stride + p];
-        acc[p] = s;
-    }
-}
-
-// Segmented form for many problems with S samples each: acc[g][p] += -esm[g*S][p] - esm[g*S+1][p] - ... in row order.  Per group
-// these are the additions of sum_neg_accum_kernel, so one group reproduces it bit for bit and a problem's samples may arrive
-// in chunks.  HBM-bound: every esm element is read once, acc is read and written once per launch.
+// Segmented sum for many problems with S samples each: acc[g][p] += -esm[g*S][p] - esm[g*S+1][p] - ... in row order,
+// starting from acc[g][p].  Walking a batch of hyper-parameter samples through a chunk-sized score buffer performs exactly
+// the additions of numpy's mean(axis=0), in the same order, without ever holding the [n_samples, na] matrix (819 MB at
+// BASELINE configs[3]), and a problem's samples may arrive in chunks.  MEAN: one group that starts from 0 and ends with
+// one division by the row count (the mean itself).  HBM-bound: every esm element is read once, acc is read and written
+// once per launch.
+template <bool MEAN>
 __global__ void sum_neg_groups_kernel(const double *__restrict__ esm, long long stride, int n_groups, int group_size, long long na,
                                       double *__restrict__ acc, long long acc_stride) {
-    for (int g = blockIdx.y; g < n_groups; g += gridDim.y) {
-        const double *e = esm + (size_t)g * group_size * stride;
-        double *a = acc + (size_t)g * acc_stride;
-        for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < na; p += (long long)gridDim.x * blockDim.x) {
-            double s = a[p];
-#pragma unroll 4
-            for (int r = 0; r < group_size; ++r) s += -e[(size_t)r * stride + p];
-            a[p] = s;
+    // (groups inside the point loop, row loop unrolled by the compiler: it then issues each row's load ahead of the previous
+    // row's addition, which measured fastest for all three entry points)
+    for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < na; p += (long long)gridDim.x * blockDim.x) {
+        for (int g = blockIdx.y; g < n_groups; g += gridDim.y) {
+            const double *e = esm + (size_t)g * group_size * stride + p;
+            double *a = acc + (size_t)g * acc_stride + p;
+            double s = MEAN ? 0.0 : *a;
+            for (int r = 0; r < group_size; ++r) s += -e[(size_t)r * stride];
+            *a = MEAN ? s / group_size : s;
         }
     }
-}
-
-__global__ void expected_var_kernel(const double *__restrict__ esm, long long na, double msm, double *__restrict__ out) {
-    for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < na; p += (long long)gridDim.x * blockDim.x)
-        out[p] = msm - esm[p];
 }
 
 // Row-wise expected variance of instances [inst0, inst0 + n_rows): out[r][p] = (Zm^2 + Zv) - esm[r][p] with Zm / Zv read
@@ -59,73 +45,85 @@ __global__ void expected_var_rows_kernel(const double *models, long long model_s
         const double msm = __dadd_rn(__dmul_rn(M[H_ZM], M[H_ZM]), M[H_ZV]);          // bq.py:374
         const double *e = esm + (size_t)r * esm_stride;
         double *o = out + (size_t)r * out_stride;
-        for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < na; p += (long long)gridDim.x * blockDim.x)
-            o[p] = __dsub_rn(msm, e[p]);
+        // esm and out may alias, so the compiler keeps each load behind the store before it: eight loads are issued ahead
+        // of their stores to keep enough of them in flight
+        const long long G = (long long)gridDim.x * blockDim.x;
+        long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+        for (; p + 7 * G < na; p += 8 * G) {
+            double v[8];
+#pragma unroll
+            for (int k = 0; k < 8; ++k) v[k] = e[p + k * G];
+#pragma unroll
+            for (int k = 0; k < 8; ++k) o[p + k * G] = __dsub_rn(msm, v[k]);
+        }
+        for (; p < na; p += G) o[p] = __dsub_rn(msm, e[p]);
     }
 }
 
+// ---- (min, first index) of double vectors
+// The rule: NaN never wins, ties keep the smaller index (np.argmin semantics for finite data).  It selects the
+// lexicographically smallest non-NaN (value, index) pair, so the result does not depend on the order of the reduction.
+constexpr long long NO_INDEX = 0x7fffffffffffffffLL;
+
 __device__ __forceinline__ void better(double &v, long long &i, double v2, long long i2) {
-    // NaN never wins; ties keep the smaller index (np.argmin semantics for finite data)
     if (v2 < v || (v2 == v && i2 < i)) { v = v2; i = i2; }
 }
 
-__global__ void argmin_kernel(const double *__restrict__ v, long long n, double *bv, long long *bi) {
+__device__ __forceinline__ void warp_argmin(double &v, long long &i) {            // every lane ends with the warp's pair
+    for (int o = 16; o > 0; o >>= 1) {
+        const double v2 = __shfl_xor_sync(0xffffffffu, v, o);
+        const long long i2 = __shfl_xor_sync(0xffffffffu, i, o);
+        better(v, i, v2, i2);
+    }
+}
+
+__device__ __forceinline__ void block_argmin(double &v, long long &i) {           // thread 0 ends with the CTA's pair
     __shared__ double sv[32];
     __shared__ long long si[32];
+    warp_argmin(v, i);
+    if ((threadIdx.x & 31) == 0) { sv[threadIdx.x >> 5] = v; si[threadIdx.x >> 5] = i; }
+    __syncthreads();
+    if (threadIdx.x == 0)
+        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) better(v, i, sv[w], si[w]);
+}
+
+// One warp: the pair of nblocks per-CTA partials (argmin_kernel's or the scoring epilogue's), in every lane
+__device__ __forceinline__ void partials_argmin(const double *bv, const long long *bi, int nblocks, double &v, long long &i) {
+    v = INFINITY;
+    i = NO_INDEX;
+    for (int b = threadIdx.x; b < nblocks; b += 32) better(v, i, bv[b], bi[b]);
+    warp_argmin(v, i);
+}
+
+__global__ void argmin_kernel(const double *__restrict__ v, long long n, double *bv, long long *bi) {
     double best = INFINITY;
-    long long idx = 0x7fffffffffffffffLL;
+    long long idx = NO_INDEX;
     for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < n; p += (long long)gridDim.x * blockDim.x)
         better(best, idx, v[p], p);
-    for (int o = 16; o > 0; o >>= 1) {
-        const double v2 = __shfl_xor_sync(0xffffffffu, best, o);
-        const long long i2 = __shfl_xor_sync(0xffffffffu, idx, o);
-        better(best, idx, v2, i2);
-    }
-    if ((threadIdx.x & 31) == 0) { sv[threadIdx.x >> 5] = best; si[threadIdx.x >> 5] = idx; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) better(best, idx, sv[w], si[w]);
-        bv[blockIdx.x] = best;
-        bi[blockIdx.x] = idx;
-    }
-}
-
-__global__ void argmin_final_kernel(double *bv, long long *bi, int nblocks) {   // one warp
-    double best = INFINITY;
-    long long idx = 0x7fffffffffffffffLL;
-    for (int b = threadIdx.x; b < nblocks; b += 32) better(best, idx, bv[b], bi[b]);
-    for (int o = 16; o > 0; o >>= 1) {
-        const double v2 = __shfl_xor_sync(0xffffffffu, best, o);
-        const long long i2 = __shfl_xor_sync(0xffffffffu, idx, o);
-        better(best, idx, v2, i2);
-    }
-    if (threadIdx.x == 0) { bv[0] = best; bi[0] = idx; }
-}
-
-// (min, global index as a double) pair for the cross-rank exchange: exact for indices < 2^53
-__global__ void argmin_pair_kernel(const double *bv, const long long *bi, long long offset, double *pair) {
-    if (threadIdx.x == 0) { pair[0] = bv[0]; pair[1] = (double)(bi[0] + offset); }
+    block_argmin(best, idx);
+    if (threadIdx.x == 0) { bv[blockIdx.x] = best; bi[blockIdx.x] = idx; }
 }
 
 // One CTA per row: (min, first index) of every instance's score vector (C5: per-problem argmin)
 __global__ void argmin_rows_kernel(const double *__restrict__ v, long long stride, long long n, double *mins, long long *idxs) {
-    __shared__ double sv[32];
-    __shared__ long long si[32];
     const double *row = v + (size_t)blockIdx.x * stride;
     double best = INFINITY;
-    long long idx = 0x7fffffffffffffffLL;
+    long long idx = NO_INDEX;
     for (long long p = threadIdx.x; p < n; p += blockDim.x) better(best, idx, row[p], p);
-    for (int o = 16; o > 0; o >>= 1) {
-        const double v2 = __shfl_xor_sync(0xffffffffu, best, o);
-        const long long i2 = __shfl_xor_sync(0xffffffffu, idx, o);
-        better(best, idx, v2, i2);
-    }
-    if ((threadIdx.x & 31) == 0) { sv[threadIdx.x >> 5] = best; si[threadIdx.x >> 5] = idx; }
-    __syncthreads();
+    block_argmin(best, idx);
+    if (threadIdx.x == 0) { mins[blockIdx.x] = best; idxs[blockIdx.x] = idx; }
+}
+
+// One warp: reduces the per-CTA partials into bv[0] / bi[0] and, when `pair` is given, emits the (min, global index as a
+// double) pair for the cross-rank exchange: exact for indices < 2^53
+__global__ void argmin_partials_kernel(double *bv, long long *bi, int nblocks, long long offset, double *pair) {
+    double best;
+    long long idx;
+    partials_argmin(bv, bi, nblocks, best, idx);
     if (threadIdx.x == 0) {
-        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) better(best, idx, sv[w], si[w]);
-        mins[blockIdx.x] = best;
-        idxs[blockIdx.x] = idx;
+        bv[0] = best;
+        bi[0] = idx;
+        if (pair) { pair[0] = best; pair[1] = (double)(idx + offset); }
     }
 }
 
@@ -140,9 +138,7 @@ __global__ void pack_info_kernel(const double *__restrict__ models, long long mo
     }
 }
 cudaError_t launch_pack_info(const double *models, long long model_stride, int off_lc, int n_inst, double *out, cudaStream_t s) {
-    const long long n = (long long)n_inst * (H_COUNT + NC_MAX);
-    const int blocks = (int)((n + 255) / 256 < 1184 ? (n + 255) / 256 : 1184);
-    pack_info_kernel<<<blocks > 0 ? blocks : 1, 256, 0, s>>>(models, model_stride, off_lc, n_inst, out);
+    pack_info_kernel<<<grid_1d((long long)n_inst * (H_COUNT + NC_MAX), 1184), 256, 0, s>>>(models, model_stride, off_lc, n_inst, out);
     return cudaGetLastError();
 }
 
@@ -152,62 +148,38 @@ cudaError_t launch_argmin_rows(const double *v, long long stride, long long n, i
     return cudaGetLastError();
 }
 
-cudaError_t launch_mean_neg(const double *esm, long long stride, int n_inst, long long na, double *loss, cudaStream_t s) {
-    const int blocks = (int)((na + 255) / 256 < 2368 ? (na + 255) / 256 : 2368);
-    mean_neg_kernel<<<blocks > 0 ? blocks : 1, 256, 0, s>>>(esm, stride, n_inst, na, loss);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_sum_neg_accum(const double *esm, long long stride, int n_rows, long long na, double *acc, cudaStream_t s) {
-    const int blocks = (int)((na + 255) / 256 < 2368 ? (na + 255) / 256 : 2368);
-    sum_neg_accum_kernel<<<blocks > 0 ? blocks : 1, 256, 0, s>>>(esm, stride, n_rows, na, acc);
-    return cudaGetLastError();
-}
-
+// mean = false: acc[g] += the negated rows of group g; mean = true: acc = the mean of the negated rows of one group
 cudaError_t launch_sum_neg_groups(const double *esm, long long stride, int n_groups, int group_size, long long na, double *acc,
-                                  long long acc_stride, cudaStream_t s) {
-    const int bx = (int)((na + 255) / 256 < 2368 ? (na + 255) / 256 : 2368);
-    const int by = n_groups < 65535 ? n_groups : 65535;
-    sum_neg_groups_kernel<<<dim3(bx > 0 ? bx : 1, by > 0 ? by : 1), 256, 0, s>>>(esm, stride, n_groups, group_size, na, acc, acc_stride);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_expected_var(const double *esm, long long na, double msm, double *out, cudaStream_t s) {
-    const int blocks = (int)((na + 255) / 256 < 2368 ? (na + 255) / 256 : 2368);
-    expected_var_kernel<<<blocks > 0 ? blocks : 1, 256, 0, s>>>(esm, na, msm, out);
+                                  long long acc_stride, bool mean, cudaStream_t s) {
+    const dim3 grid(grid_1d(na), n_groups < 1 ? 1 : n_groups < 65535 ? n_groups : 65535);
+    if (mean)
+        sum_neg_groups_kernel<true><<<grid, 256, 0, s>>>(esm, stride, n_groups, group_size, na, acc, acc_stride);
+    else
+        sum_neg_groups_kernel<false><<<grid, 256, 0, s>>>(esm, stride, n_groups, group_size, na, acc, acc_stride);
     return cudaGetLastError();
 }
 
 cudaError_t launch_expected_var_rows(const double *models, long long model_stride, int inst0, int n_rows, const double *esm,
                                      long long esm_stride, long long na, double *out, long long out_stride, cudaStream_t s) {
-    const int bx = (int)((na + 255) / 256 < 2368 ? (na + 255) / 256 : 2368);
-    const int by = n_rows < 65535 ? n_rows : 65535;
-    expected_var_rows_kernel<<<dim3(bx > 0 ? bx : 1, by > 0 ? by : 1), 256, 0, s>>>(models, model_stride, inst0, n_rows, esm,
-                                                                                  esm_stride, na, out, out_stride);
+    const dim3 grid(grid_1d(na), n_rows < 1 ? 1 : n_rows < 65535 ? n_rows : 65535);
+    expected_var_rows_kernel<<<grid, 256, 0, s>>>(models, model_stride, inst0, n_rows, esm, esm_stride, na, out, out_stride);
     return cudaGetLastError();
 }
 
-cudaError_t launch_argmin(const double *v, long long n, double *bv, long long *bi, int sm_count, cudaStream_t s) {
+cudaError_t launch_argmin_partials(double *bv, long long *bi, int nblocks, long long offset, double *pair, cudaStream_t s) {
+    argmin_partials_kernel<<<1, 32, 0, s>>>(bv, bi, nblocks, offset, pair);
+    return cudaGetLastError();
+}
+
+// (min, first index) of v [n] into bv[0] / bi[0] (bv / bi hold the per-CTA partials first), and into pair when given
+cudaError_t launch_argmin(const double *v, long long n, double *bv, long long *bi, int sm_count, long long offset, double *pair,
+                          cudaStream_t s) {
     int blocks = (int)((n + 1023) / 1024);
     if (blocks > sm_count * 2) blocks = sm_count * 2;
     if (blocks > 4096) blocks = 4096;
     if (blocks < 1) blocks = 1;
     argmin_kernel<<<blocks, 256, 0, s>>>(v, n, bv, bi);
-    argmin_final_kernel<<<1, 32, 0, s>>>(bv, bi, blocks);
-    return cudaGetLastError();
-}
-
-// final step of the fused scoring epilogue: reduce the per-CTA partials and emit the (min, index + offset) pair
-__global__ void argmin_partials_kernel(double *bv, long long *bi, int nblocks, long long offset, double *pair) {
-    double best = INFINITY;
-    long long idx = 0x7fffffffffffffffLL;
-    for (int b = threadIdx.x; b < nblocks; b += 32) better(best, idx, bv[b], bi[b]);
-    for (int o = 16; o > 0; o >>= 1) {
-        const double v2 = __shfl_xor_sync(0xffffffffu, best, o);
-        const long long i2 = __shfl_xor_sync(0xffffffffu, idx, o);
-        better(best, idx, v2, i2);
-    }
-    if (threadIdx.x == 0) { pair[0] = best; pair[1] = (double)(idx + offset); }
+    return launch_argmin_partials(bv, bi, blocks, offset, pair, s);
 }
 
 // Fused "reduce + exchange" of choose_next over a sharded query vector (bq.py:663 across ranks): the one warp that
@@ -223,14 +195,9 @@ struct PeerSlots {
 __global__ void argmin_exchange_kernel(const double *bv, const long long *bi, int nblocks, long long offset, long long cyc_block,
                                        PeerSlots peers, int world, int rank, unsigned long long seq, double *out) {
     const int lane = threadIdx.x;
-    double best = INFINITY;
-    long long idx = 0x7fffffffffffffffLL;
-    for (int b = lane; b < nblocks; b += 32) better(best, idx, bv[b], bi[b]);
-    for (int o = 16; o > 0; o >>= 1) {
-        const double v2 = __shfl_xor_sync(0xffffffffu, best, o);
-        const long long i2 = __shfl_xor_sync(0xffffffffu, idx, o);
-        better(best, idx, v2, i2);
-    }
+    double best;
+    long long idx;
+    partials_argmin(bv, bi, nblocks, best, idx);
     const int par = (int)(seq & 1ull);
     const double tag = (double)seq;
     if (lane < world) {                                   // lane r publishes to rank r
@@ -277,16 +244,6 @@ cudaError_t launch_argmin_exchange(const double *bv, const long long *bi, int nb
     PeerSlots p;
     for (int r = 0; r < 16; ++r) p.slot[r] = r < world ? (double *)peer_slots[r] : nullptr;
     argmin_exchange_kernel<<<1, 32, 0, s>>>(bv, bi, nblocks, offset, cyc_block, p, world, rank, seq, out);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_argmin_partials(double *bv, long long *bi, int nblocks, long long offset, double *pair, cudaStream_t s) {
-    argmin_partials_kernel<<<1, 32, 0, s>>>(bv, bi, nblocks, offset, pair);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_argmin_pair(const double *bv, const long long *bi, long long offset, double *pair, cudaStream_t s) {
-    argmin_pair_kernel<<<1, 32, 0, s>>>(bv, bi, offset, pair);
     return cudaGetLastError();
 }
 

@@ -119,7 +119,7 @@ def test_grouped_scoring_equals_replicated_rows(ns, generic):
 def test_segmented_reduction_matches_sum_neg_accum(na):
     import torch
     from bayesian_quadrature_b200 import _lib
-    b = _lib.Batch(1, 16)
+    b = _lib.Batch(13, 16)                                # mean_neg_device averages the first n_inst = 13 rows
     g = torch.Generator(device="cuda").manual_seed(na)
     esm = torch.rand(16, na, dtype=torch.float64, device="cuda", generator=g) * 1e-3 - 3e-4
     start = torch.rand(3, na, dtype=torch.float64, device="cuda", generator=g)
@@ -127,12 +127,27 @@ def test_segmented_reduction_matches_sum_neg_accum(na):
         b.sum_neg_accum_groups_device(esm, 3, 5, start)
         b.close()
         return
+
+    def neg_sum(acc, rows):                               # the additions of numpy's mean(axis=0), in row order
+        acc = acc.clone()
+        for r in rows:
+            acc += -r
+        return acc
+
     # one group of 16 rows, starting from a non-zero accumulator
-    want = start[0].clone()
-    b.sum_neg_accum_device(esm, 16, want)
+    want = neg_sum(start[0], esm)
+    acc = start[0].clone()
+    b.sum_neg_accum_device(esm, 16, acc)
+    assert torch.equal(acc, want)
     got = start[:1].clone()
     b.sum_neg_accum_groups_device(esm, 1, 16, got)
     assert torch.equal(got[0], want)
+    # the mean over the batch's 13 rows: the same additions from 0, then one division (in numpy: torch divides by a
+    # scalar as a multiplication with its reciprocal)
+    loss = torch.full((na,), np.nan, dtype=torch.float64, device="cuda")
+    b.mean_neg_device(esm, loss)
+    want = neg_sum(torch.zeros(na, dtype=torch.float64, device="cuda"), esm[:13]).cpu().numpy() / 13
+    assert np.array_equal(loss.cpu().numpy(), want)
     # S = 1: every row its own group
     got = start.clone()
     b.sum_neg_accum_groups_device(esm, 3, 1, got)
@@ -141,9 +156,11 @@ def test_segmented_reduction_matches_sum_neg_accum(na):
     got = start.clone()
     b.sum_neg_accum_groups_device(esm, 3, 5, got)
     for k in range(3):
-        want = start[k].clone()
-        b.sum_neg_accum_device(esm[5 * k:5 * k + 5], 5, want)
+        want = neg_sum(start[k], esm[5 * k:5 * k + 5])
         assert torch.equal(got[k], want), k
+        acc = start[k].clone()
+        b.sum_neg_accum_device(esm[5 * k:5 * k + 5], 5, acc)
+        assert torch.equal(acc, want), k
     b.close()
 
 

@@ -164,11 +164,13 @@ def test_host_and_device_resident_modes_agree(kind):
 
 @pytest.mark.parametrize("kind", ["gauss", "periodic"])
 def test_rows_kernel_equals_the_single_instance_path(kind):
-    """bqb_expected_var_rows_device: every row has the bits of bqb_expected_var_host of its instance, for strided rows of
-    esm and out, a first instance > 0 and na = 0, 1, 7, 257; esm and out may be one buffer."""
+    """bqb_expected_var_rows_device: every row has the bits of bqb_expected_var_host of its instance (staged, and with a
+    page-locked output through the scoring kernel's fused epilogue) and of (Zm * Zm + Zv) - esm in numpy, for strided rows
+    of esm and out, a first instance > 0 and na = 0, 1, 7, 257; esm and out may be one buffer."""
     import torch
     bb, _, _, grid = gaussian_case(40, P=5) if kind == "gauss" else periodic_case(P=5)
     P = bb.P
+    zm, zv = bb.info["Z_mean"], bb.info["Z_var"]
     for na in (0, 1, 7, 257):
         x = np.linspace(grid[0], grid[-1], na)
         x_d = torch.from_numpy(x).cuda()
@@ -184,10 +186,15 @@ def test_rows_kernel_equals_the_single_instance_path(kind):
         assert (got[:, :2] == -1).all() and (got[:, na + 2:] == -1).all()     # nothing written outside the rows
         inplace = esm.clone()
         bb.batch.expected_var_rows_device(0, P, inplace, inplace)
+        esm_h = esm.cpu().numpy()
         for p in range(P):
             want, _ = bb.batch.expected_var_host(x, inst=p)
             assert np.array_equal(got[p, 2:na + 2], want), (na, p)
             assert np.array_equal(inplace[p].cpu().numpy(), want), (na, p)
+            assert np.array_equal(want, (zm[p] * zm[p] + zv[p]) - esm_h[p]), (na, p)
+            if na:
+                fused, _ = bb.batch.expected_var_host(x, inst=p, out=torch.empty(na, dtype=torch.float64).pin_memory().numpy())
+                assert np.array_equal(fused, want), (na, p)
         assert np.array_equal(bb.expected_Z_var(x), got[:, 2:na + 2])
         assert np.array_equal(bb.expected_Z_var(x_d, on_device=True).cpu().numpy(), got[:, 2:na + 2])
         for name in METHODS[1:]:
