@@ -54,6 +54,9 @@ SYMBOLS = {
     "bqb_sum_neg_accum_groups_device": (ctypes.c_int, [_vp, _vp, _ll, ctypes.c_int, ctypes.c_int, _ll, _vp, _ll, _vp]),
     "bqb_predict_device": (ctypes.c_int, [_vp, _vp, _ll, ctypes.c_int, _vp, _vp, _ll, _vp]),
     "bqb_predict_host": (ctypes.c_int, [_vp, _dp, _ll, ctypes.c_int, _dp, _dp]),
+    "bqb_predict_rows_device": (ctypes.c_int, [_vp, _ip, ctypes.c_int, _vp, _ll, ctypes.c_int, _vp, _vp, _ll, _vp]),
+    "bqb_predict_rows_host": (ctypes.c_int, [_vp, _ip, ctypes.c_int, _dp, _ll, ctypes.c_int, _dp, _dp]),
+    "bqb_alpha_read": (ctypes.c_int, [_vp, ctypes.c_int, _dp]),
     "bqb_expected_var_host": (ctypes.c_int, [_vp, ctypes.c_int, _dp, ctypes.c_int, _dp, _ip]),
     "bqb_score_host": (ctypes.c_int, [_vp, _dp, _ll, ctypes.c_int, _dp, _dp, _ip]),
     "bqb_expected_var_device": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _ll, _vp, _vp]),
@@ -350,6 +353,41 @@ class Batch(object):
         stride, na = _query(x)
         _check(load().bqb_predict_device(self._h, _ptr(x), stride, na, _ptr(l_mean), _ptr(v_log_l), l_mean.stride(0),
                                          _stream(stream)), "bqb_predict_device")
+
+    @staticmethod
+    def _rows(rows):
+        """(int32 array or None, its ctypes pointer or None, its length) of an instance list (None: every instance)."""
+        if rows is None:
+            return None, None, 0
+        rows = np.ascontiguousarray(rows, dtype=np.int32).reshape(-1)
+        return rows, rows.ctypes.data_as(_ip), rows.shape[0]
+
+    def predict_rows_host(self, x, rows=None):
+        """(l_mean, v_log_l) [B, na] numpy arrays for x [na] (shared) or [B, na]: gp_l.mean(x), diag gp_log_l.cov(x) of the
+        instances in ``rows`` (default: all), for any batch and any s_l; the rows of other instances are NaN."""
+        x = _d(x)
+        B = self.n_inst
+        stride, na = _query(x, B, "x")
+        m, v = np.full((B, na), np.nan), np.full((B, na), np.nan)
+        rows, rp, n = self._rows(rows)
+        _check(load().bqb_predict_rows_host(self._h, rp, n, _pd(x), stride, na, _pd(m), _pd(v)), "bqb_predict_rows_host")
+        return m, v
+
+    def predict_rows_device(self, x, l_mean, v_log_l, rows=None, stream=None):
+        """predict_rows_host on torch CUDA tensors: x float64 [na] or [B, na]; l_mean / v_log_l float64 [B, na] with unit
+        column stride.  Only the rows of the listed instances (default: all) are written; no host synchronisation."""
+        stride, na = _query(x)
+        rows, rp, n = self._rows(rows)
+        _check(load().bqb_predict_rows_device(self._h, rp, n, _ptr(x), stride, na, _ptr(l_mean), _ptr(v_log_l),
+                                              l_mean.stride(0), _stream(stream)), "bqb_predict_rows_device")
+
+    def read_alpha(self, inst=0):
+        """alpha_l = (K_l + s_l^2 I)^-1 l_sc of instance ``inst`` (ns + nc entries): observations in ascending order, then the
+        candidates, as in the model block."""
+        hdr = self.read_model(inst)                   # H_NS, H_NC: the counts of the last setup
+        out = np.empty(int(hdr[0]) + int(hdr[1]))
+        _check(load().bqb_alpha_read(self._h, int(inst), _pd(out)), "bqb_alpha_read")
+        return out
 
     def expected_var_host(self, x_a, inst=0, out=None):
         """BQ.expected_Z_var for one instance: numpy in, numpy out, plus the OR of the status bits.

@@ -768,23 +768,34 @@ class BatchBQ(object):
         return gp_log_l, gp_l
 
     def _predict(self, x):
-        """(gp_l.mean(x), diag gp_log_l.cov(x)) [P, na] as CUDA tensors, each problem by ``BQ._predict``'s route: one
-        prediction launch for the whole batch serves the Gaussian kernel in capacity classes up to 256 where s_l = 0 and
-        the problem's points are finite; host GP objects answer every other row (noisy gp_l, the periodic kernel, the 512
-        class: the factors on the device are those of the noise-free bordered matrix, and the generic kernel has no
-        prediction mode)."""
+        """(gp_l.mean(x), diag gp_log_l.cov(x)) [P, na] as CUDA tensors, each problem by ``BQ._predict``'s route.  A problem
+        whose points are all finite is answered on the device: the Gaussian kernel with s_l = 0 in a capacity class up to 256
+        by the scoring kernel's prediction mode (one launch for the batch), every other one (a noisy gp_l, the periodic
+        kernel, the 512 class) by one launch of the prediction kernel over those problems, after the first on the same
+        stream.  Only a problem with a non-finite point builds host GP objects; only then are a device-resident batch's host
+        mirrors refreshed, so that otherwise nothing but the grid and the result crosses PCIe."""
         import torch
-        self.sync_host()
         x_h, x_d = self._grid(x)
-        if x_h is None:
-            x_h = x_d.cpu().numpy()
-        finite = np.isfinite(x_h).all(axis=-1)
-        on_dev = (not self.periodic and self._cap_class <= 256) & (self.hyp[:, 5] == 0) & finite
-        m = torch.empty(self.P, x_d.shape[-1], dtype=torch.float64, device=x_d.device)
+        P, na = self.P, x_d.shape[-1]
+        if x_h is not None:
+            finite = np.isfinite(x_h).all(axis=-1)
+        else:
+            finite = torch.isfinite(x_d).all(dim=-1).cpu().numpy()
+        finite = np.broadcast_to(finite, (P,))
+        mode2 = (not self.periodic and self._cap_class <= 256) & (self.hyp[:, 5] == 0) & finite
+        rows = np.nonzero(finite & ~mode2)[0]
+        m = torch.empty(P, na, dtype=torch.float64, device=x_d.device)
         v = torch.empty_like(m)
-        if on_dev.any() and x_d.shape[-1]:
+        if na and mode2.any():
             self.batch.predict_device(x_d, m, v)
-        for p in np.nonzero(~on_dev)[0]:
+        if na and rows.size:
+            self.batch.predict_rows_device(x_d, m, v, rows=None if rows.size == P else rows)
+        host = np.nonzero(~finite)[0]
+        if host.size:
+            self.sync_host()
+            if x_h is None:
+                x_h = x_d.cpu().numpy()
+        for p in host:
             gp_log_l, gp_l = self._host_gps(p)
             row = x_h if x_h.ndim == 1 else x_h[p]
             m[p] = torch.from_numpy(gp_l.mean(row))
@@ -792,13 +803,15 @@ class BatchBQ(object):
         return m, v
 
     def l_mean(self, x, on_device=False):
-        """Mean of the final approximation to l of every problem [P, na] (``BQ.l_mean``, bq.py:177-200)."""
+        """Mean of the final approximation to l of every problem [P, na] (``BQ.l_mean``, bq.py:177-200): device launches for
+        every problem with finite points, host GPs for the others (``_predict``)."""
         m, _ = self._predict(x)
         return m if on_device else m.cpu().numpy()
 
     def l_var(self, x, on_device=False):
         """Marginal variance of the final approximation of every problem [P, na] (``BQ.l_var``, bq.py:202-231):
-        v_log_l * m_l^2, negative values set to 0."""
+        v_log_l * m_l^2, negative values set to 0, with both factors from ``_predict`` (device launches for every problem with
+        finite points, host GPs for the others)."""
         import torch
         m, v = self._predict(x)
         lv = v * (m * m)

@@ -289,25 +289,32 @@ class BQ(object):
             self._dev_model.close()
         self._dev_model = None
 
-    # ------------------------------------------------------------------ mean / variance of l (host GPs)
+    # ------------------------------------------------------------------ mean / variance of l
     def _predict(self, x):
-        """(gp_l.mean(x), diag gp_log_l.cov(x)) for a vector of points in one device pass; None when the device factors
-        do not apply (noisy gp_l: they are those of the noise-free bordered matrix) and the host GPs must answer."""
-        if self.options["use_approx"] or self.gp_l.get_param("s") != 0 or self.ns > 256:
-            return None                                  # (the generic kernel has no prediction mode)
+        """(gp_l.mean(x), diag gp_log_l.cov(x)) for a vector of finite points in one device pass; None for other input, which
+        the host GPs answer.  The Gaussian kernel with s_l = 0 in a tensor-core capacity class (ns <= 256) takes the
+        scoring kernel's prediction mode; every other problem (the trapezoid path, the periodic kernel, a noisy gp_l, the
+        512 class) takes the prediction kernel, which reads alpha_l = (K_l + s_l^2 I)^-1 l_sc from the setup."""
         x = np.ascontiguousarray(x, dtype=DTYPE)
         if x.ndim != 1 or not np.isfinite(x).all():
             return None
-        m, v = self._device_model().batch.predict_host(x)
+        batch = self._device_model().batch
+        if self.options["use_approx"] or self.gp_l.get_param("s") != 0 or self.ns > 256:
+            m, v = batch.predict_rows_host(x)
+        else:
+            m, v = batch.predict_host(x)
         return m[0], v[0]
 
     def l_mean(self, x):
-        """Mean of the final approximation to l: the mean of the GP over exp(log l) (bq.py:177-200)."""
+        """Mean of the final approximation to l: the mean of the GP over exp(log l) (bq.py:177-200).  One device pass for a
+        1-D vector of finite points whatever the kernel, s_l or number of observations (``_predict``); the host GPs answer
+        other input."""
         pred = self._predict(x)
         return self.gp_l.mean(x) if pred is None else pred[0]
 
     def l_var(self, x):
-        """Marginal variance of the final approximation (bq.py:202-231)."""
+        """Marginal variance of the final approximation (bq.py:202-231): v_log_l * m_l^2, negative values set to 0, with both
+        factors from one device pass for a 1-D vector of finite points (``_predict``), from the host GPs otherwise."""
         pred = self._predict(x)
         if pred is None:
             v_log_l = np.diag(self.gp_log_l.cov(x)).copy()

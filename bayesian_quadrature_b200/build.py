@@ -7,7 +7,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbq_b200.so")
-SOURCES = ["bq_setup2.cu", "bq_score.cu", "bq_score_generic.cu", "bq_reduce.cu", "bq_round.cu", "bq_sort.cu", "bq_capi.cu"]
+SOURCES = ["bq_setup2.cu", "bq_score.cu", "bq_score_generic.cu", "bq_predict.cu", "bq_reduce.cu", "bq_round.cu", "bq_sort.cu", "bq_capi.cu"]
 HEADERS = ["bq_common.cuh", os.path.join("..", "..", "include", "bq_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--fmad=true", "-Xptxas", "-v"]

@@ -20,6 +20,7 @@ int setup2_two_cta_limit(int nc_max);
 size_t setup2_scratch_stride(int cap);
 cudaError_t launch_score(const ScoreArgs &a, int n_inst, int sm_count, cudaStream_t stream, int *grid_x = nullptr);
 cudaError_t launch_score_generic(const ScoreArgs &a, int n_inst, cudaStream_t stream, int *grid_x);
+cudaError_t launch_predict(const PredictArgs &a, int n_rows, cudaStream_t stream);
 cudaError_t launch_argmin_partials(double *bv, long long *bi, int nblocks, long long offset, double *pair, cudaStream_t s);
 cudaError_t launch_pack_info(const double *models, long long model_stride, int off_lc, int n_inst, double *out, cudaStream_t s);
 cudaError_t launch_sum_neg_groups(const double *esm, long long stride, int n_groups, int group_size, long long na, double *acc,
@@ -70,6 +71,12 @@ struct bqb_batch {
     bool big_class = false;            // capacity 512: no tensor-core scoring kernels
     double *d_period = nullptr, *d_xo = nullptr, *d_pxo = nullptr, *d_wp = nullptr, *d_gz = nullptr;
     int *d_inst_list = nullptr;        // setup launch groups (instances ordered by size class)
+    // alpha_l of every instance, written by each setup ([n_inst][alpha_stride], model order, zero padded), and the instance
+    // list of bqb_predict_rows_device (grown on demand)
+    double *d_alpha = nullptr;
+    long long alpha_stride = 0;
+    int *d_rows = nullptr;
+    size_t cap_rows = 0;
     // bqb_batch_log_lh_grad(_periodic): hyper-parameter rows, periods, instance list and output rows (grown on demand)
     double *d_llg_hyp = nullptr, *d_llg_out = nullptr, *d_llg_period = nullptr;
     int *d_llg_inst = nullptr;
@@ -164,6 +171,8 @@ int bqb_batch_create(bqb_batch **out, int device, int n_inst, int ns_max) {
     CU(cudaMalloc(&b->d_xc, sizeof(double) * (size_t)n_inst * NC_MAX));
     CU(cudaMalloc(&b->d_hyp, sizeof(double) * (size_t)n_inst * 6));
     CU(cudaMalloc(&b->d_prior, sizeof(double) * (size_t)n_inst * 3));
+    b->alpha_stride = cap + NC_MAX;
+    CU(cudaMalloc(&b->d_alpha, sizeof(double) * (size_t)n_inst * b->alpha_stride));
     CU(cudaMalloc(&b->d_red_val, sizeof(double) * 4096));
     CU(cudaMalloc(&b->d_red_idx, sizeof(long long) * 4096));
     if (getenv("BQB_DENSE") && atoi(getenv("BQB_DENSE"))) b->cut_arg = INFINITY;
@@ -183,7 +192,7 @@ void bqb_batch_destroy(bqb_batch *b) {
     void *ptrs[] = {b->d_models, b->d_tab, b->d_work, b->d_ns, b->d_nc, b->d_xs, b->d_ls, b->d_xc, b->d_hyp, b->d_prior,
                     b->d_xa, b->d_esm, b->d_em, b->d_st, b->d_red_val, b->d_red_idx, b->d_flags, b->d_mt, b->d_mti, b->d_overflow, b->d_work_ctr, b->d_xsorted, b->d_perm, b->d_iota, b->d_sort_tmp,
                     b->d_period, b->d_xo, b->d_pxo, b->d_wp, b->d_gz, b->d_inst_list, b->d_llg_hyp, b->d_llg_out, b->d_llg_inst,
-                    b->d_llg_period};
+                    b->d_llg_period, b->d_alpha, b->d_rows};
     for (void *p : ptrs) if (p) cudaFree(p);
     for (cudaStream_t st : b->pipe) if (st) cudaStreamDestroy(st);
     if (b->h_flags) cudaFreeHost(b->h_flags);
@@ -228,6 +237,7 @@ static int run_setup(bqb_batch *b, int check_max, cudaStream_t s) {
     a.n_max = n_max; a.nc_max = nc_max;
     a.kind = b->kind; a.period = b->d_period; a.xo = b->d_xo; a.pxo = b->d_pxo; a.n_xo = b->n_xo; a.xo_stride = b->xo_stride;
     a.wp = b->d_wp; a.gz = b->d_gz;
+    a.alpha = b->d_alpha; a.alpha_stride = b->alpha_stride;
     a.inst_list = nullptr;
     // Launch groups: the setup kernel runs two CTAs per SM while two instances fit its shared memory, sized for the
     // LARGEST instance of a launch.  When a few large instances (many surviving candidates) would push a big batch into the
@@ -779,6 +789,96 @@ int bqb_predict_host(bqb_batch *b, const double *x, long long x_stride, int na, 
     CU(cudaMemcpyAsync(l_mean, b->d_esm, sizeof(double) * B * na, cudaMemcpyDeviceToHost, s));
     CU(cudaMemcpyAsync(v_log_l, b->d_em, sizeof(double) * B * na, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
+    return 0;
+}
+
+// The checks of bqb_predict_rows_device / _host.  *listed: rows listed (rows null: every instance), 0 when there is nothing to
+// do (na = 0 or an empty list: the pointers are not looked at, as in bqb_expected_var_rows_device)
+static int predict_rows_check(bqb_batch *b, const char *who, const int *rows, int n_rows, const void *x, long long x_stride, int na,
+                              const void *l_mean, const void *v_log_l, long long out_stride, int *listed) {
+    const std::string name(who);
+    if (!b) return fail(BQB_EINVAL, name + ": null batch");
+    if (na < 0 || out_stride < na || x_stride < 0 || (x_stride && x_stride < na) || (rows && n_rows < 0))
+        return fail(BQB_EINVAL, name + ": bad arguments");
+    for (int i = 0; rows && i < n_rows; ++i)
+        if (rows[i] < 0 || rows[i] >= b->n_inst) return fail(BQB_EINVAL, name + ": row out of range");
+    *listed = (na == 0) ? 0 : rows ? n_rows : b->n_inst;
+    if (*listed == 0) return 0;
+    int rc = check_ready(b, who);
+    if (rc) return rc;
+    if (!x || !l_mean || !v_log_l) return fail(BQB_EINVAL, name + ": bad arguments");
+    return 0;
+}
+
+static int predict_rows_launch(bqb_batch *b, const int *rows, int listed, const double *d_x, long long x_stride, int na,
+                               double *d_l_mean, double *d_v_log_l, long long out_stride, cudaStream_t s) {
+    CU(cudaSetDevice(b->device));
+    PredictArgs a;
+    a.models = b->d_models; a.lay = b->lay; a.alpha = b->d_alpha; a.alpha_stride = b->alpha_stride;
+    a.x = d_x; a.x_stride = x_stride; a.na = na;
+    a.l_mean = d_l_mean; a.v_log_l = d_v_log_l; a.out_stride = out_stride;
+    if (rows) {
+        if ((size_t)listed > b->cap_rows) {
+            if (b->d_rows) cudaFree(b->d_rows);
+            b->d_rows = nullptr; b->cap_rows = 0;
+            CU(cudaMalloc(&b->d_rows, sizeof(int) * (size_t)listed));
+            b->cap_rows = listed;
+        }
+        // (pageable `rows` are staged before the copy call returns; page-locked ones are read when the stream gets there)
+        CU(cudaMemcpyAsync(b->d_rows, rows, sizeof(int) * (size_t)listed, cudaMemcpyHostToDevice, s));
+        a.rows = b->d_rows;
+    }
+    for (int r0 = 0; r0 < listed; r0 += 32768) {               // gridDim.y is limited to 65535
+        a.row0 = r0;
+        CU(launch_predict(a, std::min(listed - r0, 32768), s));
+        b->launches++;
+    }
+    return 0;
+}
+
+int bqb_predict_rows_device(bqb_batch *b, const int *rows, int n_rows, const double *d_x, long long x_stride, int na,
+                            double *d_l_mean, double *d_v_log_l, long long out_stride, void *stream) {
+    int listed = 0;
+    int rc = predict_rows_check(b, "bqb_predict_rows_device", rows, n_rows, d_x, x_stride, na, d_l_mean, d_v_log_l, out_stride,
+                                &listed);
+    if (rc || listed == 0) return rc;
+    return predict_rows_launch(b, rows, listed, d_x, x_stride, na, d_l_mean, d_v_log_l, out_stride, (cudaStream_t)stream);
+}
+
+int bqb_predict_rows_host(bqb_batch *b, const int *rows, int n_rows, const double *x, long long x_stride, int na, double *l_mean,
+                          double *v_log_l) {
+    int listed = 0;
+    int rc = predict_rows_check(b, "bqb_predict_rows_host", rows, n_rows, x, x_stride, na, l_mean, v_log_l, na, &listed);
+    if (rc || listed == 0) return rc;
+    CU(cudaSetDevice(b->device));
+    const size_t B = b->n_inst;
+    const size_t n_x = x_stride ? B * (size_t)x_stride : (size_t)na;
+    rc = grow(b, n_x, B * (size_t)na);
+    if (rc) return rc;
+    cudaStream_t s = 0;
+    CU(cudaMemcpyAsync(b->d_xa, x, sizeof(double) * n_x, cudaMemcpyHostToDevice, s));
+    rc = predict_rows_launch(b, rows, listed, b->d_xa, x_stride, na, b->d_esm, b->d_em, na, s);
+    if (rc) return rc;
+    if (!rows) {
+        CU(cudaMemcpyAsync(l_mean, b->d_esm, sizeof(double) * B * na, cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(v_log_l, b->d_em, sizeof(double) * B * na, cudaMemcpyDeviceToHost, s));
+    }
+    for (int i = 0; rows && i < listed; ++i) {                   // only the listed rows of the outputs are written
+        const size_t o = (size_t)rows[i] * na;
+        CU(cudaMemcpyAsync(l_mean + o, b->d_esm + o, sizeof(double) * na, cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(v_log_l + o, b->d_em + o, sizeof(double) * na, cudaMemcpyDeviceToHost, s));
+    }
+    CU(cudaStreamSynchronize(s));
+    return 0;
+}
+
+int bqb_alpha_read(bqb_batch *b, int inst, double *out) {
+    if (!b || !b->ready || inst < 0 || inst >= b->n_inst || !out) return fail(BQB_EINVAL, "bqb_alpha_read: bad arguments");
+    const double *h = &b->h_hdr[(size_t)inst * H_COUNT];
+    if ((int)h[H_STATUS] != SETUP_OK) return fail(BQB_ENUMERIC, "bqb_alpha_read: the instance failed setup");
+    CU(cudaSetDevice(b->device));
+    const int n = (int)h[H_NS] + (int)h[H_NC];
+    CU(cudaMemcpy(out, b->d_alpha + (size_t)inst * b->alpha_stride, sizeof(double) * n, cudaMemcpyDeviceToHost));
     return 0;
 }
 

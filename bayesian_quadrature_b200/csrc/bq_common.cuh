@@ -142,6 +142,25 @@ struct SetupArgs {
     long long xo_stride;
     double *wp;                // out [B][n_xo]: trapezoid weight x prior density
     double *gz;                // scratch [launch instances][n_xo]
+    // out [B][alpha_stride]: alpha_l = (K_l + s_l^2 I)^-1 l_sc (gp_l.inv_Kxx_y) in model order, zero padded (may be null;
+    // last members: the other parameters keep their offsets)
+    double *alpha;
+    long long alpha_stride;
+};
+
+// Arguments of one launch of the prediction kernel (bq_predict.cu); shared with the C-ABI layer (bq_capi.cu)
+struct PredictArgs {
+    const double *models = nullptr;     // [n_inst][lay.total]
+    Layout lay;
+    const double *alpha = nullptr;      // [n_inst][alpha_stride], written by the setup kernel
+    long long alpha_stride = 0;
+    const int *rows = nullptr;          // CTA row y works on instance rows[row0 + y] (null: instance row0 + y)
+    int row0 = 0;
+    const double *x = nullptr;          // [na] (x_stride = 0) or [n_inst][x_stride]
+    long long x_stride = 0;
+    int na = 0;
+    double *l_mean = nullptr, *v_log_l = nullptr;   // [n_inst][out_stride]
+    long long out_stride = 0;
 };
 
 // Arguments of one launch of the log-likelihood gradient kernel (bq_setup2.cu); shared with the C-ABI layer (bq_capi.cu).
@@ -259,6 +278,29 @@ __device__ __forceinline__ double exp_tab(double x, const double *__restrict__ t
 __device__ __forceinline__ double kernel_exp(double d, double nh, int kind, double hp) {
     if (kind) d = 2.0 * sin(d * hp);
     return exp((d * d) * nh);
+}
+
+// ---- plain-FP64 kernels (bq_score_generic.cu, bq_predict.cu): eight warps share a tile of 32 query points, lane = point
+constexpr int GEN_THREADS = 32;              // points per tile (= lanes)
+constexpr int GEN_WARPS = 8;                 // warps of a CTA: they share the tile
+
+// sum_{k <= r} F[r][k] e[k] for row r of a triangular fragment-ordered operand: a k-step is four consecutive doubles of the
+// row (32-byte aligned: two 16-byte warp-uniform loads); entries with k > r are stored as zeros, so whole k-steps are used
+// (the e buffer, [k][lane] in shared memory, is zero for k >= ns)
+__device__ __forceinline__ double tri_row_dot(const double *F, int r, const double *s_e, int lane) {
+    const int rb = r >> 3;
+    const double2 *row = reinterpret_cast<const double2 *>(F + ((rb * (rb + 1)) << 5) + ((r & 7) << 2));
+    const double *e = s_e + lane;
+    double s0 = 0.0, s1 = 0.0;
+    for (int ks = 0; ks <= (r >> 2); ++ks) {
+        const double2 f01 = row[ks << 4], f23 = row[(ks << 4) + 1];
+        const double *ek = e + (ks << 2) * GEN_THREADS;
+        s0 = fma(f01.x, ek[0], s0);
+        s1 = fma(f01.y, ek[GEN_THREADS], s1);
+        s0 = fma(f23.x, ek[2 * GEN_THREADS], s0);
+        s1 = fma(f23.y, ek[3 * GEN_THREADS], s1);
+    }
+    return s0 + s1;
 }
 
 __device__ __forceinline__ double warp_sum(double v) {

@@ -16,28 +16,7 @@
 
 namespace bqb {
 
-constexpr int GEN_THREADS = 32;              // points per tile (= lanes)
-constexpr int GEN_WARPS = 8;                 // warps of a CTA: they share the tile
 constexpr int GEN_MAX_GRID = 2048;            // the fused epilogue leaves one (min, index) partial per CTA
-
-// sum_{k <= r} F[r][k] e[k] for row r of a triangular fragment-ordered operand: a k-step is four consecutive doubles of the
-// row (32-byte aligned: two 16-byte warp-uniform loads); entries with k > r are stored as zeros, so whole k-steps are used
-// (the e buffer is zero for k >= ns)
-__device__ __forceinline__ double tri_row_dot(const double *F, int r, const double *s_e, int lane) {
-    const int rb = r >> 3;
-    const double2 *row = reinterpret_cast<const double2 *>(F + ((rb * (rb + 1)) << 5) + ((r & 7) << 2));
-    const double *e = s_e + lane;
-    double s0 = 0.0, s1 = 0.0;
-    for (int ks = 0; ks <= (r >> 2); ++ks) {
-        const double2 f01 = row[ks << 4], f23 = row[(ks << 4) + 1];
-        const double *ek = e + (ks << 2) * GEN_THREADS;
-        s0 = fma(f01.x, ek[0], s0);
-        s1 = fma(f01.y, ek[GEN_THREADS], s1);
-        s0 = fma(f23.x, ek[2 * GEN_THREADS], s0);
-        s1 = fma(f23.y, ek[3 * GEN_THREADS], s1);
-    }
-    return s0 + s1;
-}
 
 __global__ void __launch_bounds__(GEN_THREADS * GEN_WARPS) bq_score_generic_kernel(ScoreArgs a) {
     extern __shared__ double s_e[];                                  // [nsp][32] cross-kernel exponentials of the tile's points
@@ -272,7 +251,7 @@ __global__ void __launch_bounds__(GEN_THREADS * GEN_WARPS) bq_score_generic_kern
 }
 
 // Same contract as launch_score (bq_score.cu): grid_x receives the number of CTAs per instance (= partials of the fused
-// epilogue).  Prediction mode is not offered by this kernel.
+// epilogue).  Prediction mode is not offered by this kernel: bq_predict.cu predicts for every batch.
 cudaError_t launch_score_generic(const ScoreArgs &a, int n_inst, cudaStream_t stream, int *grid_x) {
     if (a.predict) return cudaErrorNotSupported;
     if (a.na <= 0 || n_inst <= 0) { if (grid_x) *grid_x = 0; return cudaSuccess; }

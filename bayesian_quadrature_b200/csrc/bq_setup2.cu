@@ -776,6 +776,12 @@ __global__ void __launch_bounds__(NT, 512 / NT) bq_setup2_kernel(SetupArgs a) {
         for (int i = tid; i < n; i += NT) p += log(T[tri(i) + i]);
         sumlog_l = block_sum2<NT>(p, red);
     }
+    // alpha_l kept for the prediction kernel (bq_predict.cu): entry k belongs to x_sc[k], i.e. to M[off_xs + k] (k < ns) or
+    // M[off_xc + k - ns]; zeros after n
+    if (a.alpha) {
+        double *ao = a.alpha + (size_t)inst * a.alpha_stride;
+        for (int i = tid; i < a.alpha_stride; i += NT) ao[i] = i < n ? alpha[i] : 0.0;
+    }
     PH(18);
     // ---- P12: Z_mean = int_K . alpha_l  (bq_c.pyx:207-209)
     double pz = 0.0;

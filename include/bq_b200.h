@@ -125,7 +125,8 @@ int bqb_batch_set_periods(bqb_batch *b, const double *period, void *stream);
  *             [n_xo] shared by all instances when xo_stride = 0, else [n_inst][xo_stride]); n_xo = 0: closed forms
  *             (Gaussian kernel only).
  *   force_generic != 0 runs the plain-FP64 scoring kernel even for the Gaussian / closed-form case (cross-checks).
- * Takes effect at the next setup call; afterwards every scoring entry point except bqb_predict_* works as before. */
+ * Takes effect at the next setup call; afterwards every scoring entry point except bqb_predict_device / _host works as
+ * before (bqb_predict_rows_* predicts for every batch). */
 int bqb_batch_set_approx(bqb_batch *b, int kernel_kind, const double *period, const double *xo, const double *p_xo, int n_xo,
                          long long xo_stride, int force_generic);
 /* The setup half: runs the setup kernel on whatever is staged on the device (after bqb_batch_stage /
@@ -191,10 +192,36 @@ int bqb_score_device_grouped(bqb_batch *b, int inst0, int n_inst, const double *
 /* Batched prediction at na points for every instance (SURVEY.md §8(f).4): l_mean = gp_l.mean(x), the mean of the final
  * approximation (BQ.l_mean, bq.py:177-200), and v_log_l = diag gp_log_l.cov(x), from which BQ.l_var (bq.py:202-231) is
  * max(v_log_l * l_mean^2, 0).  Same layout conventions as bqb_score_*; requires s_l = 0 (the scoring factors are those
- * of the noise-free bordered matrix, SURVEY appendix A.2). */
+ * of the noise-free bordered matrix, SURVEY appendix A.2) and a tensor-core batch (BQB_EUNSUPPORTED after
+ * bqb_batch_set_approx or in the 512 class); bqb_predict_rows_* below has neither limit. */
 int bqb_predict_device(bqb_batch *b, const double *d_x, long long x_stride, int na, double *d_l_mean,
                        double *d_v_log_l, long long out_stride, void *stream);
 int bqb_predict_host(bqb_batch *b, const double *x, long long x_stride, int na, double *l_mean, double *v_log_l);
+
+/* Prediction for any batch -- tensor-core or generic, Gaussian or periodic kernel, every capacity class, any s_l -- on the
+ * instances listed in `rows`: l_mean = gp_l.mean(x) (BQ.l_mean, bq.py:177-200) and v_log_l = diag gp_log_l.cov(x), from which
+ * BQ.l_var (bq.py:202-231) is max(v_log_l * l_mean^2, 0).  The mean is K_l(x, x_sc) alpha_l with the alpha_l = (K_l + s_l^2 I)^-1
+ * l_sc that the setup keeps (gp_l.inv_Kxx_y, bqb_alpha_read); the variance is K_tl(x, x) - |L_tl^-1 k_tl(x)|^2.  No shortcut,
+ * no jitter pattern: a non-finite point gives NaN in both outputs.
+ *   rows: HOST array of n_rows instance indices (any order, repeats allowed), or null for every instance (n_rows ignored).
+ *         It is copied to a batch-owned device buffer on `stream` (a page-locked array is read when the stream reaches
+ *         the copy), so calls on one batch must not overlap on different streams.
+ *   Row i of the outputs (at i * out_stride), and row i of x when x_stride != 0, belong to INSTANCE i; rows of instances
+ *   that are not listed are not written.  A point's result does not depend on the other rows or points of the call.
+ * BQB_EINVAL for a null batch or pointer, n_rows < 0, a row out of range, x_stride in (0, na) or out_stride < na;
+ * BQB_ESTATE / BQB_ENUMERIC when the batch is not set up / an instance failed setup.  na = 0 or an empty list does nothing
+ * (the pointers and the batch's state are then not looked at).
+ * The _device form takes DEVICE pointers and is asynchronous on `stream`; the _host form takes host arrays, outputs
+ * [n_inst][na], and returns when they are written. */
+int bqb_predict_rows_device(bqb_batch *b, const int *rows, int n_rows, const double *d_x, long long x_stride, int na,
+                            double *d_l_mean, double *d_v_log_l, long long out_stride, void *stream);
+int bqb_predict_rows_host(bqb_batch *b, const int *rows, int n_rows, const double *x, long long x_stride, int na,
+                          double *l_mean, double *v_log_l);
+
+/* The ns + nc entries of alpha_l = (K_l + s_l^2 I)^-1 l_sc of instance `inst` from the last setup, in model order: entry k
+ * belongs to the k-th observation in ascending order for k < ns, then to candidate k - ns.  BQB_EINVAL for bad arguments or
+ * a batch that is not set up, BQB_ENUMERIC when the instance failed setup. */
+int bqb_alpha_read(bqb_batch *b, int inst, double *out);
 
 /* out[p] = Z_mean^2 + Z_var - esm[p] for instance `inst` (BQ.expected_Z_var, bq.py:374-377).
  * DEVICE pointers. */
