@@ -68,6 +68,7 @@ SYMBOLS = {
     "bqb_choose_step_exchange": (ctypes.c_int, [_vp, ctypes.c_int, _vp, ctypes.c_int, _vp, _vp, _ll, _ll, ctypes.POINTER(_vp), ctypes.c_int,
                                                 ctypes.c_int, ctypes.c_ulonglong, _vp, _vp]),
     "bqb_argmin_rows_device": (ctypes.c_int, [_vp, _vp, _ll, _ll, _vp, _vp, _vp]),
+    "bqb_argmin_ties_rows_device": (ctypes.c_int, [_vp, _vp, _ll, _ll, _vp, _vp, _vp, _vp, _vp]),
     "bqb_batch_set_cutoff": (ctypes.c_int, [_vp, ctypes.c_double]),
     "bqb_batch_set_presort": (ctypes.c_int, [_vp, ctypes.c_int]),
     "bqb_batch_set_zero_copy": (ctypes.c_int, [_vp, ctypes.c_int]),
@@ -484,6 +485,13 @@ class Batch(object):
         """Per-instance (min, first index) of the CUDA tensor v [n_inst, n] into mins (float64) / idxs (int64)."""
         _check(load().bqb_argmin_rows_device(self._h, _ptr(v), v.stride(0), v.shape[1], _ptr(mins), _ptr(idxs),
                                              _stream(stream)), "bqb_argmin_rows_device")
+
+    def argmin_ties_rows_device(self, v, mins, u, idxs, counts=None, stream=None):
+        """Per-instance random pick among the points of v [n_inst, n] within np.isclose of mins [n_inst] (bq.py:664-665):
+        the k-th close point, k = min(floor(u * c), c - 1) of c close points, for uniforms u [n_inst] in [0, 1), into
+        idxs (int64); counts (int64, optional) receives c.  CUDA tensors, no host synchronisation."""
+        _check(load().bqb_argmin_ties_rows_device(self._h, _ptr(v), v.stride(0), v.shape[1], _ptr(mins), _ptr(u), _ptr(idxs),
+                                                  _ptr(counts), _stream(stream)), "bqb_argmin_ties_rows_device")
 
     def set_cutoff(self, cut_arg):
         """Relevance cut-off of the band skipping (default 72; float('inf') = dense algorithm)."""

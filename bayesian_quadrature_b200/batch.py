@@ -15,6 +15,9 @@ RNG), and device arrays are padded to the batch's largest ``ns`` / ``nc``.
 step (``log_lh``), and ``marginal_loss`` scores the P x S (problem, sample) instances in chunks of whole problems.  Chain p
 draws from its own counter-based stream keyed by the pair (seed, p) (the reference's single global libc ``rand`` stream
 cannot be split per problem; SURVEY appendix A.4 documents the same choice for the candidate streams).
+``choose_next(..., deterministic=False)`` breaks ties like the reference (a uniform pick among the points within
+``np.isclose`` of the minimum) with one draw from that stream, and ``marginalize`` returns Z_mean, Z_var and the per-point
+read-outs of every problem under each of its samples.
 
 ``kernel=PeriodicKernel`` runs every problem with the periodic kernel, as ``BQ(kernel=PeriodicKernel)`` does: the
 parameters of a GP are (h, w, p, s), candidates are drawn on [-pi p_tl, pi p_tl] (bq.py:217-218), and the integrals are
@@ -419,9 +422,10 @@ class BatchBQ(object):
             cache[key] = _lib.Batch(n_inst, self._cap_class, device=self.device)
         return cache[key]
 
-    def _chunks(self, S, na):
-        """(problems per setup chunk, problems per scoring launch) under MODEL_CHUNK_BYTES / LOSS_CHUNK_BYTES."""
-        model_bytes = 8 * _lib.load().bqb_model_doubles(self.batch._h)
+    def _chunks(self, S, na, row_bytes=0):
+        """(problems per setup chunk, problems per scoring launch) under MODEL_CHUNK_BYTES / LOSS_CHUNK_BYTES; row_bytes
+        of per-instance buffers that live as long as a setup chunk count against MODEL_CHUNK_BYTES."""
+        model_bytes = 8 * _lib.load().bqb_model_doubles(self.batch._h) + row_bytes
         if self.periodic:
             model_bytes += 8 * (3 * N_GRID + 2)           # grid, prior density, trapezoid weights and periods per instance
         per_score = max(1, min(self.P, self.LOSS_CHUNK_BYTES // max(8 * S * max(na, 1), 1)))
@@ -438,6 +442,45 @@ class BatchBQ(object):
         x_a = np.ascontiguousarray(x_a, dtype=np.float64)
         return x_a, torch.from_numpy(x_a).to(dev)
 
+    def _sample_rows(self, hypers_tl, hypers_l, params):
+        """Hyper-parameter rows [P, S, 6 | 8] of the (problem, sample) instances, checked as GP.set_param checks them."""
+        hyp = self._hyp_rows(hypers_tl, hypers_l, params)
+        if hyp.ndim != 3:
+            raise ValueError("hypers_tl and hypers_l must be [P, S, %d]" % len(params))
+        if hyp.shape[1] < 1:
+            raise ValueError("at least one hyper-parameter sample per problem")
+        ok = self._valid_hyp(hyp)
+        if not ok.all():
+            p, i = np.argwhere(~ok)[0]
+            raise ValueError("invalid hyper-parameters %s in sample %d of problem %d" % (hyp[p, i], i, p))
+        return hyp
+
+    def _setup_samples(self, hyp, per_setup):
+        """Sets up the P x S (problem, sample) instances of the rows hyp [P, S, 6 | 8] in chunks of per_setup whole problems,
+        each with the semantics of ``_set_gp_log_l_params`` / ``_set_gp_l_params`` (bq.py:933-965: l_c recomputed, "GP mean is
+        too large" guard) and, with the periodic kernel, its problem's grid; yields (first problem, problems, device batch,
+        info) per chunk, instance r of the batch being problem p0 + r // S, sample r % S.  The batch is reused by the next
+        chunk.  A failed setup is logged with its parameters and raised with the problem and the sample named
+        (``BQ.marginalize`` drops no sample either)."""
+        S = hyp.shape[1]
+        stride = min(self.cap, self._cap_class)
+        for p0 in range(0, self.P, per_setup):
+            cp = min(per_setup, self.P - p0)
+            rep = lambda a: np.repeat(a[p0:p0 + cp], S, axis=0)
+            batch = self._sample_batch(cp * S)
+            hrows = hyp[p0:p0 + cp].reshape(cp * S, hyp.shape[-1])
+            if self.periodic:                             # each sample's periods, its problem's grid
+                batch.set_approx(1, period=hrows[:, 6:], xo=rep(self.xo), p_xo=rep(self.p_xo))
+            info = batch.setup(rep(self.ns), rep(self.nc), rep(self.x_s[:, :stride]), rep(self.l_s[:, :stride]), rep(self.x_c),
+                               hrows[:, :6], rep(self.prior), check_max=True)
+            bad = np.nonzero(info["status"])[0]
+            if bad.size:
+                p, i = divmod(int(bad[0]), S)
+                logger.error("error with parameters %s", hyp[p0 + p, i])
+                exc, msg = _SETUP_ERRORS.get(int(info["status"][bad[0]]), (RuntimeError, "device setup failed"))
+                raise exc("%s (problem %d, sample %d)" % (msg, p0 + p, i))
+            yield p0, cp, batch, info
+
     def marginal_loss(self, x_a, hypers_tl, hypers_l, params, timings=None):
         """Marginal loss of choose_next for every problem: the mean over its S samples (hypers_tl / hypers_l
         [P, S, len(params)]) of ``-expected_squared_mean(x_a)`` (bq.py:640-663), as a [P, na] CUDA tensor; row p is
@@ -452,22 +495,13 @@ class BatchBQ(object):
         ``timings``, when a dict, receives the seconds spent in the three phases ("setup", "score", "reduce"; CUDA events
         around each launch, which then synchronise after every scoring launch -- for measurements only)."""
         import torch
-        hyp = self._hyp_rows(hypers_tl, hypers_l, params)
-        if hyp.ndim != 3:
-            raise ValueError("hypers_tl and hypers_l must be [P, S, %d]" % len(params))
-        S = hyp.shape[1]
-        if S < 1:
-            raise ValueError("at least one hyper-parameter sample per problem")
         _, x_d = self._query(x_a)
         if x_d.dim() not in (1, 2) or (x_d.dim() == 2 and x_d.shape[0] != self.P):
             raise ValueError("x_a must be [na] or [P, na]")
         na = x_d.shape[-1]
         self.sync_host()
-        ok = self._valid_hyp(hyp)
-        if not ok.all():
-            p, i = np.argwhere(~ok)[0]
-            raise ValueError("invalid hyper-parameters %s in sample %d of problem %d" % (hyp[p, i], i, p))
-        stride = min(self.cap, self._cap_class)
+        hyp = self._sample_rows(hypers_tl, hypers_l, params)
+        S = hyp.shape[1]
         per_setup, per_score = self._chunks(S, na)
         dev = x_d.device
         loss = torch.zeros(self.P, na, dtype=torch.float64, device=dev)
@@ -477,22 +511,8 @@ class BatchBQ(object):
         flags = torch.zeros(per_score * S, dtype=torch.int32, device=dev)
         bad_esm = torch.zeros(self.P, dtype=torch.bool, device=dev)
         bad_xa = torch.zeros(self.P, dtype=torch.bool, device=dev)
-        for p0 in range(0, self.P, per_setup):
-            cp = min(per_setup, self.P - p0)
-            rep = lambda a: np.repeat(a[p0:p0 + cp], S, axis=0)
-            batch = self._sample_batch(cp * S)
-            t0 = time.perf_counter()
-            hrows = hyp[p0:p0 + cp].reshape(cp * S, hyp.shape[-1])
-            if self.periodic:                             # each sample's periods, its problem's grid
-                batch.set_approx(1, period=hrows[:, 6:], xo=rep(self.xo), p_xo=rep(self.p_xo))
-            info = batch.setup(rep(self.ns), rep(self.nc), rep(self.x_s[:, :stride]), rep(self.l_s[:, :stride]), rep(self.x_c),
-                               hrows[:, :6], rep(self.prior), check_max=True)
-            bad = np.nonzero(info["status"])[0]
-            if bad.size:
-                p, i = divmod(int(bad[0]), S)
-                logger.error("error with parameters %s", hyp[p0 + p, i])
-                exc, msg = _SETUP_ERRORS.get(int(info["status"][bad[0]]), (RuntimeError, "device setup failed"))
-                raise exc("%s (problem %d, sample %d)" % (msg, p0 + p, i))
+        t0 = time.perf_counter()
+        for p0, cp, batch, _ in self._setup_samples(hyp, per_setup):
             if timings is not None:
                 timings["setup"] = timings.get("setup", 0.0) + time.perf_counter() - t0     # setup synchronises
             for q0 in range(0, cp, per_score):
@@ -513,6 +533,7 @@ class BatchBQ(object):
                 fl = flags[:cq * S].view(cq, S)
                 bad_esm[p0 + q0:p0 + q0 + cq] |= ((fl & (_lib.ST_ESM_BAD | _lib.ST_EM_BAD)) != 0).any(dim=1)
                 bad_xa[p0 + q0:p0 + q0 + cq] |= ((fl & _lib.ST_XA_BAD) != 0).any(dim=1)
+            t0 = time.perf_counter()                      # the next chunk's setup starts here
         loss /= S                                         # bq.py:662
         if bool(bad_xa.any().item()):
             raise ValueError("invalid value in x_a of problem %d" % int(torch.nonzero(bad_xa)[0, 0].item()))
@@ -522,26 +543,29 @@ class BatchBQ(object):
         return loss
 
     # ---------------------------------------------------------------- one active-sampling round
-    def choose_next(self, x_a, on_device=False, n=None, params=None, hypers=None, seed=None, max_steps=None):
-        """Deterministic choose_next of every problem over a shared grid ``x_a`` [na] or per-problem grids
-        [P, na]: index and location of the first maximiser of expected_squared_mean.  ``x_a`` may be a float64
-        CUDA tensor (it is then not uploaded again); with ``on_device=True`` the result is a pair of CUDA tensors.
+    def choose_next(self, x_a, on_device=False, n=None, params=None, hypers=None, seed=None, max_steps=None,
+                    deterministic=True):
+        """choose_next of every problem over a shared grid ``x_a`` [na] or per-problem grids [P, na]: index and location of
+        the first maximiser of expected_squared_mean.  ``x_a`` may be a float64 CUDA tensor (it is then not uploaded
+        again); with ``on_device=True`` the result is a pair of CUDA tensors.
 
         With ``n`` (and ``params``), the loss is marginalised over hyper-parameter samples like the reference's
         ``BQ.choose_next(x_a, n, params)`` (bq.py:659-681): ``sample_hypers(params, n, nburn=1, seed, max_steps)`` draws
         them, or ``hypers=(hypers_tl, hypers_l)`` ([P, S, len(params)]) gives them; the choice is the first minimiser of
         each problem's ``marginal_loss``.  Without ``seed``, the r-th sampling round of this batch uses the seed
-        ``util.stream_keys(batch seed, r)``: every round draws fresh streams, as the reference's global stream advances."""
+        ``util.stream_keys(batch seed, r)``: every round draws fresh streams, as the reference's global stream advances.
+
+        ``deterministic=False`` breaks ties like the reference (bq.py:664-665): problem p picks uniformly among the points
+        whose loss is ``np.isclose`` to its minimum, with the uniform ``util.counter_uniform(util.stream_keys(round_seed,
+        p), 2**64 - 1)`` -- its sampler chain's stream at a counter the sampler never reaches, so that a choice depends only
+        on the round's seed and the problem's own losses.  round_seed is ``seed`` when given and otherwise the next round
+        seed of the batch (every call that draws randomness takes one).  The pick runs on the device after the argmin and
+        adds no host synchronisation."""
         if n is not None or hypers is not None:
-            return self._choose_marginal(x_a, on_device, n, params, hypers, seed, max_steps)
+            return self._choose_marginal(x_a, on_device, n, params, hypers, seed, max_steps, deterministic)
         import torch
-        dev = torch.device("cuda", self.device)
-        if isinstance(x_a, torch.Tensor):
-            x_d = x_a.to(dev, torch.float64).contiguous()
-            x_a = None
-        else:
-            x_a = np.ascontiguousarray(x_a, dtype=np.float64)
-            x_d = torch.from_numpy(x_a).to(dev)
+        x_a, x_d = self._query(x_a)
+        dev = x_d.device
         na = x_d.shape[-1]
         if getattr(self, "_esm", None) is None or self._esm.shape != (self.P, na):
             self._esm = torch.empty(self.P, na, dtype=torch.float64, device=dev)
@@ -550,35 +574,31 @@ class BatchBQ(object):
             self._flags = torch.zeros(self.P, dtype=torch.int32, device=dev)
         self.batch.score_device(x_d, self._esm, None, None, self._flags)
         self._esm.neg_()                                  # loss = -esm (bq.py:660)
-        self.batch.argmin_rows_device(self._esm, self._mins, self._idxs)
+        self._pick(self._esm, self._mins, self._idxs, None if deterministic else self._round_seed(seed))
         bad = int((self._flags & (_lib.ST_ESM_BAD | _lib.ST_EM_BAD | _lib.ST_XA_BAD)).ne(0).any().item())
         if bad:
             fl = self._flags.cpu().numpy()
             raise RuntimeError("invalid expected squared mean in problem %d" % int(np.argmax(fl & 112 != 0)))
-        if on_device:
-            x_next = x_d[self._idxs] if x_d.dim() == 1 else x_d.gather(1, self._idxs[:, None])[:, 0]
-            return self._idxs, x_next
-        idx = self._idxs.cpu().numpy()
-        if x_a is None:
-            x_a = x_d.cpu().numpy()
-        x_next = x_a[idx] if x_a.ndim == 1 else x_a[np.arange(self.P), idx]
-        return idx, x_next
+        return self._chosen(x_a, x_d, self._idxs, on_device)
 
-    def _choose_marginal(self, x_a, on_device, n, params, hypers, seed, max_steps):
-        import torch
-        if params is None:
-            raise ValueError("params names the sampled hyper-parameters")
-        if hypers is None:
-            if seed is None:
-                r = self.__dict__.get("_sample_rounds", 0)
-                self._sample_rounds = r + 1
-                seed = int(util.stream_keys(self.seed, r))
-            hypers = self.sample_hypers(params, n, nburn=1, seed=seed, max_steps=max_steps)
-        x_a, x_d = self._query(x_a)
-        loss = self.marginal_loss(x_d, hypers[0], hypers[1], params)
-        mins = torch.empty(self.P, dtype=torch.float64, device=x_d.device)
-        idxs = torch.empty(self.P, dtype=torch.int64, device=x_d.device)
+    def _round_seed(self, seed):
+        """``seed``, or the seed of this batch's next sampling round (util.stream_keys(batch seed, r) for round r)."""
+        if seed is not None:
+            return seed
+        r = self.__dict__.get("_sample_rounds", 0)
+        self._sample_rounds = r + 1
+        return int(util.stream_keys(self.seed, r))
+
+    def _pick(self, loss, mins, idxs, round_seed):
+        """Per-problem choice on the loss rows [P, na]: the first minimiser, or with a round seed the reference's random
+        pick among the points within np.isclose of the minimum (bq.py:664-665; see choose_next)."""
         self.batch.argmin_rows_device(loss, mins, idxs)
+        if round_seed is not None:
+            import torch
+            u = util.counter_uniform(util.stream_keys(round_seed, np.arange(self.P)), np.uint64(2 ** 64 - 1))
+            self.batch.argmin_ties_rows_device(loss, mins, torch.from_numpy(u).to(loss.device), idxs)
+
+    def _chosen(self, x_a, x_d, idxs, on_device):
         if on_device:
             x_next = x_d[idxs] if x_d.dim() == 1 else x_d.gather(1, idxs[:, None])[:, 0]
             return idxs, x_next
@@ -587,6 +607,23 @@ class BatchBQ(object):
             x_a = x_d.cpu().numpy()
         x_next = x_a[idx] if x_a.ndim == 1 else x_a[np.arange(self.P), idx]
         return idx, x_next
+
+    def _choose_marginal(self, x_a, on_device, n, params, hypers, seed, max_steps, deterministic):
+        import torch
+        if params is None:
+            raise ValueError("params names the sampled hyper-parameters")
+        round_seed = None
+        if hypers is None:
+            round_seed = self._round_seed(seed)
+            hypers = self.sample_hypers(params, n, nburn=1, seed=round_seed, max_steps=max_steps)
+        elif not deterministic:
+            round_seed = self._round_seed(seed)
+        x_a, x_d = self._query(x_a)
+        loss = self.marginal_loss(x_d, hypers[0], hypers[1], params)
+        mins = torch.empty(self.P, dtype=torch.float64, device=x_d.device)
+        idxs = torch.empty(self.P, dtype=torch.int64, device=x_d.device)
+        self._pick(loss, mins, idxs, None if deterministic else round_seed)
+        return self._chosen(x_a, x_d, idxs, on_device)
 
     def add_observations(self, x_new, l_new):
         """Vectorised ``add_observation`` (bq.py:683-701): average into the nearest observation when it is
@@ -662,10 +699,12 @@ class BatchBQ(object):
         out[:, perm.cpu().numpy()] = h
         return out
 
-    def _check_flags(self, x_h, x_d, xs, perm, flags):
-        """BQ's post-checks from the per-problem OR of the status bits: ValueError for a non-finite point (bq.py:451-452);
-        per-point status is fetched only for problems with a bit other than ST_SHORTCUT | ST_NOTPD, which then get
-        ``BQ._report`` (bq.py:514-525: RuntimeError, or logged warnings for infinities) with the problem named."""
+    def _check_flags(self, x_h, x_d, xs, perm, flags, batch=None, S=1, p0=0):
+        """BQ's post-checks from the per-instance OR of the status bits: ValueError for a non-finite point (bq.py:451-452);
+        per-point status is fetched only for instances with a bit other than ST_SHORTCUT | ST_NOTPD, which then get
+        ``BQ._report`` (bq.py:514-525: RuntimeError, or logged warnings for infinities) with the problem named.  Row r of
+        flags is instance r of ``batch`` (default: the batch's own); with S > 1 that is sample r % S of problem
+        p0 + r // S (``marginalize``), and the sample is named too."""
         import torch
         fl = flags.cpu().numpy()
         if not (fl & ~(_lib.ST_SHORTCUT | _lib.ST_NOTPD)).any():
@@ -674,17 +713,18 @@ class BatchBQ(object):
             x_h = x_d.cpu().numpy()
         bad = np.nonzero(fl & _lib.ST_XA_BAD)[0]
         if bad.size:
-            p = int(bad[0])
+            p = p0 + int(bad[0]) // S
             row = x_h if x_h.ndim == 1 else x_h[p]
             raise ValueError("invalid value for x_a of problem %d: %s" % (p, row[np.argmax(~np.isfinite(row))]))
         na = x_d.shape[-1]
-        for p in np.nonzero(fl & ~(_lib.ST_SHORTCUT | _lib.ST_NOTPD))[0]:
-            p = int(p)
+        for r in np.nonzero(fl & ~(_lib.ST_SHORTCUT | _lib.ST_NOTPD))[0]:
+            p, i = p0 + int(r) // S, int(r) % S
             esm = torch.empty(1, na, dtype=torch.float64, device=x_d.device)
             em, st = torch.empty_like(esm), torch.empty(1, na, dtype=torch.int32, device=x_d.device)
-            self.batch.score_device_range(p, 1, xs if xs.dim() == 1 else xs[p:p + 1], esm, em, st)
+            (batch or self.batch).score_device_range(int(r), 1, xs if xs.dim() == 1 else xs[p:p + 1], esm, em, st)
             esm, em, st = (self._unsort(t, perm, False)[0] for t in (esm, em, st))
-            BQ._report(x_h if x_h.ndim == 1 else x_h[p], esm, em, st, where=" (problem %d)" % p)
+            where = " (problem %d)" % p if S == 1 else " (problem %d, sample %d)" % (p, i)
+            BQ._report(x_h if x_h.ndim == 1 else x_h[p], esm, em, st, where=where)
 
     def _score_all(self, x_a, want_em, on_device):
         """(esm, em or None) [P, na] of every problem in one scoring pass over the batch."""
@@ -753,18 +793,21 @@ class BatchBQ(object):
         self._check_flags(x_h, x_d, xs, perm, flags)
         return out
 
-    def _host_gps(self, p):
+    def _host_gps(self, p, row=None, l_c=None):
         """``BQ.init``'s two GPs of problem p (bq.py:132-171) from the batch's state: gp_log_l over (x_s, log l_s), gp_l over
-        the observations and the candidates with their values l_c from the setup."""
+        the observations and the candidates with their values l_c from the setup.  ``row`` / ``l_c``: a hyper-parameter row
+        [6 | 8] (``_rows``) and the candidates' values of that set-up instead of the batch's own (a sample of
+        ``marginalize``)."""
         n, c = int(self.ns[p]), int(self.nc[p])
-        h = self.hyp[p]
+        h = self._rows()[p] if row is None else row
+        l_c = self.info["l_c"][p] if l_c is None else l_c
         if self.periodic:
-            k_tl, k_l = PeriodicKernel(h[0], h[1], self.period[p, 0]), PeriodicKernel(h[3], h[4], self.period[p, 1])
+            k_tl, k_l = PeriodicKernel(h[0], h[1], h[6]), PeriodicKernel(h[3], h[4], h[7])
         else:
             k_tl, k_l = GaussianKernel(h[0], h[1]), GaussianKernel(h[3], h[4])
         x_s, l_s = self.x_s[p, :n], self.l_s[p, :n]
         gp_log_l = GP(k_tl, x_s, np.log(l_s), s=h[2])
-        gp_l = GP(k_l, np.concatenate([x_s, self.x_c[p, :c]]), np.concatenate([l_s, self.info["l_c"][p, :c]]), s=h[5])
+        gp_l = GP(k_l, np.concatenate([x_s, self.x_c[p, :c]]), np.concatenate([l_s, l_c[:c]]), s=h[5])
         return gp_log_l, gp_l
 
     def _predict(self, x):
@@ -817,3 +860,159 @@ class BatchBQ(object):
         lv = v * (m * m)
         lv = torch.where(lv < 0, torch.zeros_like(lv), lv)
         return lv if on_device else lv.cpu().numpy()
+
+    # ---------------------------------------------------------------- marginals over hyper-parameter samples (bq.py:604-657)
+    _SCALARS = ("Z_mean", "Z_var")
+    _SCORED = ("expected_Z_var", "expected_squared_mean", "expected_mean", "expected_squared_mean_and_mean")
+    _PREDICTED = ("l_mean", "l_var")
+
+    def marginalize(self, funs, n=None, params=None, hypers=None, seed=None, max_steps=None, on_device=False):
+        """The quantities ``funs`` of every problem under each of its hyper-parameter samples (``BQ.marginalize``,
+        bq.py:604-657): entry [p, i] of a result is what ``BQ(problem p).marginalize`` returns for sample i.
+
+        ``funs`` lists "Z_mean", "Z_var" and pairs (name, x) of a per-point read-out ("expected_Z_var",
+        "expected_squared_mean", "expected_mean", "expected_squared_mean_and_mean", "l_mean", "l_var") and its grid x, a
+        shared [na] or per-problem [P, na] (numpy or a float64 CUDA tensor), as the read-out methods take it.  The samples
+        are drawn like ``choose_next``'s, ``sample_hypers(params, n, nburn=1, seed, max_steps)`` with the next round seed of
+        the batch when ``seed`` is None, or given as ``hypers=(hypers_tl, hypers_l)`` [P, S, len(params)].  Returns a list
+        in the order of ``funs``: [P, S] numpy arrays for the scalars, [P, S, na] ([P, S, na, 2] for the pair) for the
+        read-outs, CUDA tensors with ``on_device=True``.
+
+        The P x S instances are set up in chunks of whole problems, as ``marginal_loss`` sets them up; Z_mean and Z_var come
+        from the setup.  The read-outs of one grid share one grouped scoring pass per scoring chunk (the expected mean only
+        when it is asked for; shared grids BQ would pre-sort are scored sorted), and l_mean / l_var take ``_predict``'s
+        route per instance under its sampled s_l, with host GPs of that instance for problems with a non-finite point
+        (l_mean is then NaN there and l_var raises gp_log_l.cov's ValueError, as BQ.l_mean / BQ.l_var do).
+        Host results are copied back chunk by chunk.  A sample whose setup fails raises at once, naming the problem and
+        the sample; the scoring post-checks of the read-outs name them too; Z_mean <= 0 or Z_var <= 0 give one warning per
+        call.  The batch's model, hyper-parameters and candidates are not touched."""
+        import torch
+        accepted = "'Z_mean', 'Z_var' or (name, x) with name in %s" % ", ".join(self._SCORED + self._PREDICTED)
+        specs = []
+        for f in funs:
+            if isinstance(f, str) and f in self._SCALARS:
+                specs.append((f, None))
+            elif isinstance(f, (tuple, list)) and len(f) == 2 and isinstance(f[0], str) and f[0] in self._SCORED + self._PREDICTED:
+                specs.append((f[0], f[1]))
+            else:
+                raise ValueError("unknown quantity %r: marginalize accepts %s" % (f, accepted))
+        if params is None:
+            raise ValueError("params names the sampled hyper-parameters")
+        if hypers is None:
+            if n is None:
+                raise ValueError("marginalize needs n (samples to draw) or hypers")
+            hypers = self.sample_hypers(params, n, nburn=1, seed=self._round_seed(seed), max_steps=max_steps)
+        self.sync_host()
+        hyp = self._sample_rows(hypers[0], hypers[1], params)
+        P, S = self.P, hyp.shape[1]
+        grids = {}                                        # one per distinct grid object: its read-outs share the passes
+        for name, x in specs:
+            if x is not None:
+                grids.setdefault(id(x), {"x": x, "names": set()})["names"].add(name)
+        na_score, row_bytes = 0, 0
+        for g in grids.values():
+            g["x_h"], g["x_d"] = self._grid(g["x"])
+            na = g["x_d"].shape[-1]
+            if g["names"] & set(self._SCORED):
+                g["xs"], g["perm"] = self._presort(g["x_h"], g["x_d"])
+                g["perm_h"] = None if g["perm"] is None or on_device else g["perm"].cpu().numpy()
+                na_score = max(na_score, na)
+            if g["names"] & set(self._PREDICTED):
+                if g["x_h"] is not None:
+                    fin = np.isfinite(g["x_h"]).all(axis=-1)
+                else:
+                    fin = torch.isfinite(g["x_d"]).all(dim=-1).cpu().numpy()
+                g["finite"] = np.broadcast_to(fin, (P,))
+                row_bytes += 8 * na * (3 if g["x_d"].dim() == 2 else 2)     # l_mean, v_log_l (and the repeated grid rows)
+        per_setup, per_score = self._chunks(S, na_score, row_bytes)
+        dev = torch.device("cuda", self.device)
+        f64 = torch.float64
+        out = {}
+        for name, x in specs:
+            if x is not None and (name, id(x)) not in out:
+                shape = (P, S, grids[id(x)]["x_d"].shape[-1]) + ((2,) if name == "expected_squared_mean_and_mean" else ())
+                out[(name, id(x))] = torch.empty(shape, dtype=f64, device=dev) if on_device else np.empty(shape)
+        want_em = any(g["names"] & {"expected_mean", "expected_squared_mean_and_mean"} for g in grids.values())
+        esm = torch.empty(per_score * S, na_score, dtype=f64, device=dev) if na_score else None
+        em = torch.empty_like(esm) if na_score and want_em else None
+        z_mean, z_var = np.empty((P, S)), np.empty((P, S))
+
+        def put(key, t, r0, perm, perm_h):
+            """Rows [r0, r0 + t.shape[0]) of the instances (problem-major) of result ``key``, in the caller's point order."""
+            o = out[key]
+            dst = o.reshape((P * S,) + tuple(o.shape[2:]))[r0:r0 + t.shape[0]]
+            if perm is None:
+                (dst if on_device else torch.from_numpy(dst)).copy_(t)
+            elif on_device:
+                dst.index_copy_(1, perm, t)
+            else:
+                dst[:, perm_h] = t.cpu().numpy()
+
+        for p0, cp, batch, info in self._setup_samples(hyp, per_setup):
+            z_mean[p0:p0 + cp] = info["Z_mean"][:cp * S].reshape(cp, S)
+            z_var[p0:p0 + cp] = info["Z_var"][:cp * S].reshape(cp, S)
+            for gid, g in grids.items():
+                names, na = g["names"], g["x_d"].shape[-1]
+                if names & set(self._SCORED):
+                    xs, perm, perm_h = g["xs"], g["perm"], g["perm_h"]
+                    g_em = "expected_mean" in names or "expected_squared_mean_and_mean" in names
+                    flags = torch.zeros(cp * S, dtype=torch.int32, device=dev)
+                    for q0 in range(0, cp if na else 0, per_score):
+                        cq = min(per_score, cp - q0)
+                        r0, nr = (p0 + q0) * S, cq * S
+                        e = esm[:nr, :na]
+                        m = em[:nr, :na] if g_em else None
+                        batch.score_device_grouped(q0 * S, nr, xs if xs.dim() == 1 else xs[p0 + q0:p0 + q0 + cq], S, e, m, None,
+                                                   flags[q0 * S:q0 * S + nr])
+                        if "expected_squared_mean" in names:
+                            put(("expected_squared_mean", gid), e, r0, perm, perm_h)
+                        if "expected_mean" in names:
+                            put(("expected_mean", gid), m, r0, perm, perm_h)
+                        if "expected_squared_mean_and_mean" in names:
+                            put(("expected_squared_mean_and_mean", gid), torch.stack([e, m], dim=-1), r0, perm, perm_h)
+                        if "expected_Z_var" in names:
+                            batch.expected_var_rows_device(q0 * S, nr, e, e)      # in place: esm has been read out
+                            put(("expected_Z_var", gid), e, r0, perm, perm_h)
+                    self._check_flags(g["x_h"], g["x_d"], xs, perm, flags, batch=batch, S=S, p0=p0)
+                if names & set(self._PREDICTED):
+                    self._predict_samples(g, gid, batch, info, hyp, p0, cp, put)
+        for label, v, names in (("m_Z", z_mean, ("Z_mean", "expected_Z_var")), ("V_Z", z_var, ("Z_var", "expected_Z_var"))):
+            bad = np.argwhere(v <= 0)                     # bq_c.pyx:210-211, :352-353
+            if bad.size and any(name in names for name, _ in specs):
+                warnings.warn("%s = %s in (problem, sample) %s" % (label, v[bad[:, 0], bad[:, 1]], [tuple(b) for b in bad.tolist()]))
+        return [z_mean if name == "Z_mean" else z_var if name == "Z_var" else out[(name, id(x))] for name, x in specs]
+
+    def _predict_samples(self, g, gid, batch, info, hyp, p0, cp, put):
+        """l_mean / l_var of grid g for the instances of one setup chunk of ``marginalize``: ``_predict``'s route per instance
+        (MODE 2 for the Gaussian kernel in classes up to 256 where the sampled s_l is 0, the prediction kernel for the rest,
+        host GPs of the instance for a problem with a non-finite point).  Per-problem grids are repeated per sample."""
+        import torch
+        S = hyp.shape[1]
+        x_h, x_d = g["x_h"], g["x_d"]
+        na = x_d.shape[-1]
+        hrows = hyp[p0:p0 + cp].reshape(cp * S, hyp.shape[-1])
+        finite = np.repeat(g["finite"][p0:p0 + cp], S)
+        mode2 = (not self.periodic and self._cap_class <= 256) & (hrows[:, 5] == 0) & finite
+        rows = np.nonzero(finite & ~mode2)[0]
+        x_r = x_d if x_d.dim() == 1 else x_d[p0:p0 + cp].repeat_interleave(S, dim=0)
+        m = torch.empty(cp * S, na, dtype=torch.float64, device=x_d.device)
+        v = torch.empty_like(m)
+        if na and mode2.any():
+            batch.predict_device(x_r, m, v)
+        if na and rows.size:
+            batch.predict_rows_device(x_r, m, v, rows=None if rows.size == cp * S else rows)
+        host = np.nonzero(~finite)[0]
+        if host.size and x_h is None:
+            x_h = x_d.cpu().numpy()
+        for r in host:
+            p = p0 + int(r) // S
+            gp_log_l, gp_l = self._host_gps(p, hrows[r], info["l_c"][r])
+            row = x_h if x_h.ndim == 1 else x_h[p]
+            m[r] = torch.from_numpy(gp_l.mean(row))
+            if "l_var" in g["names"]:                     # (gp_log_l.cov raises for a NaN, gp_l.mean does not: as in BQ)
+                v[r] = torch.from_numpy(np.diag(gp_log_l.cov(row)).copy())
+        if "l_mean" in g["names"]:
+            put(("l_mean", gid), m, p0 * S, None, None)
+        if "l_var" in g["names"]:
+            lv = v * (m * m)
+            put(("l_var", gid), torch.where(lv < 0, torch.zeros_like(lv), lv), p0 * S, None, None)

@@ -31,6 +31,8 @@ cudaError_t launch_argmin(const double *v, long long n, double *bv, long long *b
                           cudaStream_t s);
 cudaError_t launch_argmin_rows(const double *v, long long stride, long long n, int rows, double *mins, long long *idxs,
                                cudaStream_t s);
+cudaError_t launch_argmin_ties_rows(const double *v, long long stride, long long n, int rows, const double *mins, const double *u,
+                                    long long *idxs, long long *counts, cudaStream_t s);
 cudaError_t launch_argmin_exchange(const double *bv, const long long *bi, int nblocks, long long offset, long long cyc_block,
                                    void *const *peer_slots, int world, int rank, unsigned long long seq, double *out, cudaStream_t s);
 cudaError_t sort_points(const double *d_x, int n, double *d_x_sorted, int *d_iota, int *d_perm, void *temp, size_t *temp_bytes,
@@ -1083,6 +1085,16 @@ int bqb_argmin_rows_device(bqb_batch *b, const double *d_v, long long stride, lo
     if (!b || !d_v || n < 1 || stride < n || !d_min || !d_idx) return fail(BQB_EINVAL, "bqb_argmin_rows_device: bad arguments");
     CU(cudaSetDevice(b->device));
     CU(launch_argmin_rows(d_v, stride, n, b->n_inst, d_min, d_idx, (cudaStream_t)stream));
+    b->launches++;
+    return 0;
+}
+
+int bqb_argmin_ties_rows_device(bqb_batch *b, const double *d_v, long long stride, long long n, const double *d_min,
+                                const double *d_u, long long *d_idx, long long *d_count, void *stream) {
+    if (!b || !d_v || n < 1 || stride < n || !d_min || !d_u || !d_idx)
+        return fail(BQB_EINVAL, "bqb_argmin_ties_rows_device: bad arguments");
+    CU(cudaSetDevice(b->device));
+    CU(launch_argmin_ties_rows(d_v, stride, n, b->n_inst, d_min, d_u, d_idx, d_count, (cudaStream_t)stream));
     b->launches++;
     return 0;
 }

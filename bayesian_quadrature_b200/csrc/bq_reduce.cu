@@ -1,7 +1,8 @@
 // Reductions of choose_next / marginalize (bq.py:640-665): the mean over hyper-parameter
 // samples of -esm (sequential in sample order, like numpy's mean(axis=0) over rows), the
-// expected variance Zm^2 + Zv - esm (bq.py:374-377), and a deterministic (min, first index)
-// reduction that shards combine across GPUs.
+// expected variance Zm^2 + Zv - esm (bq.py:374-377), a deterministic (min, first index)
+// reduction that shards combine across GPUs, and the reference's random pick among the points
+// within np.isclose of the minimum (bq.py:664-665).
 #include "bq_common.cuh"
 
 namespace bqb {
@@ -114,6 +115,62 @@ __global__ void argmin_rows_kernel(const double *__restrict__ v, long long strid
     if (threadIdx.x == 0) { mins[blockIdx.x] = best; idxs[blockIdx.x] = idx; }
 }
 
+// numpy's isclose(v, m) with its default tolerances, argument order included (bq.py:664: isclose(loss, best)):
+// |v - m| <= 1e-8 + 1e-5 * |m| for a finite m, or v == m -- equal infinities are close, a finite value is never close to an
+// infinite one, NaN is close to nothing.  Each rounding step is spelled out so that no FMA contraction moves the boundary.
+__device__ __forceinline__ bool isclose_np(double v, double m) {
+    return (fabs(__dsub_rn(v, m)) <= __dadd_rn(1e-8, __dmul_rn(1e-5, fabs(m))) && isfinite(m)) || v == m;
+}
+
+// One CTA per row: the reference's random tie-break (bq.py:664-665, np.random.choice over the points isclose to the
+// minimum).  Pass 1 counts the c points of row r close to mins[r]; pass 2 finds the k-th of them in ascending index order,
+// k = min(floor(u[r] * c), c - 1), a tile of blockDim points at a time (a barrier count per tile, a ballot prefix inside the
+// tile that holds it).  The second pass stops at that tile and mostly re-reads what pass 1 left in L2.  A row with no close
+// point (all NaN) gets NO_INDEX, as argmin_rows_kernel gives it.
+__global__ void argmin_ties_rows_kernel(const double *__restrict__ v, long long stride, long long n, const double *__restrict__ mins,
+                                        const double *__restrict__ u, long long *idxs, long long *counts) {
+    __shared__ long long s_count[32];
+    __shared__ int s_warp[32];
+    const double *row = v + (size_t)blockIdx.x * stride;
+    const double m = mins[blockIdx.x];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    long long c = 0;
+    for (long long p = threadIdx.x; p < n; p += blockDim.x) c += isclose_np(row[p], m);
+    for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+    if (lane == 0) s_count[warp] = c;
+    __syncthreads();
+    c = 0;
+    for (int w = 0; w < nwarps; ++w) c += s_count[w];          // every thread: the row's count
+    if (c == 0) {
+        if (threadIdx.x == 0) {
+            idxs[blockIdx.x] = NO_INDEX;
+            if (counts) counts[blockIdx.x] = 0;
+        }
+        return;
+    }
+    long long k = (long long)__dmul_rn(u[blockIdx.x], (double)c);    // floor: the product is non-negative
+    if (k > c - 1) k = c - 1;
+    long long seen = 0;                                        // close points in the tiles before this one
+    for (long long t = 0; t < n; t += blockDim.x) {
+        const long long p = t + threadIdx.x;
+        const bool hit = p < n && isclose_np(row[p], m);
+        const unsigned ball = __ballot_sync(0xffffffffu, hit);
+        if (lane == 0) s_warp[warp] = __popc(ball);
+        // (the barrier also orders the s_warp stores before their reads; those happen only in the tile that ends the loop)
+        const int in_tile = __syncthreads_count(hit);
+        if (seen + in_tile > k) {                              // the k-th close point lies in this tile
+            if (hit) {
+                long long rank = seen + __popc(ball & ((1u << lane) - 1u));
+                for (int w = 0; w < warp; ++w) rank += s_warp[w];
+                if (rank == k) idxs[blockIdx.x] = p;
+            }
+            break;
+        }
+        seen += in_tile;
+    }
+    if (threadIdx.x == 0 && counts) counts[blockIdx.x] = c;
+}
+
 // One warp: reduces the per-CTA partials into bv[0] / bi[0] and, when `pair` is given, emits the (min, global index as a
 // double) pair for the cross-rank exchange: exact for indices < 2^53
 __global__ void argmin_partials_kernel(double *bv, long long *bi, int nblocks, long long offset, double *pair) {
@@ -145,6 +202,12 @@ cudaError_t launch_pack_info(const double *models, long long model_stride, int o
 cudaError_t launch_argmin_rows(const double *v, long long stride, long long n, int rows, double *mins, long long *idxs,
                                cudaStream_t s) {
     argmin_rows_kernel<<<rows, 256, 0, s>>>(v, stride, n, mins, idxs);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_argmin_ties_rows(const double *v, long long stride, long long n, int rows, const double *mins, const double *u,
+                                    long long *idxs, long long *counts, cudaStream_t s) {
+    argmin_ties_rows_kernel<<<rows, 256, 0, s>>>(v, stride, n, mins, u, idxs, counts);
     return cudaGetLastError();
 }
 

@@ -296,6 +296,16 @@ int bqb_choose_step_exchange(bqb_batch *b, int inst, const double *d_x_a, int na
 int bqb_argmin_rows_device(bqb_batch *b, const double *d_v, long long stride, long long n, double *d_min,
                            long long *d_idx, void *stream);
 
+/* The reference's random tie-break of choose_next (bq.py:664-665: np.random.choice over the points where
+ * np.isclose(loss, loss.min())), per instance: with c the number of j < n where d_v[r][j] is close to d_min[r]
+ * (|v - min| <= 1e-8 + 1e-5 |min| for a finite min, or v == min; NaN is close to nothing) -- d_min as
+ * bqb_argmin_rows_device writes it -- d_idx[r] is the index of the k-th close point in ascending order,
+ * k = min(floor(d_u[r] * c), c - 1), for a uniform d_u[r] in [0, 1).  A row without a close point (all NaN) gets
+ * 0x7fffffffffffffff.  d_count [n_inst] (may be NULL) receives c.  DEVICE pointers, rows d_v [n_inst][stride];
+ * asynchronous on `stream`. */
+int bqb_argmin_ties_rows_device(bqb_batch *b, const double *d_v, long long stride, long long n, const double *d_min,
+                                const double *d_u, long long *d_idx, long long *d_count, void *stream);
+
 /* Band skipping (DESIGN.md): a cross-kernel element exp(-(x_a - x_s[k])^2 / 2w^2) whose exponent lies more than
  * cut_arg below the largest one of its own query point is treated as zero, and groups of four observations in which
  * every element of a 16-point sub-tile is that small are neither exponentiated nor multiplied.  Default 72
